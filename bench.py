@@ -2,7 +2,7 @@
 """Headline benchmark: users/sec for LRURec encode + full-catalogue score + top-20 (BASELINE.json metric)
 on the scaled synthetic catalogue (configs[3]: 10M items, d=64, batch 4096, L=50), on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch of 4096 synthetic users per GPU: sequence preparation,
@@ -14,7 +14,11 @@ all-to-all of the local top-20 lists, merge of the local users' N lists.  `--sca
 the global batch at 4096 (every rank scores the same 4096 users against 1/N of the rows).
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the CPU oracle port of the reference's path on the
-host cores instead (the reference is pure Python/PyTorch; /root/reference is not on the GPU box).
+host cores instead (the reference is pure Python/PyTorch and is not part of this repository).
+
+`--dump-outputs DIR` writes what rank 0's last timed step returned (ids, scores, label_rank, metric_sums and the
+user states u) as DIR/<name>.npy: floating point as float32, integers as float64.  Inputs and weights are
+seeded, so two builds run with the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -29,6 +33,7 @@ import threading
 import time
 from types import SimpleNamespace
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -41,6 +46,7 @@ TOPK = 20
 CPU_SAMPLE_USERS = 1024      # users per pass of the CPU arms: enough to amortise the 2.56 GB table read per pass
 PARITY_USERS = 256           # users of the last timed step whose lists are re-derived independently
 WORKLOAD = "c4_10m: 10M items, d=64, batch 4096, max_len 50, top-20 (BASELINE.json configs[3])"
+DUMP_MAX_BYTES = 64 << 20
 
 
 def peaks():
@@ -185,6 +191,22 @@ def compare_lists(got_i, got_s, ref_i, ref_s, rtol=1e-5):
     return identical, tie_only, int(same.numel()) - identical - tie_only
 
 
+def dump_outputs(out, directory):
+    """Writes every tensor of one step's result as DIR/<name>.npy: floating point as float32 (float64 stays
+    float64), integers as float64, which holds them exactly.  The full arrays are written: one step of this
+    workload returns a few MB, far below DUMP_MAX_BYTES."""
+    arrays = {}
+    for name, t in out.items():
+        if torch.is_tensor(t):
+            t = t.detach().cpu()
+            arrays[name] = t.float() if t.is_floating_point() and t.dtype != torch.float64 else t.double()
+    total = sum(a.numel() * a.element_size() for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs: {total} bytes exceed {DUMP_MAX_BYTES}"
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a.numpy())
+
+
 def verbalizer_fraction(device, pk):
     """lrb_verbalizer_score at BASELINE configs[4]: CUDA-event time of the launch and its algorithmic bytes
     (hidden states once + the 20 label rows + the outputs, SURVEY 8d) against the measured copy bandwidth."""
@@ -262,9 +284,11 @@ def run_reference(args, rank, world):
         users = max(probe_users, int(users * (budget_s / (t_full_est * n_steps)) ** 2))
     times = []
     for s in range(n_steps):
-        dt, _, _ = cpu_oracle_run(sd, table, bias, ids, users)
+        dt, top_s, top_i = cpu_oracle_run(sd, table, bias, ids, users)
         if s >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs({"ids": top_i, "scores": top_s}, args.dump_outputs)
     total = sum(times)
     value = users * len(times) / total
     sample = (f"{users} of the {BATCH} users per step against the full 10M-item table "
@@ -360,6 +384,8 @@ def run_product(args, rank, world, local_rank):
     score_ms = [a.elapsed_time(b) for a, b in model.profile_events]
     model.profile_events = None
     last_main = {"ids": out["ids"].clone(), "scores": out["scores"].clone()}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)          # before any later step reuses the result buffers
 
     def timed_variant(step_fn, x):
         """W warm-up + K timed steps of another step function, device-resident, same bracketing as the headline
@@ -657,7 +683,11 @@ def main():
                          "checks or CPU legs")
     ap.add_argument("--skip-cpu-baseline", action="store_true",
                     help="profiling convenience: omit the ~20 s CPU oracle leg (the default run includes it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, for comparing builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

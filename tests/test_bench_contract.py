@@ -33,5 +33,26 @@ def test_product_arm_has_no_cpu_fallback():
 def test_cli_flags():
     r = _run(["--help"])
     assert r.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--scaling", "--shard-degree", "--exchange"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--scaling", "--shard-degree", "--exchange",
+                 "--dump-outputs"):
         assert flag in r.stdout
+
+
+def test_zero_steps_is_refused():
+    r = _run(["--steps", "0"])
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+def test_dump_outputs_dtypes_and_values(tmp_path):
+    import numpy as np
+    import torch
+    import bench                                  # the repository root is on sys.path (conftest)
+    out = {"ids": torch.tensor([[3, 1 << 30]], dtype=torch.int32), "scores": torch.tensor([[0.5, -1.25]]),
+           "u": torch.tensor([[1.5]], dtype=torch.bfloat16), "metric_sums": torch.ones(4, 3, dtype=torch.float64),
+           "note": "not an array"}
+    bench.dump_outputs(out, str(tmp_path / "d"))
+    got = {p.stem: np.load(p) for p in (tmp_path / "d").iterdir()}
+    assert set(got) == {"ids", "scores", "u", "metric_sums"}
+    assert got["ids"].dtype == np.float64 and got["ids"].tolist() == [[3.0, float(1 << 30)]]
+    assert got["scores"].dtype == np.float32 and got["scores"].tolist() == [[0.5, -1.25]]
+    assert got["u"].dtype == np.float32 and got["metric_sums"].dtype == np.float64
