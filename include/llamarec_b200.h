@@ -159,7 +159,8 @@ int lrb_ce_loss_fwd(const float* hidden, const float* table_f32, const float* bi
  * Train step: loss AND the gradient of every parameter, without the logits tensor.
  * Replaces LRUTrainer.calculate_loss + loss.backward() (trainer/lru.py:22-28, trainer/base.py:107-111),
  * i.e. the backward of model/lru.py:38-41,57-60,73-86,149-161,173-175 under
- * nn.CrossEntropyLoss(ignore_index) (trainer/lru.py:20).  Dropout is the identity; rows must be
+ * nn.CrossEntropyLoss(ignore_index) (trainer/lru.py:20), in eval mode: no dropout (lrb_train_step_dropout
+ * below is the train-mode step; this function is that call with every rate 0).  Rows must be
  * left-padded (dataloader/lru.py:98-118) -- otherwise LRB_ERR_UNSUPPORTED.
  *   ids [B][L] int64/int32 (id_bytes 8/4), labels [B*L] int64
  *   table_f32 [table_rows][64], bias_f32 [table_rows], weights = the packed blob of lrb_encode_fwd,
@@ -177,6 +178,29 @@ int lrb_train_step(const void* ids, int id_bytes, const int64_t* labels, int B, 
                    int64_t table_rows, const float* bias_f32, const float* weights, const float* params_log,
                    int n_blocks, int64_t ignore_index, float* loss_sum, float* grad_weights, float* grad_table,
                    float* grad_bias, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Train step with the reference's train-mode dropout (model/lru.py:47-52,93-97 build the modules):
+ *   site 0        embedding dropout on the gathered row, before the LayerNorm (:57-60)     width 64,  p_embed
+ *   site 1 + 3i   block i, dropout(out_proj(h).real) before the residual add (:160)      width 64,  p_attn
+ *   site 2 + 3i   block i, dropout(gelu(w_1(x))) (:174)                                   width 256, p_ffn
+ *   site 3 + 3i   block i, dropout(w_2(x_)) before the residual add (:175)               width 64,  p_ffn
+ * (p_embed = p_ffn = bert_dropout, p_attn = bert_attn_dropout in the reference.)  The masks are counter-based:
+ * element (t, j) of site s, t = b*L + l, is kept iff word (j & 3) of
+ *   Philox4x32-10(counter = (t, j >> 2, s, 0), key = (seed & 0xffffffff, seed >> 32))   (Random123 constants)
+ * is >= floor(double(p) * 2^32), and a kept element is scaled by 1.0f / (1.0f - p).  The backward recomputes the
+ * masks; nothing is stored, and the workspace is lrb_train_workspace_bytes(B, L, n_blocks).  A rate of 0 turns its
+ * site off exactly.  Every rate must satisfy 0 <= p < 1 (NaN too is rejected): LRB_ERR_BAD_ARG otherwise.
+ * torch's own dropout RNG stream is not reproduced; lrb_dropout_mask gives the masks. */
+int lrb_train_step_dropout(const void* ids, int id_bytes, const int64_t* labels, int B, int L, const float* table_f32,
+                           int64_t table_rows, const float* bias_f32, const float* weights, const float* params_log,
+                           int n_blocks, int64_t ignore_index, float* loss_sum, float* grad_weights,
+                           float* grad_table, float* grad_bias, void* workspace, size_t workspace_bytes,
+                           void* stream, float p_embed, float p_attn, float p_ffn, uint64_t seed);
+
+/* Keep bits of one dropout site of lrb_train_step_dropout: keep[t][j] (device, T x width bytes) = 1 if element
+ * (t, j) survives, 0 if it is dropped -- the same device function the train-step kernels evaluate.  Lets a caller
+ * reproduce a step outside the library.  0 <= p < 1, T >= 1, width >= 1, site >= 0. */
+int lrb_dropout_mask(uint64_t seed, int site, int T, int width, float p, uint8_t* keep, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * k-way merge + Recall/MRR/NDCG + candidate emission, one fused kernel.

@@ -7,7 +7,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import c_char_p, c_int, c_int64, c_size_t, c_void_p, POINTER
+from ctypes import c_char_p, c_float, c_int, c_int64, c_size_t, c_uint64, c_void_p, POINTER
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libllamarec_b200.so")
@@ -43,6 +43,10 @@ SIGNATURES = {
     "lrb_train_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "lrb_train_step": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
                                c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "lrb_train_step_dropout": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int64, c_void_p, c_void_p,
+                                       c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                       c_size_t, c_void_p, c_float, c_float, c_float, c_uint64]),
+    "lrb_dropout_mask": (c_int, [c_uint64, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
     "lrb_peer_push": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p]),
     "lrb_merge_metrics_scatter": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int64, c_int64, c_int64,
                                           c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p]),

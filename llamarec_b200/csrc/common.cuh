@@ -447,4 +447,46 @@ LRB_DEVINL float warp_sum(float v) {
   return v;
 }
 
+// ----------------------------------------------------------------------------
+// Counter-based dropout masks (train step).  Philox4x32-10 with the Random123 constants; the key is bumped
+// between rounds.  Element (t, j) of site s -- t = b*L + l over the [B, L] batch, j the feature inside the
+// site's width -- takes word (j & 3) of Philox(counter = (t, j >> 2, s, 0), key = (seed lo, seed hi)) and is
+// kept iff that word >= thr = floor(p * 2^32); a kept element is multiplied by 1 / (1 - p) (fp32).  The masks
+// are a pure function of (seed, s, t, j): the backward recomputes them, and oracle/dropout_oracle.py restates
+// them bit for bit.
+// ----------------------------------------------------------------------------
+LRB_DEVINL uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r > 0) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+    const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+    c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
+  }
+  return c;
+}
+
+// One dropout site as the kernels see it.  thr == 0 (p == 0, or p below 2^-32) keeps every element with
+// multiplier 1: kernels test `active()` and then evaluate no Philox and multiply by nothing.
+struct DropoutSite {
+  uint32_t key0, key1;   // seed & 0xffffffff, seed >> 32
+  uint32_t site;
+  uint32_t thr;          // floor(double(p) * 2^32)
+  float scale;           // 1.0f / (1.0f - p)
+  __host__ __device__ bool active() const { return thr != 0u; }
+};
+
+// multipliers of features 4*j4 .. 4*j4 + 3 of row t
+LRB_DEVINL float4 dropout_mult4(const DropoutSite& d, uint32_t t, uint32_t j4) {
+  const uint4 r = philox4x32_10(make_uint4(t, j4, d.site, 0u), d.key0, d.key1);
+  return make_float4(r.x >= d.thr ? d.scale : 0.f, r.y >= d.thr ? d.scale : 0.f, r.z >= d.thr ? d.scale : 0.f,
+                     r.w >= d.thr ? d.scale : 0.f);
+}
+// multiplier of feature j of row t
+LRB_DEVINL float dropout_mult(const DropoutSite& d, uint32_t t, uint32_t j) {
+  const float4 m = dropout_mult4(d, t, j >> 2);
+  const uint32_t w = j & 3u;
+  return w == 0 ? m.x : w == 1 ? m.y : w == 2 ? m.z : m.w;
+}
+
 }  // namespace lrb

@@ -8,8 +8,14 @@
 // in_proj * gamma, the diagonal linear recurrence, Re(out_proj) + residual + LayerNorm (:149-161), the PFFN (:173-175),
 // and the tied-embedding scoring matmul + bias (:85) under softmax cross-entropy.
 //
-// Scope.  Dropout is the identity (the reference's dropout mask comes from torch's RNG stream and cannot be
-// parity-matched; eval-mode autograd of the reference is the oracle).  Training batches are LEFT-padded
+// Dropout.  The four sites of model/lru.py (embedding :57-60, after out_proj :160, the PFFN hidden :174 and after
+// w_2 :175) apply counter-based masks (common.cuh, DropoutSite): Philox4x32-10 of (seed, site, token, feature), so
+// the backward recomputes them and oracle/dropout_oracle.py regenerates them.  torch's own dropout RNG stream is
+// not reproduced.  Each mask is fused into a kernel that already touches the element: the gather / scatter of the
+// embedding rows, the SGEMM epilogue before the residual add (backward: the LayerNorm backward writes the masked
+// copy the GEMMs read), and the GELU forward / backward.  With every rate 0 nothing is evaluated or multiplied.
+//
+// Scope.  Training batches are LEFT-padded
 // (dataloader/lru.py:98-118), for which the reference's recursive-doubling scan equals the recurrence
 //     h_p = lambda * (mask_{p-1} h_{p-1}) + bu_p        (SURVEY probe P1),
 // whose backward is the mirrored recurrence; a row with a zero after a non-zero id is rejected (error flag).
@@ -57,6 +63,7 @@ constexpr int BLOCK_FLOATS = B_LN2_B + D;
 // ------------------------------------------------------------------------------------------------------------
 // Tiled SGEMM, 64 x 64 output tile per CTA, 16 x 16 threads x (4 x 4) micro tile, K chunks of 16.
 //   MODE 0 (NN): C[M][N]  = A[M][K] * W[K][N] (+ bias[N]) (+ R[M][N])          forward projections
+//                with an active `drop`: C = mult (.) (A W + bias) + R   (dropout before the residual add)
 //   MODE 1 (NT): C[M][K'] = A[M][N'] * W[K'][N']^T                              dX = dY * W^T   (here K' = rows of W)
 //   MODE 2 (TN): C[K][N] += A[M][K]^T * G[M][N]  over an M slice (atomicAdd)    dW = X^T * dY
 // ------------------------------------------------------------------------------------------------------------
@@ -66,7 +73,8 @@ constexpr int GK = 16;
 template <int MODE>
 __global__ void __launch_bounds__(256) sgemm_kernel(const float* __restrict__ A, const float* __restrict__ W,
                                                     const float* __restrict__ bias, const float* __restrict__ R,
-                                                    float* __restrict__ C, int M, int N, int K, int m_per_cta) {
+                                                    float* __restrict__ C, int M, int N, int K, int m_per_cta,
+                                                    DropoutSite drop) {
   __shared__ float sA[GK][GT + 1];
   __shared__ float sB[GK][GT + 1];
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
@@ -114,16 +122,24 @@ __global__ void __launch_bounds__(256) sgemm_kernel(const float* __restrict__ A,
       }
       __syncthreads();
     }
+    const bool dropped = MODE == 0 && drop.active();
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const int m = m0 + ty * 4 + i;
       if (m >= M) continue;
+      // the thread's four columns n0 + tx*4 .. +3 are one Philox group (n0 is a multiple of 64)
+      float mult[4] = {1.f, 1.f, 1.f, 1.f};
+      if (dropped) {
+        const float4 d = dropout_mult4(drop, static_cast<uint32_t>(m), static_cast<uint32_t>((n0 + tx * 4) >> 2));
+        mult[0] = d.x; mult[1] = d.y; mult[2] = d.z; mult[3] = d.w;
+      }
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const int n = n0 + tx * 4 + j;
         if (n >= NO) continue;
         float v = acc[i][j];
         if (bias != nullptr) v += bias[n];
+        if (dropped) v *= mult[j];
         if (R != nullptr) v += R[static_cast<size_t>(m) * NO + n];
         C[static_cast<size_t>(m) * NO + n] = v;
       }
@@ -185,7 +201,7 @@ __global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ G
 __global__ void __launch_bounds__(256) gather_kernel(const void* __restrict__ ids, int id_bytes, int T, int L,
                                                      const float* __restrict__ table, long long table_rows,
                                                      float* __restrict__ out, unsigned char* __restrict__ mask,
-                                                     int* __restrict__ err_flag) {
+                                                     int* __restrict__ err_flag, DropoutSite drop) {
   const int warp = (blockIdx.x * 256 + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= T) return;
   long long id = load_id(ids, warp, id_bytes);
@@ -197,8 +213,13 @@ __global__ void __launch_bounds__(256) gather_kernel(const void* __restrict__ id
   }
   if (id < 0 || id >= table_rows) id = 0;
   const float* row = table + static_cast<size_t>(id) * D;
-  out[static_cast<size_t>(warp) * D + lane] = row[lane];
-  out[static_cast<size_t>(warp) * D + lane + 32] = row[lane + 32];
+  float v0 = row[lane], v1 = row[lane + 32];
+  if (drop.active()) {   // embedding dropout: the stored row (the LayerNorm input) is mult (.) E[id]
+    v0 *= dropout_mult(drop, warp, lane);
+    v1 *= dropout_mult(drop, warp, lane + 32);
+  }
+  out[static_cast<size_t>(warp) * D + lane] = v0;
+  out[static_cast<size_t>(warp) * D + lane + 32] = v1;
 }
 
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w,
@@ -217,10 +238,12 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
 // dx = rstd * (g*w - mean(g*w) - xhat * mean(g*w*xhat));  dw += g * xhat;  db += g.   `x` is the LayerNorm INPUT.
 // Each warp walks rows warp, warp + n_warps, ...; parameter gradients are reduced in registers, then one atomic each.
 // If `dx_accum` the result is added to dx (a residual branch already left its gradient there).
+// If `dx_drop` (only with an active `drop` and dx_accum == 0) it also receives mult (.) dx: the gradient that flows
+// into the branch the dropout sits on, while dx itself is the residual branch's.
 __global__ void __launch_bounds__(256) ln_bwd_kernel(const float* __restrict__ x, const float* __restrict__ w,
                                                      const float* __restrict__ g, float* __restrict__ dx,
                                                      float* __restrict__ dw, float* __restrict__ db, int T,
-                                                     int dx_accum) {
+                                                     int dx_accum, float* __restrict__ dx_drop, DropoutSite drop) {
   const int n_warps = gridDim.x * 8;
   const int warp0 = (blockIdx.x * 256 + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   const float w0 = w[lane], w1 = w[lane + 32];
@@ -241,21 +264,31 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const float* __restrict__ x
     const float r0 = rstd * (q0 - m1 - h0 * m2), r1 = rstd * (q1 - m1 - h1 * m2);
     if (dx_accum) { dx[o + lane] += r0; dx[o + lane + 32] += r1; }
     else { dx[o + lane] = r0; dx[o + lane + 32] = r1; }
+    if (dx_drop != nullptr) {
+      dx_drop[o + lane] = r0 * dropout_mult(drop, r, lane);
+      dx_drop[o + lane + 32] = r1 * dropout_mult(drop, r, lane + 32);
+    }
   }
   atomicAdd(dw + lane, aw0); atomicAdd(dw + lane + 32, aw1);
   atomicAdd(db + lane, ab0); atomicAdd(db + lane + 32, ab1);
 }
 
-// scatter-add of the embedding-gather gradient: dTable[id] += g[row]   (tied table: added to the scoring gradient)
+// scatter-add of the embedding-gather gradient: dTable[id] += mult (.) g[row]   (tied table: added to the scoring
+// gradient; mult is the embedding-dropout multiplier, 1 without dropout)
 __global__ void __launch_bounds__(256) scatter_rows_kernel(const void* __restrict__ ids, int id_bytes, int T,
                                                            long long table_rows, const float* __restrict__ g,
-                                                           float* __restrict__ dtable) {
+                                                           float* __restrict__ dtable, DropoutSite drop) {
   const int warp = (blockIdx.x * 256 + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= T) return;
   long long id = load_id(ids, warp, id_bytes);
   if (id < 0 || id >= table_rows) id = 0;
-  atomicAdd(dtable + static_cast<size_t>(id) * D + lane, g[static_cast<size_t>(warp) * D + lane]);
-  atomicAdd(dtable + static_cast<size_t>(id) * D + lane + 32, g[static_cast<size_t>(warp) * D + lane + 32]);
+  float g0 = g[static_cast<size_t>(warp) * D + lane], g1 = g[static_cast<size_t>(warp) * D + lane + 32];
+  if (drop.active()) {
+    g0 *= dropout_mult(drop, warp, lane);
+    g1 *= dropout_mult(drop, warp, lane + 32);
+  }
+  atomicAdd(dtable + static_cast<size_t>(id) * D + lane, g0);
+  atomicAdd(dtable + static_cast<size_t>(id) * D + lane + 32, g1);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -282,19 +315,39 @@ __global__ void __launch_bounds__(256) gamma_bwd_kernel(float* __restrict__ dbu,
   }
   atomicAdd(dgamma + (col >> 1), acc / gm);
 }
-__global__ void __launch_bounds__(256) gelu_fwd_kernel(const float* __restrict__ f, float* __restrict__ a, long long n) {
-  const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
-  if (i < n) { const float z = f[i]; a[i] = 0.5f * z * (1.0f + erff(z * 0.70710678118654752440f)); }
+// f, a, g are [T][FF]; one thread per four consecutive features (one Philox group of the hidden-dropout site)
+LRB_DEVINL float gelu(float z) { return 0.5f * z * (1.0f + erff(z * 0.70710678118654752440f)); }
+LRB_DEVINL float gelu_grad(float z) {   // d/dz [z Phi(z)] = Phi(z) + z phi(z)
+  const float cdf = 0.5f * (1.0f + erff(z * 0.70710678118654752440f));
+  const float pdf = 0.39894228040143267794f * expf(-0.5f * z * z);
+  return cdf + z * pdf;
 }
-// da -> df in place:  d/dz [z Phi(z)] = Phi(z) + z phi(z)
-__global__ void __launch_bounds__(256) gelu_bwd_kernel(const float* __restrict__ f, float* __restrict__ g, long long n) {
+// a = mult (.) GELU(f)
+__global__ void __launch_bounds__(256) gelu_fwd_kernel(const float4* __restrict__ f, float4* __restrict__ a, long long n4,
+                                                       DropoutSite drop) {
   const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
-  if (i < n) {
-    const float z = f[i];
-    const float cdf = 0.5f * (1.0f + erff(z * 0.70710678118654752440f));
-    const float pdf = 0.39894228040143267794f * expf(-0.5f * z * z);
-    g[i] *= cdf + z * pdf;
+  if (i >= n4) return;
+  const float4 z = f[i];
+  float4 v = make_float4(gelu(z.x), gelu(z.y), gelu(z.z), gelu(z.w));
+  if (drop.active()) {
+    const float4 m = dropout_mult4(drop, static_cast<uint32_t>(i / (FF / 4)), static_cast<uint32_t>(i % (FF / 4)));
+    v.x *= m.x; v.y *= m.y; v.z *= m.z; v.w *= m.w;
   }
+  a[i] = v;
+}
+// da -> df in place:  df = mult (.) da (.) GELU'(f)
+__global__ void __launch_bounds__(256) gelu_bwd_kernel(const float4* __restrict__ f, float4* __restrict__ g, long long n4,
+                                                       DropoutSite drop) {
+  const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
+  if (i >= n4) return;
+  const float4 z = f[i];
+  float4 d = g[i];
+  if (drop.active()) {
+    const float4 m = dropout_mult4(drop, static_cast<uint32_t>(i / (FF / 4)), static_cast<uint32_t>(i % (FF / 4)));
+    d.x *= m.x; d.y *= m.y; d.z *= m.z; d.w *= m.w;
+  }
+  d.x *= gelu_grad(z.x); d.y *= gelu_grad(z.y); d.z *= gelu_grad(z.z); d.w *= gelu_grad(z.w);
+  g[i] = d;
 }
 __global__ void __launch_bounds__(256) add_kernel(float* __restrict__ dst, const float* __restrict__ src, long long n) {
   const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
@@ -516,6 +569,30 @@ __global__ void __launch_bounds__(CR) ce_bwd_items_kernel(const float* __restric
   }
 }
 
+// keep[t][j] = 1 if element (t, j) of the site survives (the multiplier the kernels apply is non-zero)
+__global__ void __launch_bounds__(256) dropout_mask_kernel(DropoutSite drop, int T, int width,
+                                                           unsigned char* __restrict__ keep) {
+  const int groups = (width + 3) / 4;
+  const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
+  if (i >= static_cast<long long>(T) * groups) return;
+  const int t = static_cast<int>(i / groups), j4 = static_cast<int>(i % groups);
+  const float4 m = dropout_mult4(drop, static_cast<uint32_t>(t), static_cast<uint32_t>(j4));
+  const float mv[4] = {m.x, m.y, m.z, m.w};
+  for (int k = 0; k < 4 && 4 * j4 + k < width; ++k)
+    keep[static_cast<size_t>(t) * width + 4 * j4 + k] = mv[k] != 0.f ? 1 : 0;
+}
+
+inline bool valid_rate(float p) { return p >= 0.f && p < 1.f; }   // false for NaN
+inline DropoutSite make_site(uint64_t seed, int site, float p) {
+  DropoutSite d;
+  d.key0 = static_cast<uint32_t>(seed & 0xffffffffu);
+  d.key1 = static_cast<uint32_t>(seed >> 32);
+  d.site = static_cast<uint32_t>(site);
+  d.thr = static_cast<uint32_t>(std::floor(static_cast<double>(p) * 4294967296.0));   // < 2^32 for p < 1
+  d.scale = 1.0f / (1.0f - p);
+  return d;
+}
+
 inline size_t al(size_t x) { return (x + 255) & ~static_cast<size_t>(255); }
 inline unsigned blocks_for(long long n, int per) { return static_cast<unsigned>((n + per - 1) / per); }
 
@@ -539,10 +616,37 @@ int lrb_train_step(const void* ids, int id_bytes, const int64_t* labels, int B, 
                    int n_blocks, int64_t ignore_index,
                    float* loss_sum, float* grad_weights, float* grad_table, float* grad_bias, void* workspace,
                    size_t workspace_bytes, void* stream) {
+  return lrb_train_step_dropout(ids, id_bytes, labels, B, L, table_f32, table_rows, bias_f32, weights, params_log,
+                                n_blocks, ignore_index, loss_sum, grad_weights, grad_table, grad_bias, workspace,
+                                workspace_bytes, stream, 0.f, 0.f, 0.f, 0);
+}
+
+int lrb_dropout_mask(uint64_t seed, int site, int T, int width, float p, uint8_t* keep, void* stream) {
   using namespace lrb;
   using namespace lrb::train;
   int rc = check_arch();
   if (rc != LRB_OK) return rc;
+  LRB_REQUIRE(keep != nullptr, "lrb_dropout_mask: null pointer");
+  LRB_REQUIRE(site >= 0 && T > 0 && width > 0, "lrb_dropout_mask: bad shape");
+  LRB_REQUIRE(valid_rate(p), "lrb_dropout_mask: the rate must satisfy 0 <= p < 1");
+  const long long n = static_cast<long long>(T) * ((width + 3) / 4);
+  dropout_mask_kernel<<<blocks_for(n, 256), 256, 0, as_stream(stream)>>>(make_site(seed, site, p), T, width, keep);
+  LRB_CUDA_TRY(cudaGetLastError());
+  return LRB_OK;
+}
+
+int lrb_train_step_dropout(const void* ids, int id_bytes, const int64_t* labels, int B, int L, const float* table_f32,
+                           int64_t table_rows, const float* bias_f32, const float* weights, const float* params_log,
+                           int n_blocks, int64_t ignore_index,
+                           float* loss_sum, float* grad_weights, float* grad_table, float* grad_bias, void* workspace,
+                           size_t workspace_bytes, void* stream, float p_embed, float p_attn, float p_ffn,
+                           uint64_t seed) {
+  using namespace lrb;
+  using namespace lrb::train;
+  int rc = check_arch();
+  if (rc != LRB_OK) return rc;
+  LRB_REQUIRE(valid_rate(p_embed) && valid_rate(p_attn) && valid_rate(p_ffn),
+              "lrb_train_step: dropout rates must satisfy 0 <= p < 1 (got %g, %g, %g)", p_embed, p_attn, p_ffn);
   LRB_REQUIRE(ids && labels && table_f32 && bias_f32 && weights && params_log && loss_sum && grad_weights &&
               grad_table && grad_bias && workspace, "lrb_train_step: null pointer");
   LRB_REQUIRE(B > 0 && L > 0 && n_blocks >= 1 && table_rows > 0 && table_rows < INT_MAX, "lrb_train_step: bad shape");
@@ -583,6 +687,14 @@ int lrb_train_step(const void* ids, int id_bytes, const int64_t* labels, int B, 
   unsigned char* mask = static_cast<unsigned char*>(take(static_cast<size_t>(T)));
   int* err_flag = static_cast<int*>(take(16));
 
+  // dropout sites (model/lru.py): 0 embedding (:57-60); per block i: 1+3i after out_proj (:160), 2+3i the PFFN
+  // hidden (:174), 3+3i after w_2 (:175).  A site with p == 0 is inactive: no Philox, no multiply.
+  const DropoutSite no_drop = make_site(0, 0, 0.f);
+  const DropoutSite drop_embed = make_site(seed, 0, p_embed);
+  auto drop_attn = [&](int i) { return make_site(seed, 1 + 3 * i, p_attn); };
+  auto drop_hidden = [&](int i) { return make_site(seed, 2 + 3 * i, p_ffn); };
+  auto drop_ffn_out = [&](int i) { return make_site(seed, 3 + 3 * i, p_ffn); };
+
   LRB_CUDA_TRY(cudaMemsetAsync(err_flag, 0, 4, st));
   LRB_CUDA_TRY(cudaMemsetAsync(loss_sum, 0, 2 * sizeof(float), st));
   LRB_CUDA_TRY(cudaMemsetAsync(grad_weights, 0, n_w * sizeof(float), st));
@@ -590,37 +702,40 @@ int lrb_train_step(const void* ids, int id_bytes, const int64_t* labels, int B, 
   LRB_CUDA_TRY(cudaMemsetAsync(grad_bias, 0, static_cast<size_t>(rows) * sizeof(float), st));
 
   const unsigned warp_blocks = blocks_for(T, 8);          // one warp per row, 8 warps per CTA
-  auto gemm_nn = [&](const float* A, const float* W, const float* bias, const float* R, float* C, int M, int N, int K) {
+  auto gemm_nn = [&](const float* A, const float* W, const float* bias, const float* R, float* C, int M, int N, int K,
+                     const DropoutSite& drop) {
     dim3 grid(blocks_for(N, GT), blocks_for(M, GT));
-    sgemm_kernel<0><<<grid, 256, 0, st>>>(A, W, bias, R, C, M, N, K, 0);
+    sgemm_kernel<0><<<grid, 256, 0, st>>>(A, W, bias, R, C, M, N, K, 0, drop);
   };
   auto gemm_nt = [&](const float* dY, const float* W, float* dX, int M, int N, int K) {   // dX[M][K] = dY[M][N] W[K][N]^T
     dim3 grid(blocks_for(K, GT), blocks_for(M, GT));
-    sgemm_kernel<1><<<grid, 256, 0, st>>>(dY, W, nullptr, nullptr, dX, M, N, K, 0);
+    sgemm_kernel<1><<<grid, 256, 0, st>>>(dY, W, nullptr, nullptr, dX, M, N, K, 0, no_drop);
   };
   const int m_slice = 1024;
   auto gemm_tn = [&](const float* X, const float* dY, float* dW, float* db, int M, int N, int K) {  // dW[K][N] += X^T dY
     dim3 grid(blocks_for(N, GT), blocks_for(K, GT), blocks_for(M, m_slice));
-    sgemm_kernel<2><<<grid, 256, 0, st>>>(X, dY, nullptr, nullptr, dW, M, N, K, m_slice);
+    sgemm_kernel<2><<<grid, 256, 0, st>>>(X, dY, nullptr, nullptr, dW, M, N, K, m_slice, no_drop);
     if (db != nullptr) colsum_kernel<<<blocks_for(M, m_slice), 256, 0, st>>>(dY, db, M, N, m_slice);
   };
   auto ew_blocks = [&](long long n) { return blocks_for(n, 256); };
 
   // =========================== forward (every intermediate the backward needs is kept) ===========================
-  gather_kernel<<<warp_blocks, 256, 0, st>>>(ids, id_bytes, T, L, table_f32, table_rows, gath, mask, err_flag);
+  gather_kernel<<<warp_blocks, 256, 0, st>>>(ids, id_bytes, T, L, table_f32, table_rows, gath, mask, err_flag, drop_embed);
   ln_fwd_kernel<<<warp_blocks, 256, 0, st>>>(gath, weights + OFF_EMB_LN_W, weights + OFF_EMB_LN_B, x0, T);
   const float* x_in = x0;
   for (int i = 0; i < n_blocks; ++i) {
     const float* wb = weights + OFF_BLOCKS + static_cast<size_t>(i) * BLOCK_FLOATS;
-    gemm_nn(x_in, wb + B_WIN_T, wb + B_BIN, nullptr, sv[i].bu, T, H2, D);
+    gemm_nn(x_in, wb + B_WIN_T, wb + B_BIN, nullptr, sv[i].bu, T, H2, D, no_drop);
     gamma_fwd_kernel<<<ew_blocks(static_cast<long long>(T) * H2), 256, 0, st>>>(sv[i].bu, wb + B_GAMMA, static_cast<long long>(T) * H2);
     scan_fwd_kernel<<<B, 128, 0, st>>>(reinterpret_cast<const float2*>(sv[i].bu), reinterpret_cast<float2*>(sv[i].h), mask,
                                        wb + B_LAM_RE, wb + B_LAM_IM, L);
-    gemm_nn(sv[i].h, wb + B_WOUT_T, wb + B_BOUT, x_in, sv[i].pre1, T, D, H2);
+    gemm_nn(sv[i].h, wb + B_WOUT_T, wb + B_BOUT, x_in, sv[i].pre1, T, D, H2, drop_attn(i));
     ln_fwd_kernel<<<warp_blocks, 256, 0, st>>>(sv[i].pre1, wb + B_LN1_W, wb + B_LN1_B, sv[i].y, T);
-    gemm_nn(sv[i].y, wb + B_W1_T, wb + B_B1, nullptr, sv[i].f1, T, FF, D);
-    gelu_fwd_kernel<<<ew_blocks(static_cast<long long>(T) * FF), 256, 0, st>>>(sv[i].f1, sv[i].a, static_cast<long long>(T) * FF);
-    gemm_nn(sv[i].a, wb + B_W2_T, wb + B_B2, sv[i].y, sv[i].pre2, T, D, FF);
+    gemm_nn(sv[i].y, wb + B_W1_T, wb + B_B1, nullptr, sv[i].f1, T, FF, D, no_drop);
+    gelu_fwd_kernel<<<ew_blocks(static_cast<long long>(T) * FF / 4), 256, 0, st>>>(
+        reinterpret_cast<const float4*>(sv[i].f1), reinterpret_cast<float4*>(sv[i].a), static_cast<long long>(T) * FF / 4,
+        drop_hidden(i));
+    gemm_nn(sv[i].a, wb + B_W2_T, wb + B_B2, sv[i].y, sv[i].pre2, T, D, FF, drop_ffn_out(i));
     ln_fwd_kernel<<<warp_blocks, 256, 0, st>>>(sv[i].pre2, wb + B_LN2_W, wb + B_LN2_B, sv[i].out, T);
     x_in = sv[i].out;
   }
@@ -651,19 +766,29 @@ int lrb_train_step(const void* ids, int id_bytes, const int64_t* labels, int B, 
     const float* xin = i == 0 ? x0 : sv[i - 1].out;
     float* dpre2 = g64b;
     float* dy = g64c;
-    // out = LN2(pre2), pre2 = a W2 + b2 + y
-    ln_bwd_kernel<<<148, 256, 0, st>>>(sv[i].pre2, wb + B_LN2_W, dx, dpre2, gb + B_LN2_W, gb + B_LN2_B, T, 0);
-    gemm_tn(sv[i].a, dpre2, gb + B_W2_T, gb + B_B2, T, D, FF);
-    gemm_nt(dpre2, wb + B_W2_T, g256a, T, D, FF);                       // da [T][256]
-    gelu_bwd_kernel<<<ew_blocks(static_cast<long long>(T) * FF), 256, 0, st>>>(sv[i].f1, g256a, static_cast<long long>(T) * FF);   // -> df1
+    // out = LN2(pre2), pre2 = mult (.) (a W2 + b2) + y.  With dropout the W2 branch takes mult (.) dpre2, written
+    // to g64c (free until dy is produced below); the residual branch takes dpre2 as it is.
+    const DropoutSite d_out = drop_ffn_out(i);
+    float* dpre2_w = d_out.active() ? g64c : dpre2;
+    ln_bwd_kernel<<<148, 256, 0, st>>>(sv[i].pre2, wb + B_LN2_W, dx, dpre2, gb + B_LN2_W, gb + B_LN2_B, T, 0,
+                                       d_out.active() ? dpre2_w : nullptr, d_out);
+    gemm_tn(sv[i].a, dpre2_w, gb + B_W2_T, gb + B_B2, T, D, FF);
+    gemm_nt(dpre2_w, wb + B_W2_T, g256a, T, D, FF);                     // da [T][256]
+    gelu_bwd_kernel<<<ew_blocks(static_cast<long long>(T) * FF / 4), 256, 0, st>>>(
+        reinterpret_cast<const float4*>(sv[i].f1), reinterpret_cast<float4*>(g256a), static_cast<long long>(T) * FF / 4,
+        drop_hidden(i));                                                // -> df1
     gemm_tn(sv[i].y, g256a, gb + B_W1_T, gb + B_B1, T, FF, D);
     gemm_nt(g256a, wb + B_W1_T, dy, T, FF, D);                          // dy from the W1 branch
     add_kernel<<<ew_blocks(static_cast<long long>(T) * D), 256, 0, st>>>(dy, dpre2, static_cast<long long>(T) * D);   // + residual branch
-    // y = LN1(pre1), pre1 = h W_out + b_out + x_in
+    // y = LN1(pre1), pre1 = mult (.) (h W_out + b_out) + x_in.  The masked copy goes to g64a: dx was consumed by the
+    // LN2 backward and is written again only by the in_proj branch below.
     float* dpre1 = g64b;
-    ln_bwd_kernel<<<148, 256, 0, st>>>(sv[i].pre1, wb + B_LN1_W, dy, dpre1, gb + B_LN1_W, gb + B_LN1_B, T, 0);
-    gemm_tn(sv[i].h, dpre1, gb + B_WOUT_T, gb + B_BOUT, T, D, H2);
-    gemm_nt(dpre1, wb + B_WOUT_T, g256b, T, D, H2);                     // dh [T][256]
+    const DropoutSite d_attn = drop_attn(i);
+    float* dpre1_w = d_attn.active() ? g64a : dpre1;
+    ln_bwd_kernel<<<148, 256, 0, st>>>(sv[i].pre1, wb + B_LN1_W, dy, dpre1, gb + B_LN1_W, gb + B_LN1_B, T, 0,
+                                       d_attn.active() ? dpre1_w : nullptr, d_attn);
+    gemm_tn(sv[i].h, dpre1_w, gb + B_WOUT_T, gb + B_BOUT, T, D, H2);
+    gemm_nt(dpre1_w, wb + B_WOUT_T, g256b, T, D, H2);                   // dh [T][256]
     scan_bwd_kernel<<<B, 128, 0, st>>>(reinterpret_cast<float2*>(g256b), reinterpret_cast<const float2*>(sv[i].h), mask,
                                        wb + B_LAM_RE, wb + B_LAM_IM, gb + B_LAM_RE, gb + B_LAM_IM, L);        // -> dbu
     gamma_bwd_kernel<<<blocks_for(T, 256), 256, 0, st>>>(g256b, sv[i].bu, wb + B_GAMMA, gb + B_GAMMA, T, 256);   // -> d(pre-gamma)
@@ -672,10 +797,10 @@ int lrb_train_step(const void* ids, int id_bytes, const int64_t* labels, int B, 
     add_kernel<<<ew_blocks(static_cast<long long>(T) * D), 256, 0, st>>>(dx, dpre1, static_cast<long long>(T) * D);   // + residual branch
     params_log_grad_kernel<<<1, 128, 0, st>>>(gb, wb, params_log + static_cast<size_t>(i) * 3 * LRB_H);
   }
-  // x0 = LN_e(E[id])
+  // x0 = LN_e(mult (.) E[id]): gath holds the dropped row, so the LayerNorm backward is unchanged
   ln_bwd_kernel<<<148, 256, 0, st>>>(gath, weights + OFF_EMB_LN_W, dx, g64b, grad_weights + OFF_EMB_LN_W,
-                                     grad_weights + OFF_EMB_LN_B, T, 0);
-  scatter_rows_kernel<<<warp_blocks, 256, 0, st>>>(ids, id_bytes, T, table_rows, g64b, grad_table);
+                                     grad_weights + OFF_EMB_LN_B, T, 0, nullptr, no_drop);
+  scatter_rows_kernel<<<warp_blocks, 256, 0, st>>>(ids, id_bytes, T, table_rows, g64b, grad_table, drop_embed);
   LRB_CUDA_TRY(cudaGetLastError());
   // left-padding check (one 4-byte read back: the step's result is meaningless otherwise)
   int err = 0;

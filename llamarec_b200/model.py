@@ -42,20 +42,28 @@ def _on_model_device(fn):
 
 class _TrainStep(torch.autograd.Function):
     """loss = CrossEntropyLoss(ignore_index)(model(x).view(-1, N+1), labels.view(-1)) with a backward: ONE call of
-    lrb_train_step computes the loss and the gradient of every parameter (forward activations never leave the
-    library's workspace); backward() hands the stored gradients to autograd, scaled by the incoming gradient.
-    Inputs after (model, x, labels, ignore_index) are the model's parameters in named_parameters() order."""
+    lrb_train_step (lrb_train_step_dropout with dropout) computes the loss and the gradient of every parameter
+    (forward activations never leave the library's workspace); backward() hands the stored gradients to autograd,
+    scaled by the incoming gradient.
+    `dropout` is (p_embed, p_attn, p_ffn, seed) or None.  Inputs after (model, x, labels, ignore_index, dropout) are
+    the model's parameters in named_parameters() order."""
 
     @staticmethod
-    def forward(ctx, model, x, labels, ignore_index, *params):
-        loss, grads = model._train_step(x, labels, ignore_index)
+    def forward(ctx, model, x, labels, ignore_index, dropout, *params):
+        loss, grads = model._train_step(x, labels, ignore_index, dropout)
         ctx.grads = grads
         return loss
 
     @staticmethod
     def backward(ctx, grad_out):
         out = tuple(None if g is None else g * grad_out for g in ctx.grads)
-        return (None, None, None, None) + out
+        return (None, None, None, None, None) + out
+
+
+def _draw_seed(generator: Optional[torch.Generator]) -> int:
+    """One 64-bit draw from a CPU generator (torch's default one if None): torch.manual_seed reproduces it."""
+    v = torch.randint(-(1 << 63), (1 << 63) - 1, (), dtype=torch.int64, generator=generator)
+    return int(v) & 0xFFFF_FFFF_FFFF_FFFF
 
 
 class _Container(nn.Module):
@@ -83,6 +91,9 @@ class LRURec(nn.Module):
         n_blocks = int(getattr(args, "bert_num_blocks", 2) or 2)
         vocab = int(args.num_items) + 1
         self.num_items = int(args.num_items)
+        # train-mode dropout rates of model/lru.py:47-52,93-97 (used by ce_loss(..., dropout=True) only)
+        self.bert_dropout = float(getattr(args, "bert_dropout", 0.0) or 0.0)
+        self.bert_attn_dropout = float(getattr(args, "bert_attn_dropout", 0.0) or 0.0)
 
         self.embedding = _Container()
         self.embedding.token = nn.Embedding(vocab, d)
@@ -137,7 +148,8 @@ class LRURec(nn.Module):
 
     @_on_model_device
     def forward(self, x: torch.Tensor) -> torch.Tensor:
-        """model/lru.py:38-41 -- scores at every position, [B, L, N+1] fp32 (exact fp32 scoring)."""
+        """model/lru.py:38-41 -- scores at every position, [B, L, N+1] fp32 (exact fp32 scoring).  Eval semantics in
+        either mode: no dropout (only ce_loss(..., dropout=True) applies it)."""
         hidden = self.hidden_states(x)
         B, L, _ = hidden.shape
         rows = self.row_end - self.row_begin
@@ -156,7 +168,8 @@ class LRURec(nn.Module):
 
     @_on_model_device
     def hidden_states(self, x: torch.Tensor) -> torch.Tensor:
-        """Encoder output at every position, [B, L, 64] (model/lru.py:73-83)."""
+        """Encoder output at every position, [B, L, 64] (model/lru.py:73-83).  Eval semantics in either mode: no
+        dropout."""
         return self._encode(x, all_positions=True)[0]
 
     @_on_model_device
@@ -173,7 +186,8 @@ class LRURec(nn.Module):
                  u_bf16: Optional[torch.Tensor] = None, merge: bool = True,
                  packed_out: Optional[torch.Tensor] = None, seq: Optional[dict] = None,
                  scatter: Optional[dict] = None, packed_layout: str = "planes") -> Dict[str, torch.Tensor]:
-        """encode -> catalogue score -> (history mask) -> top-k -> (metrics), all on device.
+        """encode -> catalogue score -> (history mask) -> top-k -> (metrics), all on device.  Eval semantics in either
+        mode: no dropout.
 
         Replaces calculate_metrics / the per-user loop of generate_candidates (trainer/lru.py:30-42,
         61-88).  Returns ids/scores [B, k] sorted by (score desc, id asc); with `labels` also
@@ -237,16 +251,40 @@ class LRURec(nn.Module):
         out["u"] = u
         return out
 
-    @_on_model_device
     def ce_loss(self, x: torch.Tensor, labels: torch.Tensor, ignore_index: int = 0,
-                return_row_loss: bool = False):
+                return_row_loss: bool = False, dropout: bool = False,
+                generator: Optional[torch.Generator] = None):
         """The train-step loss, `CrossEntropyLoss(ignore_index=0)(model(x).view(-1, N+1), labels.view(-1))`
         (trainer/lru.py:20-28), without the [B*L, N+1] logits.  With autograd enabled (and no per-row losses asked
         for) the result carries a backward: `loss.backward()` fills `.grad` of every parameter from ONE fused
         forward + backward pass (lrb_train_step), like trainer/base.py:107-111 does through torch's autograd.
-        Under torch.no_grad() it is the forward value only (lrb_ce_loss_fwd).  Dropout is the identity in both."""
+        Under torch.no_grad() it is the forward value only (lrb_ce_loss_fwd).
+
+        Dropout is active when `dropout and self.training` (like nn.Dropout): the reference's four train-mode sites
+        (model/lru.py:57-60,160,174-175) at rates bert_dropout (embedding, PFFN) and bert_attn_dropout (after
+        out_proj).  The masks are counter-based (include/llamarec_b200.h, lrb_train_step_dropout) and keyed by one
+        64-bit draw per call from `generator`, a CPU torch.Generator (torch's default one if None), so
+        torch.manual_seed reproduces a run; they are not torch's own dropout masks.  Active dropout needs the
+        backward path: under torch.no_grad() or with return_row_loss it raises ValueError.  In eval mode, or with
+        dropout=False, nothing changes."""
+        rates = None
+        if dropout and self.training:
+            rates = (self.bert_dropout, self.bert_attn_dropout, self.bert_dropout)
+            if not all(0.0 <= p < 1.0 for p in rates):     # False for NaN as well
+                raise ValueError(f"dropout rates must satisfy 0 <= p < 1, got bert_dropout={self.bert_dropout}, "
+                                 f"bert_attn_dropout={self.bert_attn_dropout}")
+            if return_row_loss or not torch.is_grad_enabled():
+                raise ValueError("dropout=True in training mode runs the fused train step: it has no per-row losses "
+                                 "and no value-only path (call it with autograd enabled, or use model.eval())")
+        return self._ce_loss(x, labels, ignore_index, return_row_loss, rates, generator)
+
+    @_on_model_device
+    def _ce_loss(self, x, labels, ignore_index, return_row_loss, rates, generator):
+        if rates is not None:
+            drop = (float(rates[0]), float(rates[1]), float(rates[2]), _draw_seed(generator))
+            return _TrainStep.apply(self, x, labels, int(ignore_index), drop, *[p for _, p in self.named_parameters()])
         if torch.is_grad_enabled() and not return_row_loss and any(p.requires_grad for p in self.parameters()):
-            return _TrainStep.apply(self, x, labels, int(ignore_index), *[p for _, p in self.named_parameters()])
+            return _TrainStep.apply(self, x, labels, int(ignore_index), None, *[p for _, p in self.named_parameters()])
         with torch.no_grad():
             return self._ce_loss_value(x, labels, ignore_index, return_row_loss)
 
@@ -273,8 +311,9 @@ class LRURec(nn.Module):
         return (loss, row_loss.view(B, L)) if return_row_loss else loss
 
     @torch.no_grad()
-    def _train_step(self, x: torch.Tensor, labels: torch.Tensor, ignore_index: int = 0):
-        """-> (loss, [gradient per parameter in named_parameters() order]) from one lrb_train_step call."""
+    def _train_step(self, x: torch.Tensor, labels: torch.Tensor, ignore_index: int = 0, dropout=None):
+        """-> (loss, [gradient per parameter in named_parameters() order]) from one lrb_train_step call, or one
+        lrb_train_step_dropout call when `dropout` = (p_embed, p_attn, p_ffn, seed) is given."""
         lib = _lib.load()
         if self.row_begin != 0 or self.row_end != self.num_items + 1:
             raise RuntimeError("the train step needs the whole item table on this device (no row shard)")
@@ -297,10 +336,14 @@ class LRURec(nn.Module):
         g_table = torch.empty(rows, 64, dtype=torch.float32, device=dev)
         g_bias = torch.empty(rows, dtype=torch.float32, device=dev)
         acc = torch.empty(2, dtype=torch.float32, device=dev)
-        _lib.check(lib.lrb_train_step(_lib.ptr(x), x.element_size(), _lib.ptr(labels), B, L, _lib.ptr(c["table_f32"]), rows,
-                                      _lib.ptr(bias), _lib.ptr(c["blob"]), _lib.ptr(params_log), n_blocks,
-                                      int(ignore_index), _lib.ptr(acc), _lib.ptr(g_w), _lib.ptr(g_table), _lib.ptr(g_bias),
-                                      _lib.ptr(ws), ws_bytes, _lib.stream_handle()))
+        step_args = (_lib.ptr(x), x.element_size(), _lib.ptr(labels), B, L, _lib.ptr(c["table_f32"]), rows,
+                     _lib.ptr(bias), _lib.ptr(c["blob"]), _lib.ptr(params_log), n_blocks, int(ignore_index),
+                     _lib.ptr(acc), _lib.ptr(g_w), _lib.ptr(g_table), _lib.ptr(g_bias), _lib.ptr(ws), ws_bytes,
+                     _lib.stream_handle())
+        if dropout is None:
+            _lib.check(lib.lrb_train_step(*step_args))
+        else:
+            _lib.check(lib.lrb_train_step_dropout(*step_args, *dropout))
         loss = acc[0] / acc[1]
         named = unpack_encoder_grads(g_w, n_blocks)
         named["embedding.token.weight"] = g_table

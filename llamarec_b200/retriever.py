@@ -30,11 +30,12 @@ class LRURetriever:
         return [x.to(self.device, non_blocking=True) for x in batch]
 
     # ---- trainer/lru.py:22-28 -------------------------------------------------------------------
-    def calculate_loss(self, batch) -> torch.Tensor:
+    def calculate_loss(self, batch, dropout: bool = False) -> torch.Tensor:
         """Training loss of one batch; with autograd enabled `loss.backward()` fills the parameters' gradients
-        (fused forward + backward train step, see LRURec.ce_loss)."""
+        (fused forward + backward train step, see LRURec.ce_loss).  `dropout=True` applies the reference's
+        train-mode dropout while the model is in training mode (LRURec.ce_loss)."""
         seqs, labels = batch
-        return self.model.ce_loss(seqs, labels)
+        return self.model.ce_loss(seqs, labels, dropout=dropout)
 
     # ---- trainer/lru.py:30-42 -------------------------------------------------------------------
     def calculate_metrics(self, batch, exclude_history: bool = True) -> Dict[str, float]:
