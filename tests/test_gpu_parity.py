@@ -359,25 +359,27 @@ def test_games_shaped_batch_2048_against_oracle(games_model):
 
 
 def test_virtual_rank_sharding_is_exact(games_model):
-    """Shard -> local top-k -> concatenate -> merge on one device equals the unsharded result exactly."""
+    """Shard -> local top-k -> concatenate -> merge on one device equals the unsharded result exactly, for k = 20 and
+    k = 50 (the K <= 50 kernel and the default metric_ks)."""
     m, sd, cfg = games_model
     ids, _ = synth.make_sequences(cfg, num_users=300, seed=7)
     x = ids.cuda()
-    for prec in ("fp32", "bf16"):
-        m.set_row_shard(0, cfg.num_items + 1)
-        full = m.retrieve(x, k=20, precision=prec)
-        u = full["u"]
-        parts_s, parts_i = [], []
-        R = 4
-        per = (cfg.num_items + 1 + R - 1) // R
-        for r in range(R):
-            m.set_row_shard(r * per, min((r + 1) * per, cfg.num_items + 1))
-            loc = m.retrieve(x, k=20, precision=prec, u=u)
-            parts_s.append(loc["scores"].clone())
-            parts_i.append(loc["ids"].clone())
-        m.set_row_shard(0, cfg.num_items + 1)
-        merged = merge_lists(torch.stack(parts_s), torch.stack(parts_i), None, k_out=20, layout="list_major")
-        assert torch.equal(merged["ids"], full["ids"]) and torch.equal(merged["scores"], full["scores"])
+    for k in (20, 50):
+        for prec in ("fp32", "bf16"):
+            m.set_row_shard(0, cfg.num_items + 1)
+            full = m.retrieve(x, k=k, precision=prec)
+            u = full["u"]
+            parts_s, parts_i = [], []
+            R = 4
+            per = (cfg.num_items + 1 + R - 1) // R
+            for r in range(R):
+                m.set_row_shard(r * per, min((r + 1) * per, cfg.num_items + 1))
+                loc = m.retrieve(x, k=k, precision=prec, u=u)
+                parts_s.append(loc["scores"].clone())
+                parts_i.append(loc["ids"].clone())
+            m.set_row_shard(0, cfg.num_items + 1)
+            merged = merge_lists(torch.stack(parts_s), torch.stack(parts_i), None, k_out=k, layout="list_major")
+            assert torch.equal(merged["ids"], full["ids"]) and torch.equal(merged["scores"], full["scores"]), (k, prec)
 
 
 def test_batches_beyond_one_tile_per_sm_are_chunked(games_model):
