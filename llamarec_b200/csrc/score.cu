@@ -6,33 +6,14 @@
 #include "api_util.h"
 #include "score_topk_tc.cuh"
 
-#ifndef LRB_RESTART_TILES
-#define LRB_RESTART_TILES 150.0   // cost of one streaming top-K (re)start, in item tiles (see decompose())
-#endif
-#ifndef LRB_CAP_DIV
-#define LRB_CAP_DIV 1   // users per scoring launch = (SM pairs / LRB_CAP_DIV) x 256
-#endif
-#ifndef LRB_NS_PAIR
-#define LRB_NS_PAIR 4   // TMA stages of the K <= 20 CTA-pair kernel (20 KB each)
-#endif
-
 #include <cuda.h>
 #include <climits>
 #include <cmath>
-#include <cstdlib>
-
-// Developer-harness knobs (tools/tc_check is built with -DLRB_DEBUG_MODES; the library never is).
-#ifdef LRB_DEBUG_MODES
-static int g_debug_cap_div = 0;
-static double g_debug_restart_tiles = -1.0;
-extern "C" void lrb_debug_set_cap_div(int v) { g_debug_cap_div = v; }
-extern "C" void lrb_debug_set_restart_tiles(double v) { g_debug_restart_tiles = v; }
-#else
-static const int g_debug_cap_div = 0;
-static const double g_debug_restart_tiles = -1.0;
-#endif
 
 namespace lrb {
+
+constexpr double RESTART_TILES = 150.0;   // cost of one streaming top-K (re)start, in item tiles (see decompose())
+constexpr int NS_PAIR = 4;                // TMA stages of the K <= 20 CTA-pair kernel (20 KB each)
 
 // ============================================================================================
 // fp32 path.  Thread = user row (state in registers), CTA = 128 rows, item chunks of 64 rows
@@ -373,6 +354,27 @@ inline long long select_block_users(long long rows, size_t bytes) {
   return u / ROWS * ROWS;
 }
 
+// dense fp32 scores out[M][ld] (columns < rows) of the user states x [M][64] against table [rows][64] + bias_pad
+int launch_dense(const float* x, const float* table, const float* bias_pad, int M, int rows, float* out,
+                 long long ld, int sms, cudaStream_t st) {
+  Params p;
+  p.u = x;
+  p.table = table;
+  p.bias_pad = bias_pad;
+  p.B = M; p.rows = rows; p.row_offset = 0; p.K = 0;
+  p.excl_sorted = nullptr; p.excl_bloom = nullptr; p.excl_stride = 0;
+  p.part_scores = nullptr; p.part_ids = nullptr; p.part_cnt = nullptr; p.slots = 0;
+  p.dense_out = out; p.dense_ld = ld;
+  const int splits = splits_for(M, rows, sms, 4);   // dense variant: 49 KB / 96 registers -> 4 CTAs per SM
+  const size_t smem = (IT * D + IT) * 4 + static_cast<size_t>(ROWS) * (IT + 1) * 4;
+  auto kern = score_f32_kernel<true>;
+  LRB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  dim3 grid(static_cast<unsigned>((static_cast<long long>(M) + ROWS - 1) / ROWS), splits);
+  kern<<<grid, ROWS, smem, st>>>(p);
+  LRB_CUDA_TRY(cudaGetLastError());
+  return LRB_OK;
+}
+
 }  // namespace f32
 
 // ============================================================================================
@@ -411,7 +413,7 @@ Decomp decompose(int B, long long rows, int units, int bm = tc::BM) {
     // and 5.44 / 5.40 / 5.52 / 5.58 ms at 32768 x 1.25M, hence R0 = 150).  A full-stream CTA starts once, a
     // shared-stream CTA about m_tiles / rem + 1/2 times:
     //   (n - y) / s + R0  =  m * y / rem + (m / rem + 1/2) * R0
-    double R0 = g_debug_restart_tiles >= 0 ? g_debug_restart_tiles : LRB_RESTART_TILES;
+    double R0 = RESTART_TILES;
     if (R0 > d.n_tiles / (8.0 * d.s_full)) R0 = d.n_tiles / (8.0 * d.s_full);   // short segments: a start costs less
     const double m_over_rem = static_cast<double>(d.m_tiles) / d.rem;
     double y = (static_cast<double>(d.n_tiles) / d.s_full + R0 * (0.5 - m_over_rem)) / (1.0 / d.s_full + m_over_rem);
@@ -422,7 +424,7 @@ Decomp decompose(int B, long long rows, int units, int bm = tc::BM) {
     d.full_tiles = d.n_tiles - d.y_tiles;
   }
   d.grid = d.s_full * d.m_tiles + d.rem;
-  d.slots = tc::SLOT_PARTS * (d.s_full + (d.rem > 0 ? 2 : 0));
+  d.slots = tc::PARTS * (d.s_full + (d.rem > 0 ? 2 : 0));
   return d;
 }
 
@@ -439,22 +441,13 @@ inline int users_per_launch(int B, int sms) {
   // streaming top-K restarts once (two slots per user, union bound with c = ceil(K/2) <= 12).  Measured on B200,
   // 32768 users x 1.25M rows (one rank's call of the 8-GPU data-parallel step): launches of 9472 users (two full
   // streams, c = 5) 5.58 ms, of 18944 users 5.38 ms.
-  int cap_tiles = units / (g_debug_cap_div > 0 ? g_debug_cap_div : LRB_CAP_DIV);   // pair tiles per launch
-  if (cap_tiles < 1) cap_tiles = 1;
-  const int cap = cap_tiles * 2 * tc::BM;
+  const int cap = units * 2 * tc::BM;
   return B <= cap ? B : cap;
 }
 
 // CTA pairs (tcgen05 cta_group::2) whenever a launch has more than one user tile: the pair shares every
 // item tile, which halves the shared-memory operand traffic and the L2 -> SM traffic per MMA.
-inline int cta_group_for(int B, int sms) {
-  static const int forced = [] {
-    const char* e = std::getenv("LRB_SCORE_CTA_GROUP");   // tuning knob: "1" keeps every launch on single CTAs
-    return e ? std::atoi(e) : 0;
-  }();
-  if (forced == 1) return 1;
-  return (B > tc::BM && sms >= 2) ? 2 : 1;
-}
+inline int cta_group_for(int B, int sms) { return (B > tc::BM && sms >= 2) ? 2 : 1; }
 
 Decomp decompose_launch(int B, long long rows, int sms) {
   const int cg = cta_group_for(B, sms);
@@ -521,20 +514,16 @@ int make_tmap_bias_blocks(CUtensorMap* out, const void* ptr, unsigned long long 
   return LRB_OK;
 }
 
-// Epilogue warps of the kernel variant that serves list length K: 16 (four 64-column parts per tile) for K <= 20,
-// 8 (two 128-column parts) for the longer lists, whose per-thread candidate sets leave no room for 512 threads.
-inline int epilogue_warps_for(int K) { return K <= 20 ? LRB_EW20 : 8; }
-
 // `grid` counts MMA engines: CTAs for CG == 1, CTA pairs (clusters of 2) for CG == 2.
-template <int KMAX, int NS, bool kDense, int CG, int EW, int PROBE = 0, int CMAX = tc::MAX_C_SHARE_SMALL>
+template <int KMAX, int NS, bool kDense, int CG, int CMAX = tc::MAX_C_SHARE_SMALL>
 int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tbias, const tc::ScoreParams& p,
               int grid, cudaStream_t st, bool overlap_prev = false) {
-  using L = tc::SmemLayout<KMAX, NS, CG, EW>;
-  auto kern = tc::score_topk_tc_kernel<KMAX, NS, kDense, CG, EW, CMAX, PROBE>;
+  using L = tc::SmemLayout<KMAX, NS, CG>;
+  auto kern = tc::score_topk_tc_kernel<KMAX, NS, kDense, CG, CMAX>;
   LRB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kAlloc));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid * CG));
-  cfg.blockDim = dim3(128 + EW * 32);
+  cfg.blockDim = dim3(128 + tc::EPI_WARPS * 32);
   cfg.dynamicSmemBytes = L::kAlloc;
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
@@ -560,24 +549,6 @@ int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& t
 
 }  // namespace
 }  // namespace lrb
-
-#ifdef LRB_DEBUG_MODES
-static int g_debug_mode = 0;
-static int g_debug_scout = -1;
-static int g_debug_pair_drain = 1;
-static int g_debug_overlap = 1;
-static long long* g_debug_probe_out = nullptr;
-extern "C" void lrb_debug_set_probe_out(long long* p) { g_debug_probe_out = p; }
-extern "C" void lrb_debug_set_overlap(int v) { g_debug_overlap = v; }
-extern "C" void lrb_debug_set_pair_drain(int v) { g_debug_pair_drain = v; }
-extern "C" void lrb_debug_set_scout(int t) { g_debug_scout = t; }
-extern "C" void lrb_debug_set_score_mode(int m) { g_debug_mode = m; }
-#else
-static const int g_debug_scout = -1;
-static const int g_debug_pair_drain = 1;
-static const int g_debug_overlap = 1;
-static long long* const g_debug_probe_out = nullptr;
-#endif
 
 extern "C" {
 
@@ -607,7 +578,7 @@ static size_t gslots_bytes(int B) {
   if (sms <= 0) sms = 148;
   size_t m_tiles = (static_cast<size_t>(B) + lrb::tc::BM - 1) / lrb::tc::BM;
   if (m_tiles > static_cast<size_t>(sms)) m_tiles = static_cast<size_t>(sms);   // one launch never covers more
-  const size_t max_slots = lrb::tc::SLOT_PARTS * (static_cast<size_t>(sms) / m_tiles + 2);
+  const size_t max_slots = lrb::tc::PARTS * (static_cast<size_t>(sms) / m_tiles + 2);
   // (+1 tile: CTA pairs pad the user tiles to an even count)
   return ((m_tiles + 1) * lrb::tc::BM * max_slots * sizeof(int) + 255) & ~static_cast<size_t>(255);
 }
@@ -626,7 +597,9 @@ static size_t gslots_chunk_bytes(int cap) {
 static size_t ring_bytes() {
   int sms = lrb::device_sm_count();
   if (sms <= 0) sms = 148;
-  return static_cast<size_t>(sms) * 512 * lrb::tc::RING_GROUPS * lrb::tc::RING_REC_BYTES;   // up to 16 epilogue warps
+  // 512 rings per SM, twice the kernel's 256 epilogue threads; the size also sets the user block of the fp32 select
+  // path (f32_select_users), so it is part of the dispatch
+  return static_cast<size_t>(sms) * 512 * lrb::tc::RING_GROUPS * lrb::tc::RING_REC_BYTES;
 }
 
 // layout: [n_chunks x union-bound slots of one chunk][2 x candidate rings (consecutive chunk launches overlap)]
@@ -660,23 +633,11 @@ int lrb_score_topk(const void* u, const void* table, const float* bias_pad, cons
     const long long blk = f32_select_users(rows);
     const long long ld = (rows + 3) / 4 * 4;
     float* dense = static_cast<float*>(scratch);
-    const size_t smem = (f32::IT * f32::D + f32::IT) * 4 + static_cast<size_t>(f32::ROWS) * (f32::IT + 1) * 4;
-    auto dkern = f32::score_f32_kernel<true>;
-    LRB_CUDA_TRY(cudaFuncSetAttribute(dkern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
     for (long long b0 = 0; b0 < B; b0 += blk) {
       const int nb = static_cast<int>(B - b0 < blk ? B - b0 : blk);
-      f32::Params p;
-      p.u = static_cast<const float*>(u) + b0 * f32::D;
-      p.table = static_cast<const float*>(table);
-      p.bias_pad = bias_pad;
-      p.B = nb; p.rows = static_cast<int>(rows); p.row_offset = 0; p.K = 0;
-      p.excl_sorted = nullptr; p.excl_bloom = nullptr; p.excl_stride = 0;
-      p.part_scores = nullptr; p.part_ids = nullptr; p.part_cnt = nullptr; p.slots = 0;
-      p.dense_out = dense; p.dense_ld = ld;
-      const int splits = f32::splits_for(nb, rows, sms, 4);   // dense variant: 49 KB / 96 registers -> 4 CTAs per SM
-      dim3 grid(static_cast<unsigned>((nb + f32::ROWS - 1) / f32::ROWS), splits);
-      dkern<<<grid, f32::ROWS, smem, st>>>(p);
-      LRB_CUDA_TRY(cudaGetLastError());
+      rc = f32::launch_dense(static_cast<const float*>(u) + b0 * f32::D, static_cast<const float*>(table), bias_pad,
+                             nb, static_cast<int>(rows), dense, ld, sms, st);
+      if (rc != LRB_OK) return rc;
       f32::SelParams sp;
       sp.dense = dense; sp.ld = ld; sp.nb = nb; sp.b0 = static_cast<int>(b0);
       sp.rows = static_cast<int>(rows); sp.row_offset = static_cast<int>(row_offset); sp.K = K;
@@ -750,12 +711,10 @@ int lrb_score_topk(const void* u, const void* table, const float* bias_pad, cons
     p.excl_stride = excl_stride;
     p.gslots = reinterpret_cast<int*>(static_cast<uint8_t*>(scratch) + chunk_idx * gs_chunk);
     p.gstride = d.slots;
-    p.pair_drain = g_debug_pair_drain;
     p.ring = static_cast<uint8_t*>(scratch) + n_chunks * gs_chunk + (chunk_idx & 1) * ring_bytes();
     {
       // entries each of the PARTS*s_full full-stream threads of a user must hold for the union bound
-      const int parts = epilogue_warps_for(K) / 4;
-      const int c = d.s_full > 0 ? (K + parts * d.s_full - 1) / (parts * d.s_full) : 99;
+      const int c = d.s_full > 0 ? (K + tc::PARTS * d.s_full - 1) / (tc::PARTS * d.s_full) : 99;
       // (the K <= 20 CTA-pair kernel also exists with room for c <= 12: one full stream per user)
       const int c_max = (cg == 2 && K <= 20) ? tc::MAX_C_SHARE_LARGE : tc::MAX_C_SHARE_SMALL;
       p.c_share = c <= c_max ? c : 0;
@@ -764,49 +723,28 @@ int lrb_score_topk(const void* u, const void* table, const float* bias_pad, cons
       // (32 tiles on long segments: A/B on B200, 32768 users x 1.25M rows -- one stream per user, c = 10 --
       // 16 / 32 / 64 scout tiles give 4.95 / 4.79 / 4.90 ms; 4096 x 10M is indifferent within run-to-run noise)
       p.scout_tiles = (p.c_share > 0 && seg_tiles >= 128) ? (seg_tiles >= 512 ? 32 : 16) : 0;
-      if (g_debug_scout >= 0) p.scout_tiles = (p.c_share > 0) ? g_debug_scout : 0;
     }
     p.part_scores = part_scores + static_cast<size_t>(c0) * slots * K;
     p.part_ids = part_ids + static_cast<size_t>(c0) * slots * K;
     p.part_cnt = part_cnt + static_cast<size_t>(c0) * slots;
     p.slots = slots;
-    p.dense_out = nullptr; p.dense_ld = 0; p.probe_out = g_debug_probe_out;
+    p.dense_out = nullptr; p.dense_ld = 0;
     p.s_full = d.s_full; p.rem = d.rem; p.full_tiles = d.full_tiles; p.y_tiles = d.y_tiles;
     // Overlap with the previous chunk launch is safe for the scratch as long as chunk i never runs next to
     // chunk i-2 (they share a ring copy): one CTA fits per SM, so that cannot happen when chunk i-1 fills
     // every SM -- chunk i can then only start once chunk i-2 is gone.
-    const bool ov = g_debug_overlap && (chunk_idx == 1 || (chunk_idx > 1 && prev_ctas >= sms));
+    const bool ov = chunk_idx == 1 || (chunk_idx > 1 && prev_ctas >= sms);
     prev_ctas = d.grid * cg;
-#ifdef LRB_DEBUG_MODES
-    if (g_debug_mode >= 1 && g_debug_mode <= 6 && K <= 20) {   // pipeline probes (see the kernel's PROBE parameter)
-      const int m = g_debug_mode;
-      if (cg == 2) {
-        rc = m == 1 ? launch_tc<20, LRB_NS_PAIR, false, 2, LRB_EW20, 1>(ta, tb2, tbias, p, d.grid, st, ov)
-           : m == 2 ? launch_tc<20, LRB_NS_PAIR, false, 2, LRB_EW20, 2>(ta, tb2, tbias, p, d.grid, st, ov)
-           : m == 4 ? launch_tc<20, LRB_NS_PAIR, false, 2, LRB_EW20, 4>(ta, tb2, tbias, p, d.grid, st, ov)
-           : m == 5 ? launch_tc<20, LRB_NS_PAIR, false, 2, LRB_EW20, 5>(ta, tb2, tbias, p, d.grid, st, ov)
-                    : launch_tc<20, LRB_NS_PAIR, false, 2, LRB_EW20, 6>(ta, tb2, tbias, p, d.grid, st, ov);
-      } else {
-        rc = m == 1 ? launch_tc<20, 2, false, 1, LRB_EW20, 1>(ta, tb1, tbias1, p, d.grid, st, ov)
-           : m == 2 ? launch_tc<20, 2, false, 1, LRB_EW20, 2>(ta, tb1, tbias1, p, d.grid, st, ov)
-           : m == 4 ? launch_tc<20, 2, false, 1, LRB_EW20, 4>(ta, tb1, tbias1, p, d.grid, st, ov)
-           : m == 5 ? launch_tc<20, 2, false, 1, LRB_EW20, 5>(ta, tb1, tbias1, p, d.grid, st, ov)
-                    : launch_tc<20, 2, false, 1, LRB_EW20, 6>(ta, tb1, tbias1, p, d.grid, st, ov);
-      }
-      if (rc != LRB_OK) return rc;
-      continue;
-    }
-#endif
     if (cg == 2) {
       if (K <= 20 && p.c_share > tc::MAX_C_SHARE_SMALL)
-        rc = launch_tc<20, LRB_NS_PAIR, false, 2, LRB_EW20, 0, tc::MAX_C_SHARE_LARGE>(ta, tb2, tbias, p, d.grid, st, ov);
-      else if (K <= 20) rc = launch_tc<20, LRB_NS_PAIR, false, 2, LRB_EW20>(ta, tb2, tbias, p, d.grid, st, ov);
-      else if (K <= 32) rc = launch_tc<32, 4, false, 2, 8>(ta, tb2, tbias, p, d.grid, st, ov);
-      else rc = launch_tc<50, 3, false, 2, 8>(ta, tb2, tbias, p, d.grid, st, ov);
+        rc = launch_tc<20, NS_PAIR, false, 2, tc::MAX_C_SHARE_LARGE>(ta, tb2, tbias, p, d.grid, st, ov);
+      else if (K <= 20) rc = launch_tc<20, NS_PAIR, false, 2>(ta, tb2, tbias, p, d.grid, st, ov);
+      else if (K <= 32) rc = launch_tc<32, 4, false, 2>(ta, tb2, tbias, p, d.grid, st, ov);
+      else rc = launch_tc<50, 3, false, 2>(ta, tb2, tbias, p, d.grid, st, ov);
     } else {
-      if (K <= 20) rc = launch_tc<20, 2, false, 1, LRB_EW20>(ta, tb1, tbias1, p, d.grid, st, ov);
-      else if (K <= 32) rc = launch_tc<32, 3, false, 1, 8>(ta, tb1, tbias1, p, d.grid, st, ov);
-      else rc = launch_tc<50, 2, false, 1, 8>(ta, tb1, tbias1, p, d.grid, st, ov);
+      if (K <= 20) rc = launch_tc<20, 2, false, 1>(ta, tb1, tbias1, p, d.grid, st, ov);
+      else if (K <= 32) rc = launch_tc<32, 3, false, 1>(ta, tb1, tbias1, p, d.grid, st, ov);
+      else rc = launch_tc<50, 2, false, 1>(ta, tb1, tbias1, p, d.grid, st, ov);
     }
     if (rc != LRB_OK) return rc;
   }
@@ -823,24 +761,9 @@ int lrb_score_dense(const void* x, const void* table, const float* bias_pad, con
   LRB_REQUIRE(M > 0 && M < INT_MAX && rows > 0 && rows < INT_MAX && ld_out >= rows, "lrb_score_dense: bad shape");
   cudaStream_t st = as_stream(stream);
   int sms = device_sm_count();
-  if (precision == 1) {
-    f32::Params p;
-    p.u = static_cast<const float*>(x);
-    p.table = static_cast<const float*>(table);
-    p.bias_pad = bias_pad;
-    p.B = static_cast<int>(M); p.rows = static_cast<int>(rows); p.row_offset = 0; p.K = 0;
-    p.excl_sorted = nullptr; p.excl_bloom = nullptr; p.excl_stride = 0;
-    p.part_scores = nullptr; p.part_ids = nullptr; p.part_cnt = nullptr; p.slots = 0;
-    p.dense_out = out; p.dense_ld = ld_out;
-    const int splits = f32::splits_for(static_cast<int>(M), rows, sms, 4);
-    const size_t smem = (f32::IT * f32::D + f32::IT) * 4 + static_cast<size_t>(f32::ROWS) * (f32::IT + 1) * 4;
-    auto kern = f32::score_f32_kernel<true>;
-    LRB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    dim3 grid(static_cast<unsigned>((M + f32::ROWS - 1) / f32::ROWS), splits);
-    kern<<<grid, f32::ROWS, smem, st>>>(p);
-    LRB_CUDA_TRY(cudaGetLastError());
-    return LRB_OK;
-  }
+  if (precision == 1)
+    return f32::launch_dense(static_cast<const float*>(x), static_cast<const float*>(table), bias_pad,
+                             static_cast<int>(M), static_cast<int>(rows), out, ld_out, sms, st);
   LRB_REQUIRE(precision == 0, "precision must be 0 (bf16) or 1 (fp32)");
   const Decomp d = decompose(static_cast<int>(M), rows, sms);
   CUtensorMap ta, tb;
@@ -852,15 +775,15 @@ int lrb_score_dense(const void* x, const void* table, const float* bias_pad, con
   p.B = static_cast<int>(M); p.m_tiles = d.m_tiles; p.rows = static_cast<int>(rows); p.n_tiles = d.n_tiles;
   p.row_offset = 0; p.K = 1; p.bias_blk = static_cast<const uint8_t*>(bias_blk);
   p.excl_sorted = nullptr; p.excl_bloom = nullptr; p.excl_stride = 0;
-  p.gslots = nullptr; p.gstride = 0; p.pair_drain = 0; p.c_share = 0; p.scout_tiles = 0; p.ring = nullptr; p.part_scores = nullptr; p.part_ids = nullptr; p.part_cnt = nullptr; p.slots = 0;
-  p.dense_out = out; p.dense_ld = ld_out; p.probe_out = nullptr;
+  p.gslots = nullptr; p.gstride = 0; p.c_share = 0; p.scout_tiles = 0; p.ring = nullptr; p.part_scores = nullptr; p.part_ids = nullptr; p.part_cnt = nullptr; p.slots = 0;
+  p.dense_out = out; p.dense_ld = ld_out;
   p.s_full = d.s_full; p.rem = d.rem; p.full_tiles = d.full_tiles; p.y_tiles = d.y_tiles;
   CUtensorMap tbias = tb;   // placeholder without a bias block (never dereferenced)
   if (bias_blk != nullptr) {
     rc = make_tmap_bias_blocks(&tbias, bias_blk, static_cast<unsigned long long>((rows + tc::BN - 1) / tc::BN), tc::BN);
     if (rc != LRB_OK) return rc;
   }
-  return launch_tc<20, 3, true, 1, 8>(ta, tb, tbias, p, d.grid, st);
+  return launch_tc<20, 3, true, 1>(ta, tb, tbias, p, d.grid, st);
 }
 
 }  // extern "C"

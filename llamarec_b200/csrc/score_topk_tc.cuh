@@ -35,6 +35,9 @@ constexpr int BN = 256;
 constexpr int BK = 64;
 constexpr int A_BYTES = BM * BK * 2;
 constexpr int B_BYTES = BN * BK * 2;
+// The measurements quoted below that cite tools/tc_check, its probe builds ("MMA-only probe") or its
+// timeline were taken with a developer harness that instrumented this kernel through extra template modes.  The
+// harness has been removed; it is in the git history.
 // Accumulators: the SM's 512 TMEM columns hold FOUR stages of 128 columns; a 256-item tile is computed as two
 // N = 128 half-tiles.  With two 256-column stages the loop  release -> MMA -> commit -> read-out  ran ~1040 cycles per
 // tile although the tensor pipe needs 512 and the read-out ~700: the hand-offs between the MMA-issuing thread and the
@@ -49,22 +52,14 @@ constexpr int DONE_RING = 8;                // tiles in the ring of "half-tile c
 // two-stage kernel of early round 2 (10M rows, 4096 users): it read the accumulators a little faster in isolation
 // (tools/epi_probe: 702 vs 757 cycles per tile) but lost in the kernel (96 registers per thread, twice the per-thread
 // candidate sets): 5.86 vs 5.25 ms; the kernel below is written for 8.
-#ifndef LRB_EW20
-#define LRB_EW20 8
-#endif
-// LRB_OWN_HALF = 1 (default): the two column parts of the epilogue do not split every half-tile's columns (64 + 64)
-// but take one half-tile each (part p reads all 128 columns of half-tile p): a stage is then released by 4 warps per
-// CTA instead of 8, every warp waits / releases once per tile instead of twice, and the two warps of an SM
-// sub-partition use its TMEM read path at different times.  Same-box A/B on B200 (tools/tc_check, product build):
-// 4.76-4.91 -> 4.46-4.58 ms at 4096 x 10M, 5.07-5.31 -> 4.90-4.97 with bias + exclusion, 5.16-5.22 -> 4.95 at 32768 x 1.25M.
-#ifndef LRB_OWN_HALF
-#define LRB_OWN_HALF 1
-#endif
-constexpr int SLOT_PARTS = LRB_EW20 / 4;
-// harness timeline (PROBE builds): clock stamps of CTA 0 for tiles [TL_T0, TL_T0 + TL_N), 24 slots per tile behind the
-// per-CTA counters: {MMA warp woke up, MMA warp committed the second half-tile, 8 x epilogue warp saw the first
-// half-tile done, 8 x epilogue warp released the second half-tile, operands landed, first stage drained}
-constexpr int TL_T0 = 2000, TL_N = 16, TL_BASE = 148 * 8;    // partial-list / union-bound slots reserved per stream (>= column parts)
+constexpr int EPI_WARPS = 8;
+// Column parts of the epilogue = partial-list / union-bound slots per stream.  The two parts do not split every
+// half-tile's columns (64 + 64) but take one half-tile each (part p reads all 128 columns of half-tile p): a stage is
+// then released by 4 warps per CTA instead of 8, every warp waits / releases once per tile instead of twice, and the
+// two warps of an SM sub-partition use its TMEM read path at different times.  Same-box A/B on B200 (tools/tc_check,
+// product build): 4.76-4.91 -> 4.46-4.58 ms at 4096 x 10M, 5.07-5.31 -> 4.90-4.97 with bias + exclusion,
+// 5.16-5.22 -> 4.95 at 32768 x 1.25M.
+constexpr int PARTS = EPI_WARPS / 4;
 
 struct ScoreParams {
   int B;             // real users (rows >= B of the padded user matrix are ignored)
@@ -85,7 +80,6 @@ struct ScoreParams {
                                // valid lower bound on the user's K-th best (union bound), also used by the
                                // shared-stream CTAs, whose own slots are ignored (they may start late).
   int c_share;                 // c (1..MAX_C_SHARE); 0 disables the union bound
-  int pair_drain;              // CTA pairs: a drain request is forwarded to the peer CTA (1) or stays local (0)
   int scout_tiles;             // T0: the last T0 tiles of every segment are first run in "scout" mode (no
                                // candidate handling, only group maxima) to seed the union bound; 0 = off
   uint8_t* ring;               // [gridDim.x][epilogue threads][RING_GROUPS][RING_REC_BYTES] candidate rings
@@ -96,9 +90,6 @@ struct ScoreParams {
   int gstride;                 // stride (in ints) of gslots rows: the slot count of THIS launch
   float* dense_out;            // dense mode only: [B][dense_ld], columns < rows written
   long long dense_ld;
-  long long* probe_out;        // developer harness only (else nullptr): per CTA {SM cycles, nanoseconds, cycles epilogue
-                               // warp 0 waited for accumulators, cycles the MMA warp waited for its operands /
-                               // a free accumulator stage, 0, 0, 0, 0}
   // stream decomposition (host computed, see score_decompose())
   int s_full;        // number of full streams (each = m_tiles CTAs, one per user tile)
   int rem;           // CTAs in the shared stream
@@ -110,7 +101,7 @@ struct Segment {
   int m;      // user tile
   int n0;     // first item tile
   int n1;     // one past the last item tile
-  int slot;   // stream slot (partial-list slot = slot * SLOT_PARTS + column part)
+  int slot;   // stream slot (partial-list slot = slot * PARTS + column part)
 };
 
 // Deterministic walk over the segments owned by one CTA; every warp role runs the same walk.
@@ -260,10 +251,7 @@ __device__ __noinline__ float topk_consider(float s, int gid, int row_limit_gid,
 // lane repeatedly picks the best remaining score of its current record with a branch-free argmax
 // and all lanes insert at the same time, so the insert cost is paid once per warp, not per lane.
 // -------------------------------------------------------------------------------------------
-#ifndef LRB_RING_GROUPS
-#define LRB_RING_GROUPS 24
-#endif
-constexpr int RING_GROUPS = LRB_RING_GROUPS;
+constexpr int RING_GROUPS = 24;
 constexpr int RING_REC_BYTES = 80;   // 16 fp32 + int32 gid0, padded to a multiple of 16 B
 
 // c-th largest score of an unsorted set (1 <= c <= MAX_C_SHARE); -inf if the set holds fewer than c entries.
@@ -398,10 +386,10 @@ constexpr int ONES_BYTES = BM * 16 * 2;      // the matching [128][16] "ones" A 
 
 // CG = CTAs per MMA (tcgen05 cta_group): with CG == 2 every CTA stages only its half of the item tile
 // (128 rows) and of the bias block; the pair's MMA reads both halves.
-// EW = epilogue warps (8 or 16): warp w reads TMEM lanes 32*(w%4).. and column part w/4 of PARTS = EW/4.
-template <int KMAX, int NS, int CG, int EW>
+// Epilogue warp w reads TMEM lanes 32*(w%4).. of half-tile (column part) w/4.
+template <int KMAX, int NS, int CG>
 struct SmemLayout {
-  static constexpr int kEpiThreads = EW * 32;
+  static constexpr int kEpiThreads = EPI_WARPS * 32;
   static constexpr bool kExclSmem = (KMAX <= 20);   // larger K variants have no room for it
   static constexpr int kBBytes = B_BYTES / CG;              // this CTA's part of the item tile
   static constexpr int kBiasBytes = BIASBLK_BYTES / CG;     // ... and of the folded-bias block
@@ -439,12 +427,6 @@ LRB_DEVINL uint64_t umma_desc_k16_sw32(uint32_t smem_addr) {
   return d;
 }
 
-// PROBE (developer harness only, tools/tc_check; the library instantiates PROBE == 0):
-//   1 = null epilogue (TMA + MMA only)            2 = TMA only (no MMA, null epilogue)
-//   4 = no TMA traffic after the ring is primed, null epilogue (MMA only)
-//   5 = full pipeline, the filter never passes (threshold +inf)     6 = the product path, timed.
-// Every probe writes per-CTA {cycles, ns, wait counters} to p.probe_out.
-//
 // Synchronisation (mbarriers; "tile" = one 256-item tile of one segment, counted per CTA in issue order):
 //   full[s]        TMA bytes of shared-memory stage s have landed            producer -> MMA warp
 //   done[t % 8][h] the MMAs of half-tile h of tile t have completed (one tcgen05.commit per half-tile):
@@ -456,18 +438,15 @@ LRB_DEVINL uint64_t umma_desc_k16_sw32(uint32_t smem_addr) {
 // ~1500 cycles of hand-offs (remote mbarrier arrivals of the pair's other CTA, the MMA warp's wake-up and issue, the
 // commit's arrival) on top of the MMA itself; throughput = TMEM columns in flight / that cycle, hence four small
 // stages instead of two large ones, and every hand-off kept as short as it goes.
-template <int KMAX, int NS, bool kDense, int CG, int EW, int CMAX = MAX_C_SHARE_SMALL, int PROBE = 0>
-__global__ void __launch_bounds__(128 + EW * 32, 1)
+template <int KMAX, int NS, bool kDense, int CG, int CMAX = MAX_C_SHARE_SMALL>
+__global__ void __launch_bounds__(128 + EPI_WARPS * 32, 1)
 score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
                      const __grid_constant__ CUtensorMap tmap_b,
                      const __grid_constant__ CUtensorMap tmap_bias, const ScoreParams p) {
-  using L = SmemLayout<KMAX, NS, CG, EW>;
+  using L = SmemLayout<KMAX, NS, CG>;
   static_assert(CG == 1 || CG == 2, "cta_group is 1 or 2");
-  static_assert(EW == 8, "8 epilogue warps: two 128-column parts per tile (16 warps measured slower, see above)");
-  constexpr int EPI_THREADS = EW * 32;
+  constexpr int EPI_THREADS = EPI_WARPS * 32;
   constexpr int MAX_C_SHARE = CMAX;
-  constexpr int PARTS = EW / 4;            // column parts of a tile
-  static_assert(PARTS <= SLOT_PARTS, "slot stride too small");
   // CTA pair: cluster rank 0 leads (issues the MMAs, owns the barriers the pair synchronises on);
   // the pair walks the segments of "pair index" blockIdx.x / 2 and CTA `rank` owns user tile 2*m + rank.
   const uint32_t cta_rank = CG == 2 ? cluster_ctarank() : 0u;
@@ -496,11 +475,6 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const bool has_bias = p.bias_blk != nullptr;
-  long long probe_c0 = 0, probe_t0 = 0;
-  if (PROBE != 0 && threadIdx.x == 0) {
-    probe_c0 = clock64();
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(probe_t0));
-  }
 
   // Programmatic dependent launch: the chunk launches of one lrb_score_topk call are independent (disjoint
   // users, disjoint scratch), so the next chunk's CTAs may take over SMs as soon as CTAs of this launch
@@ -513,7 +487,8 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < NS; ++i) mbar_init(&full_bar[i], 1);
     for (int i = 0; i < 2 * DONE_RING; ++i) mbar_init(&done_bar[i], 1);
-    for (int i = 0; i < ACC_STAGES; ++i) mbar_init(&tmem_empty_bar[i], (LRB_OWN_HALF ? EW / 2 : EW) * CG);   // pair: both CTAs' epilogues arrive on the leader's
+    // a stage is read by the 4 warps of one column part; pair: both CTAs' epilogues arrive on the leader's
+    for (int i = 0; i < ACC_STAGES; ++i) mbar_init(&tmem_empty_bar[i], EPI_WARPS / PARTS * CG);
     mbar_init(a_full_bar, 1);
     mbar_init(a_empty_bar, 2);   // one commit from each MMA-issuing warp
     mbar_fence_init();
@@ -578,12 +553,6 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
           const int n = it < 0 ? sg.n1 + it : sg.n0 + it;   // scout pass re-visits the segment's last tiles
           // stage t % NS was last read by the MMAs of tile t - NS
           if (t >= NS) mbar_wait(&done_bar[((t - NS) % DONE_RING) * 2 + 1], ((t - NS) / DONE_RING) & 1);
-          if (PROBE == 4 && t >= NS) {
-            // probe: the stage still holds an item tile -- hand it to the MMA again, no TMA traffic
-            if (cta_rank == 0) mbar_arrive(&full_bar[stage]);
-            if (++stage == NS) { stage = 0; phase ^= 1; }
-            continue;
-          }
           uint8_t* st = sB + stage * L::kStage;
           if (CG == 2) {
             // each CTA fetches its 128 item rows (and its half of the bias block); all bytes are
@@ -627,7 +596,6 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
       constexpr uint32_t kHalfRows = HN / CG;
       constexpr uint32_t kHalfB = kHalfRows * BK * 2;        // bytes (whole SWIZZLE_128B atoms of 8 rows)
       constexpr uint32_t kHalfBias = kHalfRows * 32;         // bytes (whole SWIZZLE_32B atoms of 8 rows)
-      long long probe_wait = 0;
       while (walk.next(sg)) {
         if (lane == 0) mbar_wait(a_full_bar, seg_idx & 1);
         __syncwarp();
@@ -636,57 +604,41 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
         for (t += (t & 1) ^ mw; t < t_end; t += 2) {   // this warp's tiles of the segment
           const int stage = t % NS;
           const uint32_t epar = static_cast<uint32_t>(((t >> 1) & 1) ^ 1);   // this warp's stages: used once per own tile
-          {
-            const long long w0 = PROBE != 0 ? clock64() : 0;
-            // one lane, two waits in a row -- the accumulator stage (normally the later event) first.  (Two lanes
-            // polling one barrier each in a single try_wait left ~450 cycles between the later lane's success and the
-            // first MMA: harness timeline, A/B on B200 4.98 -> 4.78 ms at 4096 x 10M.)
-            if (lane == 0) {
-              mbar_wait(&tmem_empty_bar[2 * mw], epar);
-              if (PROBE != 0 && blockIdx.x == 0 && p.probe_out != nullptr && t >= TL_T0 && t < TL_T0 + TL_N)
-                p.probe_out[TL_BASE + (t - TL_T0) * 24 + 19] = clock64();
-              mbar_wait(&full_bar[stage], static_cast<uint32_t>((t / NS) & 1));
-              if (PROBE != 0 && blockIdx.x == 0 && p.probe_out != nullptr && t >= TL_T0 && t < TL_T0 + TL_N)
-                p.probe_out[TL_BASE + (t - TL_T0) * 24 + 18] = clock64();
-            }
-            __syncwarp();
-            if (PROBE != 0) probe_wait += clock64() - w0;
-            if (PROBE != 0 && blockIdx.x == 0 && lane == 0 && p.probe_out != nullptr && t >= TL_T0 && t < TL_T0 + TL_N)
-              p.probe_out[TL_BASE + (t - TL_T0) * 24 + 0] = clock64();
+          // one lane, two waits in a row -- the accumulator stage (normally the later event) first.  (Two lanes
+          // polling one barrier each in a single try_wait left ~450 cycles between the later lane's success and the
+          // first MMA: harness timeline, A/B on B200 4.98 -> 4.78 ms at 4096 x 10M.)
+          if (lane == 0) {
+            mbar_wait(&tmem_empty_bar[2 * mw], epar);
+            mbar_wait(&full_bar[stage], static_cast<uint32_t>((t / NS) & 1));
           }
+          __syncwarp();
           if (lane == 0) {
             tc_fence_after();
             const uint32_t st = smem_u32(sB + stage * L::kStage);
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
               if (h == 1) {   // second accumulator stage of this tile
-                const long long w0 = PROBE != 0 ? clock64() : 0;
                 mbar_wait(&tmem_empty_bar[2 * mw + 1], epar);
-                if (PROBE != 0) probe_wait += clock64() - w0;
                 tc_fence_after();
               }
               const uint64_t desc_b0 = umma_desc_k_sw128(st + h * kHalfB);
               const uint32_t d_h = d_addr + static_cast<uint32_t>(h * HN);
-              if (PROBE != 2) {
 #pragma unroll
-                for (int k = 0; k < BK / 16; ++k) {
-                  // advance 32 bytes (16 bf16) along K inside the 128-B swizzle atom: +2 in 16-B units
-                  if (CG == 2) umma_bf16_ss_pair(d_h, desc_a0 + 2 * k, desc_b0 + 2 * k, idesc, k > 0 ? 1u : 0u);
-                  else umma_bf16_ss(d_h, desc_a0 + 2 * k, desc_b0 + 2 * k, idesc, k > 0 ? 1u : 0u);
-                }
-                // folded bias: D += ones[128x16] * bias_blk[128x16]^T  (hi + mid + lo bf16 terms)
-                if (has_bias) {
-                  const uint64_t desc_bias = umma_desc_k16_sw32(st + L::kBBytes + h * kHalfBias);
-                  if (CG == 2) umma_bf16_ss_pair(d_h, desc_ones, desc_bias, idesc, 1u);
-                  else umma_bf16_ss(d_h, desc_ones, desc_bias, idesc, 1u);
-                }
+              for (int k = 0; k < BK / 16; ++k) {
+                // advance 32 bytes (16 bf16) along K inside the 128-B swizzle atom: +2 in 16-B units
+                if (CG == 2) umma_bf16_ss_pair(d_h, desc_a0 + 2 * k, desc_b0 + 2 * k, idesc, k > 0 ? 1u : 0u);
+                else umma_bf16_ss(d_h, desc_a0 + 2 * k, desc_b0 + 2 * k, idesc, k > 0 ? 1u : 0u);
+              }
+              // folded bias: D += ones[128x16] * bias_blk[128x16]^T  (hi + mid + lo bf16 terms)
+              if (has_bias) {
+                const uint64_t desc_bias = umma_desc_k16_sw32(st + L::kBBytes + h * kHalfBias);
+                if (CG == 2) umma_bf16_ss_pair(d_h, desc_ones, desc_bias, idesc, 1u);
+                else umma_bf16_ss(d_h, desc_ones, desc_bias, idesc, 1u);
               }
               // one commit per half-tile: accumulator stage full (epilogues); the second one also means
               // "shared-memory stage free" (producers)
               if (CG == 2) umma_commit_pair(&done_bar[(t % DONE_RING) * 2 + h], 0b11);
               else umma_commit(&done_bar[(t % DONE_RING) * 2 + h]);
-              if (PROBE != 0 && h == 1 && blockIdx.x == 0 && p.probe_out != nullptr && t >= TL_T0 && t < TL_T0 + TL_N)
-                p.probe_out[TL_BASE + (t - TL_T0) * 24 + 1] = clock64();
             }
           }
           __syncwarp();
@@ -699,7 +651,6 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
         __syncwarp();
         ++seg_idx;
       }
-      if (PROBE != 0 && lane == 0 && warp == 1 && p.probe_out != nullptr) p.probe_out[blockIdx.x * 8 + 3] = probe_wait;
     }
   } else if (warp == 3) {
     // ===================== threshold service =====================
@@ -720,7 +671,7 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
             for (int sl = 0; sl < p.s_full; ++sl) {
 #pragma unroll
               for (int pt = 0; pt < PARTS; ++pt) {
-                const int v = gs[sl * SLOT_PARTS + pt];
+                const int v = gs[sl * PARTS + pt];
                 mn = v < mn ? v : mn;
               }
             }
@@ -734,9 +685,9 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
   } else {
     setmaxnreg_inc<224>();
     // ===================== epilogue =====================
-    const int ew = warp - 4;          // 0..EW-1
+    const int ew = warp - 4;          // 0..EPI_WARPS-1
     const int quad = ew & 3;          // TMEM lane quadrant == warp % 4
-    const int part = ew >> 2;         // column part of the tile
+    const int part = ew >> 2;         // column part of the tile = the half-tile this warp reads
     const int et = ew * 32 + lane;    // epilogue thread index
     const int r = quad * 32 + lane;   // row inside the user tile
     const uint32_t ls = smem_u32(sListS + et);
@@ -747,62 +698,35 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
     Segment sg;
     int t = 0;                        // tiles consumed so far (same count as the MMA warp's)
     int seg_idx = -1;
-    long long probe_epi_wait = 0, probe_drain_cyc = 0, probe_drains = 0, probe_appends = 0;
     // "accumulator stage drained": local barrier, or the leader's for a CTA pair
     const uint32_t acc_empty_addr0 = CG == 2 ? mapa_u32(smem_u32(&tmem_empty_bar[0]), 0) : smem_u32(&tmem_empty_bar[0]);
     const uint32_t peer_drain_addr =
         CG == 2 ? mapa_u32(smem_u32(const_cast<int*>(&sSvc[3])), cta_rank ^ 1u) : 0u;
-    // Half-tile h of tile tt lives in accumulator stage (tt & 1) * 2 + h; this warp reads its HCOLS = 64 columns
-    // [part * 64, part * 64 + 64) of every half-tile.  Column c of half-tile h holds the item
+    // Half-tile h of tile tt lives in accumulator stage (tt & 1) * 2 + h; this warp reads all 128 columns of half-tile
+    // `part` as two 64-column BLOCKS q = 0, 1 (columns [q * 64, q * 64 + 64)).  Column c of half-tile h holds the item
     //     pair:   (c / 64) * 128 + h * 64 + c % 64   (columns 0..63 come from the leader CTA's item rows, 64..127 from the peer's)
     //     single: h * 128 + c
-    // of the 256-item tile, i.e. this warp's columns are 64 consecutive items starting at item_off(h).
-    constexpr int HCOLS = HN / PARTS;   // 64
-    static_assert(HCOLS == 64, "one tcgen05.ld.32x32b.x64 per warp and half-tile");
-    // A warp's work per tile = two 64-column BLOCKS q = 0, 1.  Shared half-tiles (LRB_OWN_HALF == 0): block q is this
-    // warp's column part of half-tile q.  Own half-tiles: both blocks are the two column halves of half-tile `part`.
-    constexpr bool kOwn = LRB_OWN_HALF != 0;
+    // of the 256-item tile, i.e. block q is 64 consecutive items starting at item_off(q).
+    constexpr int HCOLS = HN / 2;   // 64
+    static_assert(HCOLS == 64, "one tcgen05.ld.32x32b.x64 per warp and block");
     const uint32_t taddr_quad = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
     auto half_taddr = [&](int tt, int q) {
-      const int h = kOwn ? part : q, cb = kOwn ? q : part;
-      return taddr_quad + static_cast<uint32_t>(((tt & 1) * 2 + h) * HN + cb * HCOLS);
+      return taddr_quad + static_cast<uint32_t>(((tt & 1) * 2 + part) * HN + q * HCOLS);
     };
-    auto item_off = [&](int q) {
-      const int h = kOwn ? part : q, cb = kOwn ? q : part;
-      return CG == 2 ? cb * 128 + h * 64 : h * 128 + cb * 64;
-    };
-    auto wait_half_raw = [&](int tt, int h) {   // the accumulator of half-tile h of tile tt is complete
-      uint64_t* bar = &done_bar[(tt % DONE_RING) * 2 + h];
-      if (PROBE != 0) {
-        const long long w0 = clock64();
-        mbar_wait(bar, (tt / DONE_RING) & 1);
-        probe_epi_wait += clock64() - w0;
-        if (h == 0 && blockIdx.x == 0 && lane == 0 && p.probe_out != nullptr && tt >= TL_T0 && tt < TL_T0 + TL_N)
-          p.probe_out[TL_BASE + (tt - TL_T0) * 24 + 2 + ew] = clock64();
-      } else {
-        mbar_wait(bar, (tt / DONE_RING) & 1);
-      }
+    auto item_off = [&](int q) { return CG == 2 ? q * 128 + part * 64 : part * 128 + q * 64; };
+    // a warp waits for its half-tile before its first block and releases the accumulator stage after its second
+    auto wait_half = [&](int tt) {   // the accumulator of half-tile `part` of tile tt is complete
+      mbar_wait(&done_bar[(tt % DONE_RING) * 2 + part], (tt / DONE_RING) & 1);
       tc_fence_after();
     };
-    auto release_half_raw = [&](int tt, int h) {   // this warp's loads of that accumulator stage have landed in its registers
+    auto release_half = [&](int tt) {   // this warp's loads of that accumulator stage have landed in its registers
       tc_fence_before();
       __syncwarp();
       if (lane == 0) {            // (consecutive mbarriers are 8 bytes apart, in either address window)
-        const uint32_t stg = static_cast<uint32_t>((tt & 1) * 2 + h);
+        const uint32_t stg = static_cast<uint32_t>((tt & 1) * 2 + part);
         if (CG == 2) mbar_arrive_cluster(acc_empty_addr0 + stg * 8u);
         else mbar_arrive(&tmem_empty_bar[stg]);
-        if (PROBE != 0 && h == 1 && blockIdx.x == 0 && p.probe_out != nullptr && tt >= TL_T0 && tt < TL_T0 + TL_N)
-          p.probe_out[TL_BASE + (tt - TL_T0) * 24 + 10 + ew] = clock64();
       }
-    };
-    // block-level wrappers: with own half-tiles a warp waits before its first block and releases after its second
-    auto wait_half = [&](int tt, int q) {
-      if (!kOwn) wait_half_raw(tt, q);
-      else if (q == 0) wait_half_raw(tt, part);
-    };
-    auto release_half = [&](int tt, int q) {
-      if (!kOwn) release_half_raw(tt, q);
-      else if (q == 1) release_half_raw(tt, part);
     };
     while (walk.next(sg)) {
       ++seg_idx;
@@ -815,7 +739,7 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
       float own_thr = -INFINITY;
       int published = INT_MIN;
       if (part == 0) rowthr[r] = INT_MIN;
-      const int my_slot = sg.slot * SLOT_PARTS + part;
+      const int my_slot = sg.slot * PARTS + part;
       const bool publishes = sg.slot < p.s_full;   // only full-stream threads feed the union bound
       const int* excl = nullptr;
       uint32_t bloom0 = 0u, bloom1 = 0u, bloom2 = 0u, bloom3 = 0u;
@@ -861,21 +785,17 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
         for (int j = 0; j < MAX_C_SHARE; ++j) tm[j] = -INFINITY;
         for (int it = 0; it < n_scout_run; ++it, ++t) {
 #pragma unroll 1
-          for (int h = 0; h < 2; ++h) {
-            wait_half(t, h);
-            if (PROBE == 1 || PROBE == 2 || PROBE == 4) {   // null epilogue
-              release_half(t, h);
-              continue;
-            }
+          for (int blk = 0; blk < 2; ++blk) {
+            if (blk == 0) wait_half(t);
             // Columns past the end of the table (the ragged last tile) must not count as admissible items:
             // without a folded-bias block they score exactly 0 (TMA zero-fills out-of-bounds rows), and a
             // bound published from them could exceed a user's true K-th best.  valid = real items among
-            // this thread's 64 columns of the half-tile (warp-uniform; < 64 only in the last tile).
-            const int valid = p.rows - ((sg.n1 - n_scout_run + it) * BN + item_off(h));
+            // this thread's 64 columns of the block (warp-uniform; < 64 only in the last tile).
+            const int valid = p.rows - ((sg.n1 - n_scout_run + it) * BN + item_off(blk));
             uint32_t w[64];
-            tmem_ld_32x64(half_taddr(t, h), w);
+            tmem_ld_32x64(half_taddr(t, blk), w);
             tmem_ld_wait();
-            release_half(t, h);
+            if (blk == 1) release_half(t);
 #pragma unroll
             for (int g = 0; g < 4; ++g) {
               float q[16];
@@ -943,39 +863,24 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
       dst.excl_stride = p.excl_stride; dst.K = p.K; dst.limit_gid = limit_gid; dst.c_share = p.c_share;
       dst.published = published; dst.live = live;
       auto drain = [&]() {
-        if (PROBE != 0) {
-          const long long d0 = clock64();
-          probe_appends += cnt;
-          own_thr = drain_rings<EPI_THREADS, KMAX, CMAX>(&dst, cnt, own_thr);
-          probe_drain_cyc += clock64() - d0;
-          probe_drains += 1;
-        } else {
-          own_thr = drain_rings<EPI_THREADS, KMAX, CMAX>(&dst, cnt, own_thr);
-        }
+        own_thr = drain_rings<EPI_THREADS, KMAX, CMAX>(&dst, cnt, own_thr);
         cnt = 0;
       };
 
       const uint32_t rowthr_s = smem_u32(rowthr + r);
       const uint32_t drain_seq_s = smem_u32(const_cast<int*>(&sSvc[3]));
 
-      if (PROBE == 1 || PROBE == 2 || PROBE == 4) {   // null epilogue (harness)
-        for (int n = sg.n0; n < sg.n1; ++n, ++t) {
-          wait_half(t, 0);
-          release_half(t, 0);
-          wait_half(t, 1);
-          release_half(t, 1);
-        }
-      } else if (kDense) {
+      if (kDense) {
         for (int n = sg.n0; n < sg.n1; ++n, ++t) {
 #pragma unroll 1
-          for (int h = 0; h < 2; ++h) {
-            wait_half(t, h);
+          for (int blk = 0; blk < 2; ++blk) {
+            if (blk == 0) wait_half(t);
             uint32_t v[64];
-            tmem_ld_32x64(half_taddr(t, h), v);
+            tmem_ld_32x64(half_taddr(t, blk), v);
             tmem_ld_wait();
-            release_half(t, h);
+            if (blk == 1) release_half(t);
             const int row = m_own * BM + r;
-            const int col0 = n * BN + item_off(h);
+            const int col0 = n * BN + item_off(blk);
             if (row < p.B) {
               float* dstp = p.dense_out + static_cast<size_t>(row) * p.dense_ld + col0;
               if (col0 + HCOLS <= p.rows && (p.dense_ld & 3) == 0) {
@@ -1034,17 +939,11 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
           // key_to_float(INT_MIN) is a NaN, which fmaxf ignores: an unset shared threshold leaves own_thr.
           const int kk = lds_volatile_s32(rowthr_s);
           const int seq0 = lds_volatile_s32(drain_seq_s);
-          float t_eff = fmaxf(own_thr, key_to_float(kk));
-          if (PROBE == 5) t_eff = INFINITY;
+          const float t_eff = fmaxf(own_thr, key_to_float(kk));
           const int tile_gid0 = p.row_offset + n * BN;
 
-          wait_half(t, 0);
+          wait_half(t);
           tmem_ld_32x64(half_taddr(t, 0), va);
-          if (!kOwn) {
-            tmem_ld_wait();
-            release_half(t, 0);
-            wait_half(t, 1);
-          }
           tmem_ld_32x64(half_taddr(t, 1), vb);     // in flight while the first block is reduced
           float ga[4];
 #pragma unroll
@@ -1053,7 +952,7 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
           if (__builtin_expect(hit_a, 0)) dump_half(va, ga, t_eff, tile_gid0 + item_off(0));
 
           tmem_ld_wait();
-          release_half(t, 1);
+          release_half(t);
           float gb[4];
 #pragma unroll
           for (int q = 0; q < 4; ++q) gb[q] = group_max(vb, q * 16);
@@ -1067,14 +966,14 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
             // within the first microseconds, which defines the union bound.  Drains are synchronised across the
             // CTA's epilogue warps: a warp that must drain bumps a shared sequence number and every warp drains at
             // its next tile boundary.  A drain stalls the accumulator ring for everybody, so simultaneous
-            // drains cost one stall, not EW.
+            // drains cost one stall, not one per warp.
             const bool need = __any_sync(0xffffffffu, cnt > RING_GROUPS - 8 || (boot && cnt > 0));
             int seq = lds_volatile_s32(drain_seq_s);
             if (need && seq == drain_seen) {
               if (lane == 0) {
                 atomicAdd(const_cast<int*>(&sSvc[3]), 1);
                 // a drain stalls the pair's accumulator ring: let the peer CTA drain at the same time
-                if (CG == 2 && p.pair_drain) red_add_cluster_u32(peer_drain_addr, 1u);
+                if (CG == 2) red_add_cluster_u32(peer_drain_addr, 1u);
               }
               seq += 1;
             }
@@ -1101,20 +1000,8 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
       asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS));  // before the next segment resets its buffer
     }
     if (et == 0) sSvc[2] = 1;   // all segments of this CTA are done: stop the threshold service
-    if (PROBE != 0 && et == 0 && p.probe_out != nullptr) {
-      p.probe_out[blockIdx.x * 8 + 2] = probe_epi_wait;
-      p.probe_out[blockIdx.x * 8 + 5] = probe_drain_cyc;
-      p.probe_out[blockIdx.x * 8 + 6] = probe_drains;
-      p.probe_out[blockIdx.x * 8 + 7] = probe_appends;
-    }
   }
 
-  if (PROBE != 0 && threadIdx.x == 0 && p.probe_out != nullptr) {
-    long long t1;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-    p.probe_out[blockIdx.x * 8] = clock64() - probe_c0;
-    p.probe_out[blockIdx.x * 8 + 1] = t1 - probe_t0;
-  }
   // ... but no launch may COMPLETE before its predecessor has: what follows the last chunk in the stream
   // (the merge kernel) must see the results of every chunk.
   asm volatile("griddepcontrol.wait;" ::: "memory");

@@ -6,6 +6,7 @@ K <= 20 / 32 / 50 kernel variants (the longer lists keep no shared-memory copy o
 one launch each, the merge's register or global-memory path, and on the exact-fp32 side the dense + select path (in
 user blocks) or the streaming kernel.  Each case below names the branch it targets and asserts it through a Python
 restatement of the host-side decomposition (score.cu); the CPU test pins that restatement to lrb_score_topk_slots.
+The dense mode of the same tensor-core kernel (lrb_score_dense, precision 0) is checked against the same fp64 scores.
 
 Reference: plain torch float64 GEMMs (cuBLAS DGEMM) over the exact operands the kernel consumed -- the bf16 user
 states and table upcast, or the fp32 ones -- plus the fp32 bias; -inf at every history id and at item 0 (global ids);
@@ -26,7 +27,6 @@ in the scouted tail of every full-stream segment and in the ragged last tile; ev
 holding them (with duplicates), so the exclusion list, the scout's count of excluded ids and the history mask all
 decide the lists."""
 import math
-import os
 from types import SimpleNamespace
 
 import numpy as np
@@ -40,10 +40,9 @@ from oracle import metrics_oracle as MO
 # Restatement of the host-side dispatch of lrb_score_topk (score.cu, score_topk_tc.cuh)
 # ------------------------------------------------------------------------------------------------
 BM, BN = 128, 256              # users per CTA tile, items per tile
-SLOT_PARTS = 2                 # LRB_EW20 / 4: partial-list slots per stream
-PARTS = 2                      # epilogue_warps_for(K) / 4 (8 epilogue warps for every K)
+PARTS = 2                      # tc::PARTS: column parts of the 8 epilogue warps = partial-list slots per stream
 MAX_C_SMALL, MAX_C_LARGE = 6, 12
-RESTART_TILES = 150.0          # LRB_RESTART_TILES
+RESTART_TILES = 150.0          # RESTART_TILES in score.cu
 EX_CAP = 56                    # ints per row of the shared-memory exclusion copy
 RING_BYTES_PER_SM = 512 * 24 * 80   # epilogue threads x RING_GROUPS x RING_REC_BYTES
 MERGE_REG_ENTRIES = 32 * 32    # lrb_merge_metrics keeps up to 32 entries per lane in registers
@@ -58,8 +57,6 @@ def users_per_launch(B, sms):
 
 
 def cta_group_for(B, sms):
-    if os.environ.get("LRB_SCORE_CTA_GROUP", "") == "1":
-        return 1
     return 2 if (B > BM and sms >= 2) else 1
 
 
@@ -83,7 +80,7 @@ def decompose(B, rows, units, bm):
         if y_tiles <= 0:
             y_tiles, rem = 0, 0
         full_tiles = n_tiles - y_tiles
-    slots = SLOT_PARTS * (s_full + (2 if rem > 0 else 0))
+    slots = PARTS * (s_full + (2 if rem > 0 else 0))
     return dict(m_tiles=m_tiles, n_tiles=n_tiles, s_full=s_full, rem=rem, y_tiles=y_tiles, full_tiles=full_tiles,
                 slots=slots)
 
@@ -437,16 +434,16 @@ def _world_300k(worlds, regime):
 @pytest.mark.parametrize("regime", ["zero", "bias"])
 def test_cta_pairs_union_bound_scout_and_global_exclusion(worlds, regime):
     """2048 users x 300,001 rows, L = 200: CTA pairs, 9 full streams plus a shared stream, union bound with c = 3 / 2,
-    scout 16, exclusion lists too long for shared memory; K = 50, 33, 21 (the K <= 50 and K <= 32 kernels); and the
-    same shape without exclusion (item 0 and history items compete)."""
+    scout 16, exclusion lists too long for shared memory; K = 50, 33, 21, 20 (the K <= 50, K <= 32 and K <= 20
+    kernels); and the same shape without exclusion (item 0 and history items compete)."""
     B, rows, L = 2048, 300_001, 200
-    for K, c, kmax in ((50, 3, 50), (33, 2, 50), (21, 2, 32)):
+    for K, c, kmax in ((50, 3, 50), (33, 2, 50), (21, 2, 32), (20, 2, 20)):
         plan = _assert_bf16_branch(B, rows, K, L, cg=2, s_full=9, c_share=c, scout=16, kmax=kmax, excl_in_smem=False)
         assert plan[0]["rem"] > 0 and plan[0]["y_tiles"] > 0          # a shared stream
     w = _world_300k(worlds, regime)
     x = _histories(B, L, w.hot, rows, seed=1).cuda()
     u = w.users(B, seed=2)
-    for K in (50, 33, 21):
+    for K in (50, 33, 21, 20):
         w.check(f"pairs_{regime}_K{K}", x, u, w.run(x, u, K, "bf16"), K, "bf16")
     w.check(f"pairs_{regime}_noexcl", x, u, w.run(x, u, 50, "bf16", exclude=False), 50, "bf16", exclude=False)
 
@@ -511,13 +508,13 @@ def _world_3m(worlds):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("K", [32, 50])
+@pytest.mark.parametrize("K", [5, 32, 50])
 def test_many_full_streams_ragged_last_pair_tile(worlds, K):
     """300 users x 3,000,001 rows: 37 full streams (no shared stream), c = 1, scout 16; the second pair tile holds
-    256 + 44 users."""
+    256 + 44 users.  K = 5 runs the K <= 20 kernel with lists shorter than its capacity."""
     B, rows, L = 300, 3_000_001, 200
     plan = _assert_bf16_branch(B, rows, K, L, cg=2, m_tiles=2, s_full=37, rem=0, c_share=1, scout=16)
-    assert B - 256 == 44 and plan[0]["kmax"] == (32 if K == 32 else 50)
+    assert B - 256 == 44 and plan[0]["kmax"] == {5: 20, 32: 32, 50: 50}[K]
     w = _world_3m(worlds)
     x = _histories(B, L, w.hot, rows, seed=7).cuda()
     u = w.users(B, seed=8)
@@ -602,6 +599,42 @@ def test_fewer_admissible_items_than_k():
     res = w.run(x, u, K, "bf16")
     w.check("tiny_K50", x, u, res, K, "bf16")
     assert bool((res["ids"][:, -1] == -1).all())
+
+
+UNTOUCHED = 0x7FA5A5A5   # a float32 NaN pattern the kernel never writes
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("with_bias", [True, False])
+@pytest.mark.parametrize("M, rows, ld", [(200, 1000, 1000), (128, 256, 260), (1, 77, 83)])
+def test_dense_bf16_scores_against_fp64(M, rows, ld, with_bias):
+    """lrb_score_dense with precision 0 (the tensor-core kernel's dense mode; LRURec.forward always asks for fp32):
+    every score of the M x rows block within 128 * 2^-24 * (sum_k |u_k e_nk| + |bias_n|) of the fp64 score of the
+    same bf16 operands, with a folded-bias block and with bias_blk = NULL (zero bias).  Output columns >= rows of
+    every row (ld > rows) and rows >= M are left untouched; ld = 83 takes the kernel's scalar store path."""
+    lib = _lib.load()
+    dev = torch.device("cuda")
+    g = torch.Generator(device=dev).manual_seed(1000 * M + rows)
+    table = torch.randn(rows, 64, device=dev, generator=g) * 0.05
+    bias = torch.randn(rows, device=dev, generator=g) * 0.05 if with_bias else torch.zeros(rows, device=dev)
+    table16 = torch.empty(rows, 64, dtype=torch.bfloat16, device=dev)
+    bias_pad = torch.empty((rows + BN - 1) // BN * BN, dtype=torch.float32, device=dev)
+    bias_blk = torch.empty(lib.lrb_bias_blk_bytes(rows), dtype=torch.uint8, device=dev) if with_bias else None
+    _lib.check(lib.lrb_prepare_table(_lib.ptr(table), _lib.ptr(bias), 0, rows, _lib.ptr(table16), _lib.ptr(bias_pad),
+                                     _lib.ptr(bias_blk), _lib.stream_handle()))
+    u16 = torch.randn(M, 64, device=dev, generator=g).to(torch.bfloat16)
+    out = torch.full((M + 3, ld), UNTOUCHED, dtype=torch.int32, device=dev)
+    _lib.check(lib.lrb_score_dense(_lib.ptr(u16), _lib.ptr(table16), _lib.ptr(bias_pad), _lib.ptr(bias_blk), M, rows,
+                                   0, _lib.ptr(out), ld, _lib.stream_handle()))
+    torch.cuda.synchronize()
+    U, E, b64 = u16.double(), table16.double(), bias.double()
+    ref = torch.addmm(b64, U, E.t())
+    tol = TOL_C * 2.0 ** -24 * torch.addmm(b64.abs(), U.abs(), E.abs().t())
+    err = (out[:M, :rows].view(torch.float32).double() - ref).abs()
+    bad = ~(err <= tol)
+    assert not bool(bad.any()), (f"{int(bad.sum())} of {M * rows} scores off; first at "
+                                 f"{bad.nonzero()[0].tolist()}, max |err|/tol = {float((err / tol).max()):.3f}")
+    assert bool((out[:M, rows:] == UNTOUCHED).all()) and bool((out[M:] == UNTOUCHED).all())
 
 
 # ------------------------------------------------------------------------------------------------
