@@ -145,9 +145,11 @@ int lrb_score_dense(const void* x, const void* table, const float* bias_pad, con
  * the catalogue fused with the scoring contraction (exact fp32 path).
  *   hidden [M][64] fp32: encoder output at every position (lrb_encode_fwd, all_positions = 1), M = B*L
  *   table_f32 [rows][64], bias_pad: as for lrb_score_dense (rows = N+1, the whole table)
- *   labels [M] int64; rows whose label == ignore_index do not count
- * Outputs: row_loss [M] (optional, 0 for ignored rows); loss_sum[2] += {sum of row losses, counted
- *   rows} (the caller zeroes it; mean loss = loss_sum[0] / loss_sum[1]).
+ *   labels [M] int64; rows whose label == ignore_index do not count.  Neither does a row whose label
+ *   is outside [0, rows): this call does not synchronise, so it cannot raise the error torch's
+ *   cross_entropy raises for such a label (lrb_train_step does); the row only leaves the mean.
+ * Outputs: row_loss [M] (optional, 0 for rows that do not count); loss_sum[2] += {sum of row losses,
+ *   counted rows} (the caller zeroes it; mean loss = loss_sum[0] / loss_sum[1]).
  * Workspace: lrb_ce_workspace_bytes(M, rows).
  * ------------------------------------------------------------------------------------------ */
 size_t lrb_ce_workspace_bytes(int64_t M, int64_t rows);
@@ -162,7 +164,9 @@ int lrb_ce_loss_fwd(const float* hidden, const float* table_f32, const float* bi
  * nn.CrossEntropyLoss(ignore_index) (trainer/lru.py:20), in eval mode: no dropout (lrb_train_step_dropout
  * below is the train-mode step; this function is that call with every rate 0).  Rows must be
  * left-padded (dataloader/lru.py:98-118) -- otherwise LRB_ERR_UNSUPPORTED.
- *   ids [B][L] int64/int32 (id_bytes 8/4), labels [B*L] int64
+ *   ids [B][L] int64/int32 (id_bytes 8/4), labels [B*L] int64: each is ignore_index or in [0, table_rows),
+ *   like the targets torch's cross_entropy accepts -- otherwise LRB_ERR_BAD_ARG (found on the device: the
+ *   outputs are then meaningless)
  *   table_f32 [table_rows][64], bias_f32 [table_rows], weights = the packed blob of lrb_encode_fwd,
  *   params_log [n_blocks][3][128] (nu_log, theta_log, gamma_log of every block, model/lru.py:119)
  * Outputs (overwritten)
@@ -171,7 +175,8 @@ int lrb_ce_loss_fwd(const float* hidden, const float* table_f32, const float* bi
  *                     lambda_re / lambda_im / gamma slots hold d nu_log / d theta_log / d gamma_log
  *   grad_table [table_rows][64]  (scoring matmul + embedding gather: the table is tied)
  *   grad_bias  [table_rows]
- * Workspace: lrb_train_workspace_bytes(B, L, n_blocks).  Synchronises the stream once (error flag).
+ * Workspace: lrb_train_workspace_bytes(B, L, n_blocks).  Synchronises the stream once (the error flag of the
+ * two input checks above).
  * ------------------------------------------------------------------------------------------ */
 size_t lrb_train_workspace_bytes(int B, int L, int n_blocks);
 int lrb_train_step(const void* ids, int id_bytes, const int64_t* labels, int B, int L, const float* table_f32,

@@ -18,9 +18,11 @@
 // Scope.  Training batches are LEFT-padded
 // (dataloader/lru.py:98-118), for which the reference's recursive-doubling scan equals the recurrence
 //     h_p = lambda * (mask_{p-1} h_{p-1}) + bu_p        (SURVEY probe P1),
-// whose backward is the mirrored recurrence; a row with a zero after a non-zero id is rejected (error flag).
+// whose backward is the mirrored recurrence; a row with a zero after a non-zero id is rejected (error flag), and so
+// is a label outside [0, rows) that is not ignore_index (torch's cross_entropy raises for one as well).
 //
-// fp32 throughout (gradients are compared with the fp32 reference at rtol 1e-3).  Complex parameters are carried
+// fp32 throughout.  The gradients are compared with the reference's fp32 autograd at rtol 1e-3, and with the oracle
+// run in float64 at 1e-4 of each tensor's largest entry (tests/test_gpu_train_encoder_paths.py).  Complex parameters are carried
 // as (re, im) pairs, so the gradients that come out are (dL/dre, dL/dim) -- torch's convention for real-valued
 // losses.  The softmax-CE backward recomputes the logits tile by tile in two passes (rows own dH, items own dE
 // and dbias: no atomics on the big outputs, deterministic); everything between is small dense algebra over
@@ -38,6 +40,8 @@ constexpr int D = LRB_D;        // 64
 constexpr int H2 = 2 * LRB_H;   // 256 reals = 128 complex channels, (re, im) interleaved
 constexpr int FF = LRB_FF;      // 256
 constexpr float LN_EPS = 1e-5f;
+constexpr int ERR_NOT_LEFT_PADDED = 1;   // bits of the step's error flag
+constexpr int ERR_BAD_LABEL = 2;
 
 // packed weight / gradient blob (floats) -- the layout of llamarec_b200/packing.py and encode.cu
 constexpr int OFF_EMB_LN_W = 0;
@@ -209,7 +213,7 @@ __global__ void __launch_bounds__(256) gather_kernel(const void* __restrict__ id
     mask[warp] = id > 0 ? 1 : 0;
     const int t = warp % L;
     // left padding only: a zero id must not follow a non-zero one inside a row
-    if (t > 0 && id <= 0 && load_id(ids, warp - 1, id_bytes) > 0) atomicExch(err_flag, 1);
+    if (t > 0 && id <= 0 && load_id(ids, warp - 1, id_bytes) > 0) atomicOr(err_flag, ERR_NOT_LEFT_PADDED);
   }
   if (id < 0 || id >= table_rows) id = 0;
   const float* row = table + static_cast<size_t>(id) * D;
@@ -428,11 +432,12 @@ __global__ void params_log_grad_kernel(float* __restrict__ gblk, const float* __
 constexpr int CR = 128;   // rows (pass A) or items (pass B) per CTA
 constexpr int CI = 64;    // staged rows of the other operand
 
-// per row: lse over all items and the label's logit  ->  lse[m], row loss; loss_sum[0] += sum, loss_sum[1] += count
+// per row: lse over all items and the label's logit  ->  lse[m], row loss; loss_sum[0] += sum, loss_sum[1] += count.
+// A label outside [0, rows) that is not ignore_index sets ERR_BAD_LABEL (the row is not counted by any pass).
 __global__ void __launch_bounds__(CR) ce_stats_kernel(const float* __restrict__ hid, const float* __restrict__ table,
                                                       const float* __restrict__ bias, const long long* __restrict__ labels,
                                                       long long ignore_index, int M, int rows, float* __restrict__ lse,
-                                                      float* __restrict__ loss_sum) {
+                                                      float* __restrict__ loss_sum, int* __restrict__ err_flag) {
   __shared__ __align__(16) float sE[CI * D];
   __shared__ float sBias[CI];
   const int tid = threadIdx.x, m = blockIdx.x * CR + tid;
@@ -441,6 +446,7 @@ __global__ void __launch_bounds__(CR) ce_stats_kernel(const float* __restrict__ 
 #pragma unroll
   for (int k = 0; k < D; ++k) u[k] = live ? hid[static_cast<size_t>(m) * D + k] : 0.f;
   const long long label = live ? labels[m] : -1;
+  if (live && label != ignore_index && (label < 0 || label >= rows)) atomicOr(err_flag, ERR_BAD_LABEL);
   float run_max = -INFINITY, run_sum = 0.f, lab_logit = 0.f;
   for (int i0 = 0; i0 < rows; i0 += CI) {
     __syncthreads();
@@ -741,7 +747,8 @@ int lrb_train_step_dropout(const void* ids, int id_bytes, const int64_t* labels,
   }
   const float* hidden = x_in;
   const long long* lab = reinterpret_cast<const long long*>(labels);
-  ce_stats_kernel<<<blocks_for(T, CR), CR, 0, st>>>(hidden, table_f32, bias_f32, lab, ignore_index, T, rows, lse, loss_sum);
+  ce_stats_kernel<<<blocks_for(T, CR), CR, 0, st>>>(hidden, table_f32, bias_f32, lab, ignore_index, T, rows, lse, loss_sum,
+                                                     err_flag);
   LRB_CUDA_TRY(cudaGetLastError());
 
   // =========================== backward ===========================
@@ -802,11 +809,14 @@ int lrb_train_step_dropout(const void* ids, int id_bytes, const int64_t* labels,
                                      grad_weights + OFF_EMB_LN_B, T, 0, nullptr, no_drop);
   scatter_rows_kernel<<<warp_blocks, 256, 0, st>>>(ids, id_bytes, T, table_rows, g64b, grad_table, drop_embed);
   LRB_CUDA_TRY(cudaGetLastError());
-  // left-padding check (one 4-byte read back: the step's result is meaningless otherwise)
+  // input checks (one 4-byte read back: the step's result is meaningless otherwise)
   int err = 0;
   LRB_CUDA_TRY(cudaMemcpyAsync(&err, err_flag, 4, cudaMemcpyDeviceToHost, st));
   LRB_CUDA_TRY(cudaStreamSynchronize(st));
-  if (err != 0)
+  if (err & ERR_BAD_LABEL)
+    return set_error(LRB_ERR_BAD_ARG, "lrb_train_step: a label is outside [0, %d) and is not ignore_index %lld", rows,
+                     static_cast<long long>(ignore_index));
+  if (err & ERR_NOT_LEFT_PADDED)
     return set_error(LRB_ERR_UNSUPPORTED, "lrb_train_step: sequences must be left-padded (a zero id follows a non-zero id)");
   return LRB_OK;
 }

@@ -26,7 +26,7 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-from .lru_oracle import _ln, lru_constants, n_blocks_of, tree_scan
+from .lru_oracle import _ln, cast_state_dict, complex_of, lru_constants, n_blocks_of, tree_scan
 
 _M0, _M1 = np.uint64(0xD2511F53), np.uint64(0xCD9E8D57)
 _W0, _W1 = np.uint64(0x9E3779B9), np.uint64(0xBB67AE85)
@@ -81,11 +81,15 @@ def site_multipliers(seed: int, B: int, L: int, n_blocks: int, p_embed: float, p
 
 
 def ce_loss_train(ids: torch.Tensor, labels: torch.Tensor, sd: Dict[str, torch.Tensor],
-                  mults: Optional[Dict[int, torch.Tensor]] = None, ignore_index: int = 0) -> torch.Tensor:
+                  mults: Optional[Dict[int, torch.Tensor]] = None, ignore_index: int = 0,
+                  dtype: Optional[torch.dtype] = None, reduction: str = "mean") -> torch.Tensor:
     """trainer/lru.py:20-28 in train mode: CrossEntropyLoss(ignore_index) on the logits at every position of the
     reference's forward (model/lru.py:38-41,57-60,73-86,149-161,164-175) with dropout multipliers `mults`
-    ({site: [B, L, width]}, a missing site = multiplier 1).  Differentiable in every tensor of `sd`."""
+    ({site: [B, L, width]}, a missing site = multiplier 1).  Differentiable in every tensor of `sd`.
+    `dtype` (e.g. torch.float64) computes with `sd` and the multipliers cast to it (complex parts too); None computes
+    in the dtypes of `sd`.  `reduction` is cross_entropy's ('none': the row losses, 0 where ignored)."""
     mults = mults or {}
+    sd = cast_state_dict(sd, dtype)
     B, L = ids.shape
     Lp = 1 << max(0, math.ceil(math.log2(L))) if L > 1 else 1
 
@@ -93,8 +97,9 @@ def ce_loss_train(ids: torch.Tensor, labels: torch.Tensor, sd: Dict[str, torch.T
         m = mults.get(site)
         if m is None:
             return v
+        m = m.to(v.dtype)
         if v.shape[1] != L:                                    # padded positions: multiplier 1
-            m = torch.cat((torch.ones(B, v.shape[1] - L, m.shape[-1]), m), 1)
+            m = torch.cat((torch.ones(B, v.shape[1] - L, m.shape[-1], dtype=v.dtype), m), 1)
         return v * m
 
     x = drop(sd["embedding.token.weight"][ids], 0)
@@ -104,7 +109,7 @@ def ce_loss_train(ids: torch.Tensor, labels: torch.Tensor, sd: Dict[str, torch.T
     for i in range(n_blocks_of(sd)):
         p = f"model.lru_blocks.{i}.lru_layer."
         lam, gamma = lru_constants(sd[p + "params_log"])
-        bu = F.linear(x.to(torch.cfloat), sd[p + "in_proj.weight"], sd[p + "in_proj.bias"]) * gamma
+        bu = F.linear(x.to(complex_of(x.dtype)), sd[p + "in_proj.weight"], sd[p + "in_proj.bias"]) * gamma
         h = tree_scan(bu, lam, mask)
         o = drop(F.linear(h, sd[p + "out_proj.weight"], sd[p + "out_proj.bias"]).real, 1 + 3 * i)
         x = _ln(o + x, sd[p + "layer_norm.weight"], sd[p + "layer_norm.bias"])
@@ -114,13 +119,16 @@ def ce_loss_train(ids: torch.Tensor, labels: torch.Tensor, sd: Dict[str, torch.T
         x = _ln(z + x, sd[q + "layer_norm.weight"], sd[q + "layer_norm.bias"])
     hidden = x[:, Lp - L:, :]
     logits = torch.matmul(hidden, sd["embedding.token.weight"].t()) + sd["model.bias"]
-    return F.cross_entropy(logits.reshape(-1, logits.shape[-1]), labels.reshape(-1), ignore_index=ignore_index)
+    return F.cross_entropy(logits.reshape(-1, logits.shape[-1]), labels.reshape(-1), ignore_index=ignore_index,
+                           reduction=reduction)
 
 
 def loss_and_grads(ids: torch.Tensor, labels: torch.Tensor, sd: Dict[str, torch.Tensor],
-                   mults: Optional[Dict[int, torch.Tensor]] = None, ignore_index: int = 0):
-    """-> (loss, {parameter name: gradient as numpy}) of ce_loss_train by torch autograd."""
-    leaves = {k: v.detach().clone().requires_grad_(True) for k, v in sd.items()}
+                   mults: Optional[Dict[int, torch.Tensor]] = None, ignore_index: int = 0,
+                   dtype: Optional[torch.dtype] = None):
+    """-> (loss, {parameter name: gradient as numpy}) of ce_loss_train by torch autograd.  With `dtype` the leaves
+    are `sd` cast to it, so the gradients come out in that dtype (complex128 for the complex parameters of fp64)."""
+    leaves = {k: v.detach().clone().requires_grad_(True) for k, v in cast_state_dict(sd, dtype).items()}
     loss = ce_loss_train(ids, labels, leaves, mults, ignore_index)
     loss.backward()
     return loss.item(), {k: v.grad.numpy() for k, v in leaves.items()}

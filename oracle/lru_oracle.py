@@ -28,6 +28,18 @@ def _ln(x: torch.Tensor, w: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
     return F.layer_norm(x, (x.shape[-1],), w, b, LN_EPS)
 
 
+def complex_of(dtype: torch.dtype) -> torch.dtype:
+    """The complex dtype whose parts are `dtype`: complex64 for float32 (the reference), complex128 for float64."""
+    return torch.complex128 if dtype == torch.float64 else torch.complex64
+
+
+def cast_state_dict(sd: Dict[str, torch.Tensor], dtype: Optional[torch.dtype]) -> Dict[str, torch.Tensor]:
+    """Real tensors to `dtype`, complex ones to complex_of(dtype); None keeps `sd` as it is.  Differentiable."""
+    if dtype is None:
+        return sd
+    return {k: v.to(complex_of(dtype) if v.is_complex() else dtype) for k, v in sd.items()}
+
+
 def n_blocks_of(sd: Dict[str, torch.Tensor]) -> int:
     n = 0
     while f"model.lru_blocks.{n}.lru_layer.params_log" in sd:
@@ -54,7 +66,7 @@ def lru_constants(params_log: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]
 def tree_scan(bu: torch.Tensor, lam: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
     """model/lru.py:135-147,155-159 -- the recursive-doubling scan.
 
-    bu [B, Lp, H] complex64 with Lp a power of two, lam [1, H] complex64, mask [B, Lp] bool.
+    bu [B, Lp, H] complex with Lp a power of two, lam [1, H] of the same dtype, mask [B, Lp] bool.
     Level i works on aligned blocks of 2^i: every element j (0-based) of the second half receives
     lambda^(j+1) * (last element of the first half) * mask(last element of the first half).
     The power table doubles each level exactly as the reference builds it (table ++ table*last).
@@ -80,7 +92,7 @@ def lru_layer(x: torch.Tensor, mask: torch.Tensor, sd: Dict[str, torch.Tensor], 
     """model/lru.py:149-161 -- in_proj (complex) * gamma, tree scan, Re(out_proj) + residual, LayerNorm."""
     p = f"model.lru_blocks.{blk}.lru_layer."
     lam, gamma = lru_constants(sd[p + "params_log"])
-    bu = F.linear(x.to(torch.cfloat), sd[p + "in_proj.weight"], sd[p + "in_proj.bias"]) * gamma
+    bu = F.linear(x.to(complex_of(x.dtype)), sd[p + "in_proj.weight"], sd[p + "in_proj.bias"]) * gamma
     h = tree_scan(bu, lam, mask)
     y = F.linear(h, sd[p + "out_proj.weight"], sd[p + "out_proj.bias"]).real + x
     return _ln(y, sd[p + "layer_norm.weight"], sd[p + "layer_norm.bias"])
@@ -94,11 +106,14 @@ def pffn(x: torch.Tensor, sd: Dict[str, torch.Tensor], blk: int) -> torch.Tensor
     return _ln(z + x, sd[p + "layer_norm.weight"], sd[p + "layer_norm.bias"])
 
 
-def hidden_states(ids: torch.Tensor, sd: Dict[str, torch.Tensor]) -> torch.Tensor:
+def hidden_states(ids: torch.Tensor, sd: Dict[str, torch.Tensor],
+                  dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     """model/lru.py:38-41,73-83 -- encoder output at every position, [B, L, 64] fp32.
 
     The sequence is left-padded with zero vectors / False mask to the next power of two before the
-    blocks run and cut back afterwards."""
+    blocks run and cut back afterwards.  `dtype` (e.g. torch.float64) runs the same arithmetic with
+    `sd` cast to it (complex parts too); None computes in the dtypes of `sd`, the reference's fp32."""
+    sd = cast_state_dict(sd, dtype)
     x, mask = embed(ids, sd)
     L = ids.shape[1]
     Lp = 1 << max(0, math.ceil(math.log2(L))) if L > 1 else 1
@@ -111,13 +126,15 @@ def hidden_states(ids: torch.Tensor, sd: Dict[str, torch.Tensor]) -> torch.Tenso
     return x[:, Lp - L:, :]
 
 
-def encode(ids: torch.Tensor, sd: Dict[str, torch.Tensor]) -> torch.Tensor:
+def encode(ids: torch.Tensor, sd: Dict[str, torch.Tensor], dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     """User state = encoder output at the last position (trainer/lru.py:33 takes scores[:, -1])."""
-    return hidden_states(ids, sd)[:, -1, :]
+    return hidden_states(ids, sd, dtype)[:, -1, :]
 
 
-def forward_scores(ids: torch.Tensor, sd: Dict[str, torch.Tensor]) -> torch.Tensor:
+def forward_scores(ids: torch.Tensor, sd: Dict[str, torch.Tensor],
+                   dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     """model/lru.py:85 -- scores at every position, [B, L, N+1] (tied embedding + bias)."""
+    sd = cast_state_dict(sd, dtype)
     return torch.matmul(hidden_states(ids, sd), sd["embedding.token.weight"].t()) + sd["model.bias"]
 
 
