@@ -258,7 +258,11 @@ int lrb_merge_metrics_scatter(const float* list_scores, const int32_t* list_ids,
  * ManualVerbalizer.process_logits (trainer/verb.py:546-586: project -> [normalize -> log] ->
  * aggregate) by computing only the label-word rows of the lm_head.
  *   hidden  [B][H] bf16 last-position hidden states     lm_head [V][H] bf16
- *   word_ids [C][W] int32 first sub-token id of each label word, word_mask [C][W] (0/1)
+ *   H must be one of 256, 512, 768, 1024, 1536, 2048, 3072, 3584, 4096, 5120, 8192 (the instantiated
+ *     kernels); any other H returns LRB_ERR_UNSUPPORTED without touching out.  C * W <= 32.
+ *   word_ids [C][W] int32 first sub-token id of each label word, word_mask [C][W] (0/1).  A token id
+ *     outside [0, V) is read as token 0 (here and in lrb_verbalizer_from_logits): callers must validate
+ *     the ids (ManualVerbalizer raises IndexError, as the reference's indexing does).
  *   mode 0 = raw label logits (post_log_softmax=False, the reference default, trainer/llm.py:96)
  *        1 = log(softmax over all C*W label words + 1e-15)   (post_log_softmax=True)
  *   round_bf16 != 0: round each logit to bf16 first, as a bf16 lm_head GEMM followed by

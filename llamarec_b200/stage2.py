@@ -52,7 +52,11 @@ def rank_candidates(llm, tokenizer, prompt: str, candidates: Sequence[int], verb
 @torch.no_grad()
 def rerank_metrics(scores: torch.Tensor, labels: torch.Tensor, ks: Sequence[int]) -> Dict[str, float]:
     """`compute_metrics_for_ks(ks, verbalizer)` (trainer/llm.py:63-72) for label scores that are already on the
-    device: Recall/MRR/NDCG@ks of the label index among the C candidates, same keys as the reference."""
+    device: Recall/MRR/NDCG@ks of the label index among the C candidates, same keys as the reference.
+
+    Ties are ranked by (score desc, index asc), the merge kernel's order: the label's 0-based rank is the number of
+    candidates with a higher score plus the tied ones with a lower index.  bf16-rounded label logits tie exactly
+    quite often; the reference's `(-scores).argsort()` leaves the order of ties undefined."""
     return absolute_recall_mrr_ndcg_for_ks(scores, labels.view(-1), list(ks))
 
 

@@ -103,6 +103,14 @@ class ManualVerbalizer:
         self.label_words_mask = torch.clamp(words_ids_mask.sum(dim=-1), max=1)   # [C, W]
         self._dev_cache = {}
 
+    def _check_token_ids(self, V: int) -> None:
+        """The reference indexes `logits[:, label_words_ids]` (trainer/verb.py:539), which raises IndexError for a
+        token id >= V; the kernels would read token 0 instead, for a negative id too.  Checked on the host copy of the
+        ids, so no device synchronisation."""
+        lo, hi = int(self.label_words_ids.min()), int(self.label_words_ids.max())
+        if lo < 0 or hi >= V:
+            raise IndexError(f"label word token ids span [{lo}, {hi}], outside the {V} rows of the logits / lm_head")
+
     # ---- fused fast path ---------------------------------------------------------------------------
     def _device_params(self, dev):
         key = str(dev)
@@ -122,6 +130,7 @@ class ManualVerbalizer:
         if self.multi_token_handler != "first":
             raise NotImplementedError("the fused kernel implements multi_token_handler='first' "
                                       "(the reference default, trainer/verb.py:441)")
+        self._check_token_ids(lm_head_weight.shape[0])
         if not hidden_last.is_cuda:
             raise RuntimeError("score_hidden runs on the GPU only (no CPU fallback)")
         lib = _lib.load()
@@ -151,21 +160,24 @@ class ManualVerbalizer:
         device first when there is one."""
         if self.multi_token_handler not in self._HANDLERS:
             raise ValueError(f"multi_token_handler {self.multi_token_handler} not configured")
+        self._check_token_ids(logits.shape[-1])
         if not logits.is_cuda and torch.cuda.is_available():
             return self.process_logits(logits.cuda()).to(logits.device)
         if logits.is_cuda:
             lib = _lib.load()
             dev = logits.device
             lg = logits.to(torch.float32)
-            if lg.stride(-1) != 1:
-                lg = lg.contiguous()
-            ids, tmask, wmask = self._device_token_params(dev)
             B, V = lg.shape
+            # the kernel reads rows at a pitch >= V with unit inner stride: broadcast rows (stride 0) are copied
+            if lg.stride(-1) != 1 or (B > 1 and lg.stride(0) < V):
+                lg = lg.contiguous()
+            ld = lg.stride(0) if B > 1 else V       # the pitch of a single row is never used
+            ids, tmask, wmask = self._device_token_params(dev)
             C, W, T = ids.shape
             out = torch.empty(B, C, dtype=torch.float32, device=dev)
             cal = self._calib_ptr(dev, V)
             with _lib.on_device(lg):
-                _lib.check(lib.lrb_verbalizer_from_logits(lg.data_ptr(), lg.stride(0), B, V, _lib.ptr(ids),
+                _lib.check(lib.lrb_verbalizer_from_logits(lg.data_ptr(), ld, B, V, _lib.ptr(ids),
                                                           _lib.ptr(tmask), _lib.ptr(wmask), C, W, T,
                                                           self._HANDLERS[self.multi_token_handler],
                                                           1 if self.post_log_softmax else 0,

@@ -10,6 +10,7 @@ import torch
 from conftest import CASES, GOLDEN, load_case
 from oracle import dropout_oracle as DO
 from oracle import lru_oracle as O
+from oracle import verbalizer_oracle as VO
 
 F64 = torch.float64
 
@@ -42,6 +43,46 @@ def test_fp64_loss_and_grads_match_reference_autograd(golden_sd, name):
         assert w64.dtype == (np.complex128 if np.iscomplexobj(want) else np.float64), k
         scale = float(np.abs(w64).max())
         np.testing.assert_allclose(w64, want, rtol=1e-4, atol=1e-4 * scale, err_msg=k)
+
+
+def test_fp64_verbalizer_oracle_matches_the_fixtures():
+    """process_logits on float64 inputs computes in float64 and reproduces the reference's own outputs
+    (verbalizer_case.npz, verbalizer_handlers.npz) at the fp32 oracle's tolerances: every handler, both modes,
+    multi-word classes and calibration.  The hidden-state outputs are compared on the bf16 logits the reference's
+    lm_head produced, widened to float64."""
+    from llamarec_b200 import ManualVerbalizer
+
+    class Tok:
+        def encode(self, word, add_special_tokens=False):
+            return [17 + (ord(c) * 7) % 250 for c in word]
+    d = np.load(os.path.join(GOLDEN, "verbalizer_case.npz"))
+    h = np.load(os.path.join(GOLDEN, "verbalizer_handlers.npz"))
+    logits = torch.from_numpy(d["logits"]).to(F64)
+    ids, tm, wm = (torch.from_numpy(d[k]) for k in ("label_words_ids", "words_ids_mask", "label_words_mask"))
+    lg = VO.lm_head_last(torch.from_numpy(d["hidden"]).to(torch.bfloat16),
+                         torch.from_numpy(d["lm_head"]).to(torch.bfloat16)).to(F64)
+    for pls in (0, 1):
+        o = VO.process_logits(logits, ids, tm, wm, bool(pls))
+        assert o.dtype == F64
+        np.testing.assert_allclose(o.numpy(), d[f"out_pls{pls}"], atol=1e-6)
+        np.testing.assert_allclose(VO.process_logits(lg, ids, tm, wm, bool(pls)).numpy(), d[f"hidden_out_pls{pls}"],
+                                   atol=1e-5)
+    ids2, tm2, wm2 = (torch.from_numpy(d[k]) for k in ("multi_label_words_ids", "multi_words_ids_mask",
+                                                       "multi_label_words_mask"))
+    np.testing.assert_allclose(VO.process_logits(logits, ids2, tm2, wm2, True).numpy(), d["multi_out"], atol=1e-6)
+    lw = {i: ([chr(ord("A") + i), "xy" + chr(ord("a") + i)] if i % 4 else [chr(ord("A") + i) + "q"]) for i in range(16)}
+    cal = torch.from_numpy(h["calibrate_logits"]).to(F64)
+    for handler in ("first", "max", "mean"):
+        v = ManualVerbalizer(Tok(), classes=list(range(16)), label_words=lw, prefix="", multi_token_handler=handler)
+        for pls in (0, 1):
+            o = VO.process_logits(logits, v.label_words_ids, v.words_ids_mask, v.label_words_mask, bool(pls), handler)
+            assert o.dtype == F64
+            np.testing.assert_allclose(o.numpy(), h[f"{handler}_pls{pls}"], atol=1e-6)
+        if handler != "max":
+            o = VO.process_logits(logits, v.label_words_ids, v.words_ids_mask, v.label_words_mask, True, handler,
+                                  calibrate_logits=cal)
+            assert o.dtype == F64
+            np.testing.assert_allclose(o.numpy(), h[f"{handler}_calibrated"], atol=1e-5)
 
 
 def test_default_dtype_is_the_fp32_restatement(golden_sd):
