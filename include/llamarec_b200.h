@@ -139,6 +139,42 @@ int lrb_score_dense(const void* x, const void* table, const float* bias_pad, con
                     int64_t M, int64_t rows, int precision, float* out, int64_t ld_out, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Exact fp32 top-K on large catalogues (LRURec.retrieve(precision="exact")): the ranking of the fp32
+ * reference `x @ E^T + bias` (model/lru.py:85) -> torch.topk (trainer/lru.py:82-84) at the speed of the bf16
+ * tensor cores.  The scores and lists equal those of lrb_score_topk precision 1 bit for bit.
+ * eps_u bounds |bf16-operand score - fp32 score| for every item (DESIGN.md section 2.1); it is built from
+ * bound[65] = {c_i = max_j |table_f32[j][i]| over the shard, i < 64; b_max = max_j |bias_j| (0 without bias)}.
+ *
+ * lrb_exact_rescore: pass A.  cand_scores/cand_ids [B][Kc] = the bf16 top-Kc list of every user (lrb_score_topk
+ *   precision 0 merged by lrb_merge_metrics; ids < 0 = missing entries), Kc in [K, LRB_MAX_K].  One warp per user
+ *   rescores the list with the fp32 path's arithmetic and sorts it.  Outputs per user:
+ *     path[b] = 0  certified: out_scores/out_ids [B][K], out_cnt [B] hold the exact list (score desc, id asc)
+ *     path[b] = 1  not certified: every item of the exact top K has a bf16 score >= tau[b]; fk[b] = the K-th best
+ *                  rescored score, a lower bound on the exact K-th best
+ *     path[b] = 2  eps_u or a rescored score is not finite: the user needs lrb_score_topk precision 1
+ * lrb_score_collect: pass B, the tensor-core scores of u_bf16 [M][64] against table_bf16 (+ bias_blk, as for
+ *   lrb_score_dense precision 0); every shard item j (global id row_offset + j) with score >= tau[m] is appended to
+ *   cand_ids[m][0 .. cap) in no particular order.  cand_cnt [M] (zeroed here) counts every such item, also past cap.
+ * lrb_exact_select: for the users[n] rows of the batch (cand_ids/cand_cnt row i belongs to user users[i]): drops
+ *   history ids (excl_sorted, NULL = none) and ids outside the shard, rescores in fp32 and writes the exact top K
+ *   into out_* row users[i].  A user whose cand_cnt exceeds cap, or with a non-finite rescored score, gets
+ *   path = 2 and no list.  cand_ids is overwritten.  Workspace: lrb_exact_select_workspace_bytes(n, cap).
+ * ------------------------------------------------------------------------------------------ */
+int lrb_exact_rescore(const float* u, const float* table_f32, const float* bias_pad, const float* bound, int B,
+                      int64_t rows, int64_t row_offset, const float* cand_scores, const int32_t* cand_ids, int Kc,
+                      int K, float* out_scores, int32_t* out_ids, int32_t* out_cnt, int8_t* path, float* tau,
+                      float* fk, void* stream);
+int lrb_score_collect(const void* u_bf16, const void* table_bf16, const void* bias_blk, int M, int64_t rows,
+                      int64_t row_offset, const float* tau, int cap, int32_t* cand_ids, int32_t* cand_cnt,
+                      void* stream);
+size_t lrb_exact_select_workspace_bytes(int n, int cap);
+int lrb_exact_select(const int32_t* users, int n, const float* u, const float* table_f32, const float* bias_pad,
+                     int64_t rows, int64_t row_offset, const int32_t* excl_sorted, int excl_stride, const float* fk,
+                     int32_t* cand_ids, const int32_t* cand_cnt, int cap, int K, float* out_scores,
+                     int32_t* out_ids, int32_t* out_cnt, int8_t* path, void* workspace, size_t workspace_bytes,
+                     void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Train-step forward loss without the logits tensor.
  * Replaces, in value, LRUTrainer.calculate_loss (trainer/lru.py:22-28): `model(seqs).view(-1, N+1)`
  * followed by nn.CrossEntropyLoss(ignore_index=0) (trainer/lru.py:20) -- an online log-sum-exp over

@@ -34,6 +34,14 @@ SIGNATURES = {
                                c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "lrb_score_dense": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p, c_int64,
                                 c_void_p]),
+    "lrb_exact_rescore": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p,
+                                  c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "lrb_score_collect": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_int, c_void_p,
+                                  c_void_p, c_void_p]),
+    "lrb_exact_select_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "lrb_exact_select": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
+                                 c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                 c_void_p, c_size_t, c_void_p]),
     "lrb_merge_metrics": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int64, c_int64, c_int64, c_int,
                                   c_int, c_int, c_void_p, POINTER(ctypes.c_int32), c_int, c_void_p, c_void_p,
                                   c_int64, c_void_p, c_void_p, c_void_p]),

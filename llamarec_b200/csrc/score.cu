@@ -3,6 +3,8 @@
 //                    precision 1 -> score_topk_f32_kernel (fp32 FFMA, bit-comparable with the
 //                                   fp32 reference `x @ E^T + bias`, model/lru.py:85)
 //   lrb_score_dense  API-compatible dense logits for LRURec.forward
+//   lrb_score_collect  bf16 tensor-core scores, every item at or above a per-user threshold collected
+//                      (candidate pass of precision="exact", see exact.cu)
 #include "api_util.h"
 #include "score_topk_tc.cuh"
 
@@ -515,11 +517,11 @@ int make_tmap_bias_blocks(CUtensorMap* out, const void* ptr, unsigned long long 
 }
 
 // `grid` counts MMA engines: CTAs for CG == 1, CTA pairs (clusters of 2) for CG == 2.
-template <int KMAX, int NS, bool kDense, int CG, int CMAX = tc::MAX_C_SHARE_SMALL>
+template <int KMAX, int NS, bool kDense, int CG, int CMAX = tc::MAX_C_SHARE_SMALL, bool kCollect = false>
 int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tbias, const tc::ScoreParams& p,
               int grid, cudaStream_t st, bool overlap_prev = false) {
   using L = tc::SmemLayout<KMAX, NS, CG>;
-  auto kern = tc::score_topk_tc_kernel<KMAX, NS, kDense, CG, CMAX>;
+  auto kern = tc::score_topk_tc_kernel<KMAX, NS, kDense, CG, CMAX, kCollect>;
   LRB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kAlloc));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid * CG));
@@ -784,6 +786,39 @@ int lrb_score_dense(const void* x, const void* table, const float* bias_pad, con
     if (rc != LRB_OK) return rc;
   }
   return launch_tc<20, 3, true, 1>(ta, tb, tbias, p, d.grid, st);
+}
+
+int lrb_score_collect(const void* u_bf16, const void* table_bf16, const void* bias_blk, int M, int64_t rows,
+                      int64_t row_offset, const float* tau, int cap, int32_t* cand_ids, int32_t* cand_cnt,
+                      void* stream) {
+  using namespace lrb;
+  int rc = check_arch();
+  if (rc != LRB_OK) return rc;
+  LRB_REQUIRE(u_bf16 && table_bf16 && tau && cand_cnt, "lrb_score_collect: null pointer");
+  LRB_REQUIRE(cap >= 0 && (cap == 0 || cand_ids != nullptr), "lrb_score_collect: bad cap / cand_ids");
+  LRB_REQUIRE(M > 0 && rows > 0 && rows + row_offset < INT_MAX && row_offset >= 0, "lrb_score_collect: bad shape");
+  cudaStream_t st = as_stream(stream);
+  const int sms = device_sm_count();
+  // the dense mode's decomposition and launch shape (one CTA per tile, no CTA pairs): the collect pass differs
+  // from it only in the epilogue
+  const Decomp d = decompose(M, rows, sms);
+  CUtensorMap ta, tb;
+  rc = make_tmap_bf16_k64(&ta, u_bf16, static_cast<unsigned long long>(M), tc::BM);
+  if (rc != LRB_OK) return rc;
+  rc = make_tmap_bf16_k64(&tb, table_bf16, static_cast<unsigned long long>(rows), tc::BN);
+  if (rc != LRB_OK) return rc;
+  CUtensorMap tbias = tb;   // placeholder without a bias block (never dereferenced)
+  if (bias_blk != nullptr) {
+    rc = make_tmap_bias_blocks(&tbias, bias_blk, static_cast<unsigned long long>((rows + tc::BN - 1) / tc::BN), tc::BN);
+    if (rc != LRB_OK) return rc;
+  }
+  tc::ScoreParams p = {};
+  p.B = M; p.m_tiles = d.m_tiles; p.rows = static_cast<int>(rows); p.n_tiles = d.n_tiles;
+  p.row_offset = static_cast<int>(row_offset); p.K = 1; p.bias_blk = static_cast<const uint8_t*>(bias_blk);
+  p.s_full = d.s_full; p.rem = d.rem; p.full_tiles = d.full_tiles; p.y_tiles = d.y_tiles;
+  p.collect_tau = tau; p.collect_ids = cand_ids; p.collect_cnt = cand_cnt; p.collect_cap = cap;
+  LRB_CUDA_TRY(cudaMemsetAsync(cand_cnt, 0, static_cast<size_t>(M) * sizeof(int32_t), st));
+  return launch_tc<20, 3, true, 1, tc::MAX_C_SHARE_SMALL, true>(ta, tb, tbias, p, d.grid, st);
 }
 
 }  // extern "C"

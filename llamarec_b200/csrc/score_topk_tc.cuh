@@ -95,6 +95,12 @@ struct ScoreParams {
   int rem;           // CTAs in the shared stream
   int full_tiles;    // item tiles covered by the full streams  [0, full_tiles)
   int y_tiles;       // item tiles covered by the shared stream [full_tiles, n_tiles)
+  // collect mode only (kDense && kCollect): every item of row b with score >= collect_tau[b] is appended to
+  // collect_ids[b][0 .. collect_cap); collect_cnt[b] (zeroed by the host wrapper) counts past the cap
+  const float* collect_tau;
+  int* collect_ids;
+  int* collect_cnt;
+  int collect_cap;
 };
 
 struct Segment {
@@ -438,7 +444,8 @@ LRB_DEVINL uint64_t umma_desc_k16_sw32(uint32_t smem_addr) {
 // ~1500 cycles of hand-offs (remote mbarrier arrivals of the pair's other CTA, the MMA warp's wake-up and issue, the
 // commit's arrival) on top of the MMA itself; throughput = TMEM columns in flight / that cycle, hence four small
 // stages instead of two large ones, and every hand-off kept as short as it goes.
-template <int KMAX, int NS, bool kDense, int CG, int CMAX = MAX_C_SHARE_SMALL>
+// kCollect (with kDense): threshold collect instead of the dense write-out (lrb_score_collect).
+template <int KMAX, int NS, bool kDense, int CG, int CMAX = MAX_C_SHARE_SMALL, bool kCollect = false>
 __global__ void __launch_bounds__(128 + EPI_WARPS * 32, 1)
 score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
                      const __grid_constant__ CUtensorMap tmap_b,
@@ -881,7 +888,29 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
             if (blk == 1) release_half(t);
             const int row = m_own * BM + r;
             const int col0 = n * BN + item_off(blk);
-            if (row < p.B) {
+            if (kCollect) {
+              if (row < p.B) {
+                const float tau = p.collect_tau[row];
+#pragma unroll
+                for (int g = 0; g < 4; ++g) {
+                  float q[16];
+#pragma unroll
+                  for (int j = 0; j < 16; ++j) q[j] = __uint_as_float(v[g * 16 + j]);
+                  const float gm = fmaxf(max3(max3(q[0], q[1], q[2]), max3(q[3], q[4], q[5]), max3(q[6], q[7], q[8])),
+                                         max3(max3(q[9], q[10], q[11]), max3(q[12], q[13], q[14]), q[15]));
+                  if (gm >= tau) {
+                    for (int j = 0; j < 16; ++j) {
+                      const int c = col0 + g * 16 + j;
+                      if (c < p.rows && q[j] >= tau) {
+                        const int slot = atomicAdd(p.collect_cnt + row, 1);
+                        if (slot < p.collect_cap)
+                          p.collect_ids[static_cast<size_t>(row) * p.collect_cap + slot] = p.row_offset + c;
+                      }
+                    }
+                  }
+                }
+              }
+            } else if (row < p.B) {
               float* dstp = p.dense_out + static_cast<size_t>(row) * p.dense_ld + col0;
               if (col0 + HCOLS <= p.rows && (p.dense_ld & 3) == 0) {
 #pragma unroll

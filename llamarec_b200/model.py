@@ -25,6 +25,7 @@ from . import _lib
 from .packing import pack_encoder_weights, unpack_encoder_grads
 
 SMALL_CATALOGUE_ROWS = 1 << 17   # up to here 'auto' precision scores in exact fp32
+EXACT_CAP = 4096                 # precision="exact": collected ids per user before it goes to the fp32 path
 
 
 def _on_model_device(fn):
@@ -185,7 +186,8 @@ class LRURec(nn.Module):
                  precision: str = "auto", u: Optional[torch.Tensor] = None,
                  u_bf16: Optional[torch.Tensor] = None, merge: bool = True,
                  packed_out: Optional[torch.Tensor] = None, seq: Optional[dict] = None,
-                 scatter: Optional[dict] = None, packed_layout: str = "planes") -> Dict[str, torch.Tensor]:
+                 scatter: Optional[dict] = None, packed_layout: str = "planes",
+                 exact_cap: int = EXACT_CAP) -> Dict[str, torch.Tensor]:
         """encode -> catalogue score -> (history mask) -> top-k -> (metrics), all on device.  Eval semantics in either
         mode: no dropout.
 
@@ -200,6 +202,17 @@ class LRURec(nn.Module):
         that were encoded on other ranks.  `scatter` ({"dst_scores": [...], "dst_ids": [...], "users_per_dst": n,
         "out_stride": s} of raw device/peer addresses) makes the merge write every user's list straight into
         the buffer of the rank that owns the user (lrb_merge_metrics_scatter).
+
+        precision: "fp32" scores in exact fp32 (the reference's arithmetic), "bf16" on the tensor cores with bf16
+        operands, "auto" = fp32 up to 131 072 rows, bf16 above.  "exact" returns what "fp32" returns, bit for bit,
+        at close to the bf16 speed on large catalogues (DESIGN section 2.1): the bf16 top-min(50, 2k) list is
+        rescored in fp32 and certified by a per-user error bound; users it cannot certify get every item whose
+        bf16 score reaches a threshold collected (at most `exact_cap` per user) and selected in fp32, and the
+        rest go through the fp32 path.  `exact_path` [B] int8 says which: 0 = certified, 1 = collected,
+        2 = fp32 path (every user on catalogues of up to 131 072 rows); `exact_collected` [B] int32 is the number
+        of ids collected for each user (also past `exact_cap`; 0 where nothing was collected).  An exact call
+        synchronises with the host at most twice, to size the collected and the fp32 sub-batches.  It needs the
+        fp32 states (`u`, or `x`).
         """
         lib = _lib.load()
         c = self._prepare()
@@ -215,12 +228,37 @@ class LRURec(nn.Module):
             B = x.shape[0]
             if seq is None:
                 seq = self._prepare_sequences(x, all_positions=False, want_excl=exclude_history)
+        if prec == 2 and x is None and u is None:
+            raise ValueError('precision="exact" needs the fp32 user states (u), not only u_bf16')
         if u is None and u_bf16 is not None and prec == 0:
             pass                                    # bf16 states supplied by the caller
         elif u is None:
             u, u_bf16, _ = self._encode(x, all_positions=False, want_bf16=(prec == 0), seq=seq)
         elif prec == 0 and u_bf16 is None:
             u_bf16 = u.to(torch.bfloat16).contiguous()
+        if prec == 2:
+            return self._retrieve_exact(u, seq if exclude_history else None, k, labels, ks, merge, packed_out,
+                                        scatter, packed_layout, exact_cap)
+        if precision == "exact":
+            # small catalogue: the fp32 dense + select path is exact already
+            res = self._retrieve_lists(u, u_bf16, 1, seq if exclude_history else None, k, merge, labels, ks,
+                                       packed_out, scatter, packed_layout)
+            res["exact_path"] = torch.full((B,), 2, dtype=torch.int8, device=dev)
+            res["exact_collected"] = torch.zeros(B, dtype=torch.int32, device=dev)
+            return res
+        return self._retrieve_lists(u, u_bf16, prec, seq if exclude_history else None, k, merge, labels, ks,
+                                    packed_out, scatter, packed_layout)
+
+    def _retrieve_lists(self, u, u_bf16, prec, seq, k, merge, labels=None, ks=None, packed_out=None, scatter=None,
+                        packed_layout="planes"):
+        """lrb_score_topk at `prec` (0 = bf16, 1 = fp32) for the rows of u / u_bf16, history of `seq` (None = no
+        exclusion), then the merge unless merge=False."""
+        lib = _lib.load()
+        c = self._prepare()
+        dev = c["table_f32"].device
+        rows = self.row_end - self.row_begin
+        B = (u if u is not None else u_bf16).shape[0]
+        exclude_history = seq is not None
         slots = _lib.c_int(0)
         _lib.check(lib.lrb_score_topk_slots(B, rows, prec, _lib.ctypes.byref(slots)))
         S = slots.value
@@ -239,7 +277,8 @@ class LRURec(nn.Module):
             _lib.ptr(uu), _lib.ptr(table), _lib.ptr(c["bias_pad"]), _lib.ptr(bias_blk), B, rows, self.row_begin,
             _lib.ptr(seq["excl_sorted"]) if exclude_history else None,
             _lib.ptr(seq["excl_bloom"]) if exclude_history else None,
-            seq["excl_stride"], k, prec, _lib.ptr(part_s), _lib.ptr(part_i), _lib.ptr(part_c), S,
+            seq["excl_stride"] if exclude_history else 0, k, prec, _lib.ptr(part_s), _lib.ptr(part_i),
+            _lib.ptr(part_c), S,
             _lib.ptr(scratch), _lib.stream_handle()))
         if self.profile_events is not None:
             ev1.record()
@@ -249,6 +288,78 @@ class LRURec(nn.Module):
         out = merge_lists(part_s, part_i, part_c, k_out=k, labels=labels, ks=ks, packed_out=packed_out,
                           scatter=scatter, packed_layout=packed_layout)
         out["u"] = u
+        return out
+
+    def _retrieve_exact(self, u, seq, k, labels, ks, merge, packed_out, scatter, packed_layout, cap):
+        """precision="exact" on a catalogue shard of more than 131 072 rows (see retrieve)."""
+        lib = _lib.load()
+        c = self._prepare()
+        dev = u.device
+        rows = self.row_end - self.row_begin
+        B = u.shape[0]
+        u = u.contiguous()
+        u_bf16 = u.to(torch.bfloat16)
+        excl = seq["excl_sorted"] if seq is not None else None
+        stride = seq["excl_stride"] if seq is not None else 0
+        # pass A: bf16 top-Kc candidates, rescored in fp32 and certified (Kc = 2k leaves room above the k-th entry
+        # for the certificate's gap; 50 is the kernels' list limit)
+        kc = min(50, 2 * k)
+        cand = self._retrieve_lists(None, u_bf16, 0, seq, kc, merge=True)
+        out_s = torch.empty(B, 1, k, dtype=torch.float32, device=dev)
+        out_i = torch.empty(B, 1, k, dtype=torch.int32, device=dev)
+        out_c = torch.zeros(B, 1, dtype=torch.int32, device=dev)
+        path = torch.empty(B, dtype=torch.int8, device=dev)
+        tau = torch.empty(B, dtype=torch.float32, device=dev)
+        fk = torch.empty(B, dtype=torch.float32, device=dev)
+        _lib.check(lib.lrb_exact_rescore(
+            _lib.ptr(u), _lib.ptr(c["table_f32_shard"]), _lib.ptr(c["bias_pad"]), _lib.ptr(c["exact_bound"]), B, rows,
+            self.row_begin, _lib.ptr(cand["scores"]), _lib.ptr(cand["ids"]), kc, k, _lib.ptr(out_s), _lib.ptr(out_i),
+            _lib.ptr(out_c), _lib.ptr(path), _lib.ptr(tau), _lib.ptr(fk), _lib.stream_handle()))
+        collected = torch.zeros(B, dtype=torch.int32, device=dev)
+        order = torch.argsort(path, stable=True).to(torch.int32)
+        n_cert, n_coll, n_fb = torch.bincount(path.to(torch.int64), minlength=3).tolist()     # host sync 1
+        if n_coll > 0:
+            # pass B: every item whose bf16 score reaches tau, then the exact selection among them
+            users = order[n_cert:n_cert + n_coll].contiguous()
+            ub = u_bf16.index_select(0, users)
+            tb = tau.index_select(0, users)
+            cap = max(int(cap), 0)
+            ids = torch.empty(n_coll, max(cap, 1), dtype=torch.int32, device=dev)
+            cnt = torch.empty(n_coll, dtype=torch.int32, device=dev)
+            _lib.check(lib.lrb_score_collect(_lib.ptr(ub), _lib.ptr(c["table_bf16"]), _lib.ptr(c["bias_blk"]), n_coll,
+                                             rows, self.row_begin, _lib.ptr(tb), cap, _lib.ptr(ids), _lib.ptr(cnt),
+                                             _lib.stream_handle()))
+            ws_bytes = lib.lrb_exact_select_workspace_bytes(n_coll, cap)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            _lib.check(lib.lrb_exact_select(
+                _lib.ptr(users), n_coll, _lib.ptr(u), _lib.ptr(c["table_f32_shard"]), _lib.ptr(c["bias_pad"]), rows,
+                self.row_begin, _lib.ptr(excl), stride, _lib.ptr(fk), _lib.ptr(ids), _lib.ptr(cnt), cap, k,
+                _lib.ptr(out_s), _lib.ptr(out_i), _lib.ptr(out_c), _lib.ptr(path), _lib.ptr(ws), ws_bytes,
+                _lib.stream_handle()))
+            collected[users.to(torch.int64)] = cnt
+            fb = torch.nonzero(path == 2).flatten().to(torch.int32)                        # host sync 2
+            n_fb = fb.numel()
+        else:
+            fb = order[n_cert:]
+        if n_fb > 0:
+            # users without a finite bound, or with more than `cap` collected ids: the fp32 path
+            fb64 = fb.to(torch.int64)
+            sub = None
+            if seq is not None:
+                sub = {"excl_sorted": seq["excl_sorted"].index_select(0, fb64).contiguous(),
+                       "excl_bloom": seq["excl_bloom"].index_select(0, fb64).contiguous(), "excl_stride": stride}
+            r = self._retrieve_lists(u.index_select(0, fb64).contiguous(), None, 1, sub, k, merge=True)
+            out_s[fb64, 0] = r["scores"]
+            out_i[fb64, 0] = r["ids"]
+            out_c[fb64, 0] = (r["ids"] >= 0).sum(1, dtype=torch.int32)
+        if not merge:
+            return {"part_scores": out_s, "part_ids": out_i, "part_cnt": out_c, "u": u, "exact_path": path,
+                    "exact_collected": collected}
+        out = merge_lists(out_s, out_i, out_c, k_out=k, labels=labels, ks=ks, packed_out=packed_out, scatter=scatter,
+                          packed_layout=packed_layout)
+        out["u"] = u
+        out["exact_path"] = path
+        out["exact_collected"] = collected
         return out
 
     def ce_loss(self, x: torch.Tensor, labels: torch.Tensor, ignore_index: int = 0,
@@ -360,8 +471,12 @@ class LRURec(nn.Module):
     # ------------------------------------------------------------------ internals
     @staticmethod
     def _precision(precision: str, rows: int) -> int:
+        """0 = bf16, 1 = fp32, 2 = the exact mode's bf16 candidates + fp32 rescoring (above SMALL_CATALOGUE_ROWS;
+        at or below it "exact" is the fp32 path)."""
         if precision == "auto":
             return 1 if rows <= SMALL_CATALOGUE_ROWS else 0
+        if precision == "exact":
+            return 1 if rows <= SMALL_CATALOGUE_ROWS else 2
         if precision in ("fp32", "f32", 1):
             return 1
         if precision in ("bf16", 0):
@@ -403,9 +518,14 @@ class LRURec(nn.Module):
         _lib.check(lib.lrb_prepare_table(_lib.ptr(table_f32), _lib.ptr(bias), self.row_begin, rows,
                                          _lib.ptr(table_bf16), _lib.ptr(bias_pad), _lib.ptr(bias_blk),
                                          _lib.stream_handle()))
+        # precision="exact": c_i = max_j |E[j, i]| over the shard's rows, then b_max = max_j |bias_j| (0 without a
+        # bias block); the per-user error bound of the bf16 scores is built from them (DESIGN section 2.1)
+        shard = table_f32[self.row_begin:self.row_end]
+        b_max = bias[self.row_begin:self.row_end].abs().amax() if has_bias else torch.zeros((), device=dev)
+        exact_bound = torch.cat([shard.abs().amax(0), b_max.reshape(1)]).contiguous()
         self._cache = {
             "blob": blob, "table_f32": table_f32, "table_bf16": table_bf16, "bias_pad": bias_pad,
-            "bias_blk": bias_blk, "table_f32_shard": table_f32[self.row_begin:self.row_end],
+            "bias_blk": bias_blk, "table_f32_shard": shard, "exact_bound": exact_bound,
             "n_blocks": len(self.model.lru_blocks),
         }
         self._prepared_sig = sig

@@ -16,9 +16,13 @@ from .metrics import absolute_metrics_batch_wrapper, metrics_from_sums
 
 
 class LRURetriever:
-    def __init__(self, args, model, val_loader=None, test_loader=None, device: Optional[str] = None):
+    def __init__(self, args, model, val_loader=None, test_loader=None, device: Optional[str] = None,
+                 precision: str = "auto"):
+        """`precision` is handed to LRURec.retrieve: "auto" (default), "fp32", "bf16" or "exact" (the fp32 ranking
+        at close to the bf16 speed on large catalogues)."""
         self.args = args
         self.model = model
+        self.precision = precision
         self.val_loader = val_loader
         self.test_loader = test_loader
         self.metric_ks: List[int] = list(getattr(args, "metric_ks", None) or [1, 5, 10, 20, 50])
@@ -42,7 +46,8 @@ class LRURetriever:
         """Batch-mean Recall/MRR/NDCG@ks, keys in the reference's order (k descending)."""
         seqs, labels = batch
         ks = self.metric_ks
-        res = self.model.retrieve(seqs, k=max(ks), exclude_history=exclude_history, labels=labels.view(-1), ks=ks)
+        res = self.model.retrieve(seqs, k=max(ks), exclude_history=exclude_history, labels=labels.view(-1), ks=ks,
+                                  precision=self.precision)
         m = metrics_from_sums(res["metric_sums"], ks, seqs.shape[0])
         return {key: m[key] for k in sorted(ks, reverse=True)
                 for key in ("Recall@%d" % k, "MRR@%d" % k, "NDCG@%d" % k)}
@@ -63,7 +68,7 @@ class LRURetriever:
         for batch in loader:
             seqs, labels = self.to_device(batch)
             labels = labels.view(-1)
-            res = self.model.retrieve(seqs, k=k, exclude_history=True, labels=labels, ks=ks)
+            res = self.model.retrieve(seqs, k=k, exclude_history=True, labels=labels, ks=ks, precision=self.precision)
             sums += res["metric_sums"].double().cpu()
             ids = res["ids"].cpu()
             rank = res["label_rank"].cpu()

@@ -50,6 +50,9 @@ class CudaBackend:
     """Product backend: llamarec_b200.LRURec restricted to this rank's row shard."""
 
     def __init__(self, model, rank: int, world: int, precision: str = "auto"):
+        if precision == "exact":
+            # _precision would resolve it to a per-shard choice; exact retrieval across row shards is not built
+            raise ValueError('precision="exact" is not supported by the sharded backend (use LRURec.retrieve)')
         self.model = model
         # 'auto' is resolved ONCE from the whole catalogue, not from this rank's shard: shard_range gives the
         # last rank a shorter shard, and ranks that disagree would exchange states of different widths and
