@@ -39,7 +39,8 @@ extern "C" {
 #define LRB_H 128         /* complex LRU state width (2*d), model/lru.py:105         */
 #define LRB_FF 256        /* PFFN inner width (4*d), model/lru.py:96                 */
 #define LRB_MAX_LEN 256   /* max sequence length (ML-100k uses 200, config.py:59)    */
-#define LRB_MAX_K 50      /* max top-k list length (= max of metric_ks, config.py:137) */
+#define LRB_MAX_K 50      /* max top-k list length of the streaming kernels (= max of metric_ks, config.py:137) */
+#define LRB_MAX_K_WIDE 1024 /* max top-k list length of the dense + select and the wide paths */
 
 const char* lrb_last_error(void);
 int lrb_version(void);
@@ -125,6 +126,10 @@ int lrb_encode_fwd(const void* ids, int id_bytes, int B, int L, const float* tab
  *   (BaseTrainer.validate calls calculate_metrics(exclude_history=False), trainer/base.py:141).
  * Outputs (caller allocated): part_scores/part_ids [B][slots][K], part_cnt [B][slots];
  *   scratch: lrb_score_scratch_bytes(B) (both precisions).
+ * K: 1..LRB_MAX_K on every path.  K in (LRB_MAX_K, LRB_MAX_K_WIDE] only at precision 1 on the dense + select path
+ *   (slots == 1, rows <= ~568 k on 148 SMs), and only when K <= rows (LRB_ERR_BAD_ARG otherwise, as torch.topk
+ *   refuses k > N+1); elsewhere it returns LRB_ERR_UNSUPPORTED (the bf16 path has lrb_wide_*).  K > LRB_MAX_K_WIDE:
+ *   LRB_ERR_BAD_ARG.
  * ------------------------------------------------------------------------------------------ */
 int lrb_score_topk_slots(int B, int64_t rows, int precision, int* slots);
 size_t lrb_score_scratch_bytes(int B);
@@ -173,6 +178,43 @@ int lrb_exact_select(const int32_t* users, int n, const float* u, const float* t
                      int32_t* cand_ids, const int32_t* cand_cnt, int cap, int K, float* out_scores,
                      int32_t* out_ids, int32_t* out_cnt, int8_t* path, void* workspace, size_t workspace_bytes,
                      void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Wide top-K on the bf16 path: K in (LRB_MAX_K, LRB_MAX_K_WIDE] (LRURec.retrieve(k > 50), DESIGN.md section 2.2).
+ * Every score is the single-CTA tensor-core score of lrb_score_dense precision 0.  Per call:
+ *   1. lrb_wide_sample_threshold: tau[b] = the m-th best score of user b over the shard rows j = 0 (mod r), its
+ *      history excluded (-inf when fewer than m such rows are admissible).  The rows are read through strided
+ *      tensor maps over table_bf16 / bias_blk (no copy); the exclusion list (excl_sorted, NULL = none) is mapped
+ *      onto the lattice inside.  m in [1, LRB_MAX_K], r >= 1.  Workspace:
+ *      lrb_wide_sample_workspace_bytes(B, rows, excl_stride, r, m) (excl_stride 0 without exclusion).
+ *   2. lrb_score_collect_scores: lrb_score_collect that also writes the score of every stored id to
+ *      cand_scores[m][slot] (bit-equal to lrb_score_dense precision 0).  History items are collected too.
+ *   3. lrb_wide_select: one warp per user selects the top K by (score desc, id asc), history ids (excl_sorted) and
+ *      ids outside the shard dropped, -inf and NaN scores never emitted.  Row i of the input belongs to user
+ *      users[i]; the list goes to out_scores/out_ids [B][K], out_cnt [B] at row users[i].  Two loaders:
+ *      - cand_scores != NULL: candidate lists cand_scores/cand_ids [n][cap], cand_cnt [n] of step 2 (compacted in
+ *        place).  path[users[i]] = ok_path when cand_cnt <= cap and at least K admissible items were collected (the
+ *        list is exact: every item >= tau was collected and the K-th best is >= tau); = -1 on overflow
+ *        (cand_cnt > cap with >= K admissible stored items), no list, tau_out[users[i]] = the K-th best stored
+ *        admissible score, a valid threshold for a second collect; = -2 otherwise (short), no list.
+ *      - cand_scores == NULL: dense bf16 rows of u_bf16 [n][64] (row i = user users[i]) against table_bf16 /
+ *        bias_blk, scored in blocks of ~1 GiB of workspace (lrb_wide_select_workspace_bytes(n, rows)); always exact,
+ *        path = ok_path, lists shorter than K when fewer items are admissible.
+ *      K <= rows (LRB_ERR_BAD_ARG otherwise).  ok_path in [0, 127].
+ * ------------------------------------------------------------------------------------------ */
+size_t lrb_wide_sample_workspace_bytes(int B, int64_t rows, int excl_stride, int r, int m);
+int lrb_wide_sample_threshold(const void* u_bf16, const void* table_bf16, const void* bias_blk, int B, int64_t rows,
+                              int64_t row_offset, const int32_t* excl_sorted, int excl_stride, int r, int m,
+                              float* tau, void* workspace, size_t workspace_bytes, void* stream);
+int lrb_score_collect_scores(const void* u_bf16, const void* table_bf16, const void* bias_blk, int M, int64_t rows,
+                             int64_t row_offset, const float* tau, int cap, int32_t* cand_ids, float* cand_scores,
+                             int32_t* cand_cnt, void* stream);
+size_t lrb_wide_select_workspace_bytes(int n, int64_t rows);
+int lrb_wide_select(const int32_t* users, int n, const void* u_bf16, const void* table_bf16, const void* bias_blk,
+                    int64_t rows, int64_t row_offset, const int32_t* excl_sorted, int excl_stride, float* cand_scores,
+                    int32_t* cand_ids, const int32_t* cand_cnt, int cap, int K, int ok_path, float* out_scores,
+                    int32_t* out_ids, int32_t* out_cnt, int8_t* path, float* tau_out, void* workspace,
+                    size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Train-step forward loss without the logits tensor.

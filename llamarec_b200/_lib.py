@@ -42,6 +42,15 @@ SIGNATURES = {
     "lrb_exact_select": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
                                  c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                  c_void_p, c_size_t, c_void_p]),
+    "lrb_wide_sample_workspace_bytes": (c_size_t, [c_int, c_int64, c_int, c_int, c_int]),
+    "lrb_wide_sample_threshold": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_int,
+                                          c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "lrb_score_collect_scores": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_int,
+                                         c_void_p, c_void_p, c_void_p, c_void_p]),
+    "lrb_wide_select_workspace_bytes": (c_size_t, [c_int, c_int64]),
+    "lrb_wide_select": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int,
+                                c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "lrb_merge_metrics": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int64, c_int64, c_int64, c_int,
                                   c_int, c_int, c_void_p, POINTER(ctypes.c_int32), c_int, c_void_p, c_void_p,
                                   c_int64, c_void_p, c_void_p, c_void_p]),

@@ -84,6 +84,48 @@ __global__ void __launch_bounds__(WARPS * 32) merge_metrics_kernel(const Params 
     const int* id = p.list_ids + static_cast<size_t>(b) * p.stride_user;
     const int total_slots = p.n_lists * p.K_in;
     const bool in_regs = total_slots <= 32 * PER_LANE;
+    float* out_s = p.top_scores + static_cast<size_t>(b) * p.out_stride;
+    int* out_i = p.top_ids + static_cast<size_t>(b) * p.out_stride;
+    if (p.users_per_dst > 0) {
+      const int d = b / p.users_per_dst;
+      const size_t row = static_cast<size_t>(b - d * p.users_per_dst);
+      out_s = p.dst_scores[d] + row * p.out_stride;
+      out_i = p.dst_ids[d] + row * p.out_stride;
+    }
+    int my_rank = -1;
+    const long long label = p.labels ? p.labels[b] : -1;
+    // One list that is already sorted -- strictly by (score key desc, id asc), every entry finite or +inf -- is its
+    // own merge (the one list per user of the select paths): one warp pass checks it and it is copied instead of
+    // running K_out selection rounds.  Same output as the rounds.
+    bool copied = false;
+    if (p.n_lists == 1) {
+      int cnt = p.list_cnt ? p.list_cnt[static_cast<size_t>(b) * p.cnt_stride_user] : p.K_in;
+      cnt = cnt < p.K_in ? cnt : p.K_in;
+      bool ok = true;
+      for (int i = lane; i < cnt; i += 32) {
+        const float s = sc[i];
+        const int d = id[i];
+        const int k = float_to_key(s);
+        ok = ok && s > -INFINITY && d != INT_MAX;      // (false for NaN too)
+        if (i + 1 < cnt) {
+          const int k1 = float_to_key(sc[i + 1]);
+          ok = ok && (k > k1 || (k == k1 && d < id[i + 1]));
+        }
+      }
+      copied = __all_sync(0xffffffffu, ok);
+      if (copied) {
+        for (int k = lane; k < p.K_out; k += 32) {
+          const bool v = k < cnt;
+          const int d = v ? id[k] : -1;
+          out_s[k] = v ? sc[k] : -INFINITY;
+          out_i[k] = d;
+          const unsigned hit = __ballot_sync(__activemask(), v && static_cast<long long>(d) == label);
+          if (my_rank < 0 && hit) my_rank = (k - lane) + __ffs(hit) - 1;
+        }
+        my_rank = __reduce_max_sync(0xffffffffu, my_rank);
+      }
+    }
+    if (!copied) {
 
     float es[PER_LANE];
     int ei[PER_LANE];
@@ -105,16 +147,6 @@ __global__ void __launch_bounds__(WARPS * 32) merge_metrics_kernel(const Params 
       }
     }
 
-    float* out_s = p.top_scores + static_cast<size_t>(b) * p.out_stride;
-    int* out_i = p.top_ids + static_cast<size_t>(b) * p.out_stride;
-    if (p.users_per_dst > 0) {
-      const int d = b / p.users_per_dst;
-      const size_t row = static_cast<size_t>(b - d * p.users_per_dst);
-      out_s = p.dst_scores[d] + row * p.out_stride;
-      out_i = p.dst_ids[d] + row * p.out_stride;
-    }
-    int my_rank = -1;
-    const long long label = p.labels ? p.labels[b] : -1;
     // floor for the global-memory path: entries must be strictly "after" the previous winner
     float prev_s = INFINITY;
     int prev_id = -1;
@@ -123,6 +155,8 @@ __global__ void __launch_bounds__(WARPS * 32) merge_metrics_kernel(const Params 
     // stores over NVLink (8-GPU step: 132 us for 32768 users before this change)
     float res_s[2] = {-INFINITY, -INFINITY};
     int res_i[2] = {-1, -1};
+    float wide_s = -INFINITY;
+    int wide_i = -1;
     for (int k = 0; k < p.K_out; ++k) {
       float w_s;
       int w_id;
@@ -182,14 +216,18 @@ __global__ void __launch_bounds__(WARPS * 32) merge_metrics_kernel(const Params 
         if (k < 32) { res_s[0] = valid ? w_s : -INFINITY; res_i[0] = valid ? w_id : -1; }
         else if (k < 64) { res_s[1] = valid ? w_s : -INFINITY; res_i[1] = valid ? w_id : -1; }
       }
-      if (k >= 64 && lane == 0) {   // (lists longer than 64 entries: not used by any caller, kept correct)
-        out_s[k] = valid ? w_s : -INFINITY;
-        out_i[k] = valid ? w_id : -1;
+      if (k >= 64) {   // wide lists (K_out > 64): entries staged per group of 32, one coalesced store per group
+        if (lane == (k & 31)) { wide_s = valid ? w_s : -INFINITY; wide_i = valid ? w_id : -1; }
+        if ((k & 31) == 31 || k == p.K_out - 1) {
+          const int g = k & ~31;
+          if (g + lane <= k) { out_s[g + lane] = wide_s; out_i[g + lane] = wide_i; }
+        }
       }
       if (valid && my_rank < 0 && static_cast<long long>(w_id) == label) my_rank = k;
     }
     if (lane < p.K_out) { out_s[lane] = res_s[0]; out_i[lane] = res_i[0]; }
     if (lane + 32 < p.K_out) { out_s[lane + 32] = res_s[1]; out_i[lane + 32] = res_i[1]; }
+    }
     if (p.label_rank && lane == 0) p.label_rank[b] = my_rank;
     if (p.labels && my_rank >= 0 && lane == 0) {
       // one relevant item per user: Recall@k = [r<k], MRR@k = [r<k]/(r+1), NDCG@k = [r<k]/log2(r+2)

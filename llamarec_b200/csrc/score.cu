@@ -4,7 +4,10 @@
 //                                   fp32 reference `x @ E^T + bias`, model/lru.py:85)
 //   lrb_score_dense  API-compatible dense logits for LRURec.forward
 //   lrb_score_collect  bf16 tensor-core scores, every item at or above a per-user threshold collected
-//                      (candidate pass of precision="exact", see exact.cu)
+//                      (candidate pass of precision="exact", see exact.cu); lrb_score_collect_scores also
+//                      stores the collected scores (candidate pass of the wide top-K)
+//   lrb_wide_sample_threshold / lrb_wide_select  top-K lists of up to LRB_MAX_K_WIDE entries on the bf16 path
+//                      (DESIGN.md section 2.2)
 #include "api_util.h"
 #include "score_topk_tc.cuh"
 
@@ -177,8 +180,18 @@ inline int splits_for(int B, long long rows, int sms, int ctas_per_sm = 2) {
 //   3. one more pass collecting everything above the K-th key plus the lowest-id entries equal to it,
 //   4. a rank sort of the <= K survivors into (score desc, id asc) order.
 // The output is ONE sorted list per user (slots == 1), in the part_* layout the merge kernel consumes.
+//
+// Lists longer than 64 entries (K in [51, LRB_MAX_K_WIDE], CAP = 1024) take the wide variant of the kernel: the radix
+// select runs on a 64-bit key (score key, then ~id), so the K selected entries are exactly the K best by
+// (score desc, id asc) whatever order they are read in; it stops after the 8-bit pass whose bin holds exactly the
+// entries still needed (the 4 score passes unless the K-th score is tied).  A warp-wide bitonic sort of the <= 1024
+// survivors in shared memory replaces the rank sort.  Its loader is either a dense score row (implicit ids, as
+// above) or an explicit candidate list of (score, id) pairs (kCand: the collect pass of the wide bf16 top-K,
+// lrb_wide_select), whose history / out-of-shard ids are dropped first.
 // --------------------------------------------------------------------------------------------
 constexpr int SEL_WARPS = 8;
+constexpr int SEL_WARPS_WIDE = 4;   // 4 x (4 KB histogram + 8 KB of 64-bit keys) = 48 KB of static shared memory
+constexpr int SEL_CAP_WIDE = 1024;
 
 struct SelParams {
   float* dense;          // [nb][ld] scores of this user block (scratch; the history mask is written into it)
@@ -193,11 +206,28 @@ struct SelParams {
   int* part_cnt;         // [B]
 };
 
+// the wide variant's parameters (K > 64), kept out of SelParams so that the K <= 64 kernel compiles as before
+struct SelParamsWide : SelParams {
+  const int* users;      // row i of the block belongs to user users[i] (null: user b0 + i)
+  float* cand_scores;    // kCand: [nb][cap] collected (score, id) pairs, compacted in place
+  int* cand_ids;
+  const int* cand_cnt;   // [nb] collected items, also past cap
+  int cap;
+  int8_t* path;          // [B] (null: not written) ok_path / -1 overflow, tau_out valid / -2 short
+  int ok_path;
+  float* tau_out;        // [B] overflow: the K-th best admissible score among the stored pairs
+};
+
 LRB_DEVINL unsigned sel_key(float v) {   // order-preserving unsigned key; NaN sorts below everything
   return (v == v) ? (static_cast<unsigned>(float_to_key(v)) ^ 0x80000000u) : 0u;
 }
 
-__global__ void __launch_bounds__(SEL_WARPS * 32) select_topk_kernel(const SelParams p) {
+template <int CAP, bool kCand, class Prm = SelParamsWide>
+__global__ void __launch_bounds__((CAP <= 64 ? SEL_WARPS : SEL_WARPS_WIDE) * 32) select_topk_kernel(const Prm p);
+
+// K <= 64 (CAP == 64): dense rows only
+template <>
+__global__ void __launch_bounds__(SEL_WARPS * 32) select_topk_kernel<64, false, SelParams>(const SelParams p) {
   __shared__ unsigned s_hist[SEL_WARPS][4 * 256];
   __shared__ float s_sc[SEL_WARPS][64];
   __shared__ int s_id[SEL_WARPS][64];
@@ -349,6 +379,203 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) select_topk_kernel(const SelPa
   if (lane == 0) p.part_cnt[b] = n_valid;
 }
 
+LRB_DEVINL unsigned long long sel_key64(float v, int id) {
+  return (static_cast<unsigned long long>(sel_key(v)) << 32) | static_cast<unsigned>(~id);
+}
+LRB_DEVINL float sel_key_score(unsigned long long k) {
+  return key_to_float(static_cast<int>(static_cast<unsigned>(k >> 32) ^ 0x80000000u));
+}
+
+template <int CAP, bool kCand, class Prm>
+__global__ void __launch_bounds__(SEL_WARPS_WIDE * 32) select_topk_kernel(const Prm p) {
+  static_assert(CAP == SEL_CAP_WIDE, "wide variant");
+  __shared__ unsigned s_hist[SEL_WARPS_WIDE][4 * 256];
+  __shared__ unsigned long long s_key[SEL_WARPS_WIDE][CAP];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int bl = blockIdx.x * SEL_WARPS_WIDE + warp;
+  if (bl >= p.nb) return;                       // (no block-level barrier below)
+  const int b = p.users != nullptr ? p.users[bl] : p.b0 + bl;
+  const int* ex = p.excl_sorted != nullptr ? p.excl_sorted + static_cast<size_t>(b) * p.excl_stride : nullptr;
+  unsigned* hist = s_hist[warp];
+  unsigned long long* keys = s_key[warp];
+  const unsigned lt_mask = (1u << lane) - 1u;
+
+  // 1. loader: n entries, entry j = (score, id)
+  float* row = nullptr;
+  int* cid = nullptr;
+  int n = 0, cnt = 0;
+  if constexpr (kCand) {
+    cnt = p.cand_cnt[bl];
+    const int stored = cnt < p.cap ? cnt : p.cap;
+    row = p.cand_scores + static_cast<size_t>(bl) * p.cap;
+    cid = p.cand_ids + static_cast<size_t>(bl) * p.cap;
+    // drop history ids and ids outside the shard (compaction in place: writes only to positions <= those read)
+    for (int base = 0; base < stored; base += 32) {
+      const int j = base + lane;
+      const int id = j < stored ? cid[j] : -1;
+      const float v = j < stored ? row[j] : 0.f;
+      const long long local = static_cast<long long>(id) - p.row_offset;
+      bool ok = j < stored && local >= 0 && local < p.rows;
+      if (ok && ex != nullptr) {
+        int lo = 0, hi = p.excl_stride;
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (__ldg(ex + mid) < id) lo = mid + 1; else hi = mid;
+        }
+        ok = !(lo < p.excl_stride && __ldg(ex + lo) == id);
+      }
+      const unsigned bal = __ballot_sync(0xffffffffu, ok);
+      __syncwarp();
+      if (ok) {
+        const int idx = n + __popc(bal & lt_mask);
+        cid[idx] = id;
+        row[idx] = v;
+      }
+      n += __popc(bal);
+    }
+  } else {
+    row = p.dense + static_cast<size_t>(bl) * p.ld;
+    n = p.rows;
+    if (ex != nullptr) {                        // the history mask, as in the K <= 64 variant
+      for (int j = lane; j < p.excl_stride; j += 32) {
+        const int id = ex[j];
+        const long long col = static_cast<long long>(id) - p.row_offset;
+        if (id != INT_MAX && col >= 0 && col < n) row[col] = -INFINITY;
+      }
+    }
+  }
+  __syncwarp();
+  auto key_at = [&](int j) -> unsigned long long {
+    if constexpr (kCand) return sel_key64(row[j], cid[j]);
+    else return sel_key64(row[j], j + p.row_offset);
+  };
+
+  // 2. radix select of the K_eff-th largest 64-bit key, 8 bits per pass
+  const int K_eff = p.K < n ? p.K : n;
+  unsigned long long prefix = 0ull;
+  int need = K_eff;
+  int bits = 0;                                 // leading key bits that decide: entries with top bits >= prefix's
+#pragma unroll 1
+  for (int pass = 0; pass < 8 && need > 0; ++pass) {
+    const int shift = 56 - 8 * pass;
+    const unsigned long long hi_mask = pass == 0 ? 0ull : (~0ull << (shift + 8));
+#pragma unroll
+    for (int j = 0; j < 32; ++j) hist[lane + 32 * j] = 0u;
+    __syncwarp();
+    unsigned* my_hist = hist + (lane & 3) * 256;
+    for (int base = lane; base < n; base += 128) {
+      unsigned long long kk[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) kk[q] = (base + 32 * q < n) ? key_at(base + 32 * q) : 0ull;
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        if (base + 32 * q < n && (kk[q] & hi_mask) == prefix)
+          atomicAdd(&my_hist[static_cast<unsigned>(kk[q] >> shift) & 255u], 1u);
+    }
+    __syncwarp();
+    unsigned own[8];
+    unsigned mine = 0u;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int bi = lane * 8 + j;
+      own[j] = hist[bi] + hist[256 + bi] + hist[512 + bi] + hist[768 + bi];
+      mine += own[j];
+    }
+    unsigned incl = mine;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned v = __shfl_down_sync(0xffffffffu, incl, o);
+      if (lane + o < 32) incl += v;
+    }
+    const unsigned above = incl - mine;
+    const bool holder = above < static_cast<unsigned>(need) && static_cast<unsigned>(need) <= incl;
+    int bin = 0;
+    unsigned above_bin = 0u, bin_cnt = 0u;
+    if (holder) {
+      unsigned acc = above;
+#pragma unroll
+      for (int j = 7; j >= 0; --j) {
+        if (acc < static_cast<unsigned>(need) && static_cast<unsigned>(need) <= acc + own[j]) {
+          bin = lane * 8 + j; above_bin = acc; bin_cnt = own[j];
+        }
+        acc += own[j];
+      }
+    }
+    const int src = __ffs(__ballot_sync(0xffffffffu, holder)) - 1;
+    bin = __shfl_sync(0xffffffffu, bin, src);
+    above_bin = __shfl_sync(0xffffffffu, above_bin, src);
+    bin_cnt = __shfl_sync(0xffffffffu, bin_cnt, src);
+    prefix |= static_cast<unsigned long long>(bin) << shift;
+    need -= static_cast<int>(above_bin);
+    bits = 8 * (pass + 1);
+    __syncwarp();
+    if (bin_cnt == static_cast<unsigned>(need)) break;   // every entry of the bin is wanted (keys are distinct)
+  }
+
+  // 3. collect the K_eff entries whose leading `bits` bits reach the prefix's
+  int ns = 0;
+  if (K_eff > 0) {
+    const int sh = 64 - bits;
+    const unsigned long long thr = prefix >> sh;
+    for (int base = 0; base < n; base += 128) {
+      unsigned long long kk[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) kk[q] = (base + 32 * q + lane < n) ? key_at(base + 32 * q + lane) : 0ull;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const bool sel = base + 32 * q + lane < n && (kk[q] >> sh) >= thr;
+        const unsigned bs = __ballot_sync(0xffffffffu, sel);
+        const int idx = ns + __popc(bs & lt_mask);
+        if (sel && idx < CAP) keys[idx] = kk[q];
+        ns += __popc(bs);
+      }
+      if (ns >= K_eff) break;                   // warp-uniform
+    }
+    ns = ns < K_eff ? ns : K_eff;
+  }
+  // 4. bitonic sort (descending) of the survivors, padded with key 0 to a power of two
+  int P = 32;
+  while (P < ns) P <<= 1;
+  for (int j = ns + lane; j < P; j += 32) keys[j] = 0ull;
+  __syncwarp();
+  for (int k = 2; k <= P; k <<= 1) {
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      for (int i = lane; i < P; i += 32) {
+        const int ixj = i ^ j;
+        if (ixj > i) {
+          const unsigned long long a = keys[i], c = keys[ixj];
+          if (((i & k) == 0) ? (a < c) : (a > c)) { keys[i] = c; keys[ixj] = a; }
+        }
+      }
+      __syncwarp();
+    }
+  }
+  // 5. -inf (masked / padding) and NaN entries sort last and are not emitted
+  const unsigned long long lowest = static_cast<unsigned long long>(sel_key(-INFINITY)) << 32 | 0xffffffffull;
+  int n_valid = 0;
+  for (int base = 0; base < ns; base += 32) {
+    const int j = base + lane;
+    n_valid += __popc(__ballot_sync(0xffffffffu, j < ns && keys[j] > lowest));
+  }
+  int8_t st = static_cast<int8_t>(p.ok_path);
+  if constexpr (kCand) {
+    if (n_valid < p.K) st = -2;                 // short: tau was above the K-th best, or too few admissible items
+    else if (cnt > p.cap) st = -1;              // overflow: retry at the K-th best stored score
+  }
+  if (st >= 0) {
+    for (int j = lane; j < n_valid; j += 32) {
+      const unsigned long long k = keys[j];
+      p.part_scores[static_cast<size_t>(b) * p.K + j] = sel_key_score(k);
+      p.part_ids[static_cast<size_t>(b) * p.K + j] = static_cast<int>(~static_cast<unsigned>(k));
+    }
+    if (lane == 0) p.part_cnt[b] = n_valid;
+  }
+  if (lane == 0) {
+    if (p.path != nullptr) p.path[b] = st;
+    if (st == -1) p.tau_out[b] = sel_key_score(keys[p.K - 1]);
+  }
+}
+
 // users whose score rows fit in `bytes` of scratch (multiple of 128, the dense kernel's user tile), 0 = none
 inline long long select_block_users(long long rows, size_t bytes) {
   const long long ld = (rows + 3) / 4 * 4;
@@ -378,6 +605,51 @@ int launch_dense(const float* x, const float* table, const float* bias_pad, int 
 }
 
 }  // namespace f32
+
+// ============================================================================================
+// Wide top-K helpers (lrb_wide_sample_threshold)
+// ============================================================================================
+namespace wide {
+
+__global__ void fill_kernel(float* out, int n, float v) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = v;
+}
+
+// The exclusion list of the lattice view (row i of the view = shard row r * i): shard-local ids divisible by r, as
+// view rows, ascending and INT_MAX padded, with their bloom filter (the layout of lrb_prepare_sequences).  One warp
+// per user.
+__global__ void __launch_bounds__(256) lattice_excl_kernel(const int* excl, int stride, int B, int row_offset, int rows,
+                                                           int r, int* out, uint32_t* bloom) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int b = blockIdx.x * 8 + warp;
+  if (b >= B) return;
+  const int* ex = excl + static_cast<size_t>(b) * stride;
+  int* o = out + static_cast<size_t>(b) * stride;
+  uint32_t w0 = 0u, w1 = 0u, w2 = 0u, w3 = 0u;
+  int n = 0;
+  for (int base = 0; base < stride; base += 32) {
+    const int j = base + lane;
+    const int id = j < stride ? ex[j] : INT_MAX;
+    const long long local = static_cast<long long>(id) - row_offset;
+    const bool ok = id != INT_MAX && local >= 0 && local < rows && local % r == 0;
+    const int v = ok ? static_cast<int>(local / r) : 0;
+    const unsigned bal = __ballot_sync(0xffffffffu, ok);
+    if (ok) {
+      o[n + __popc(bal & ((1u << lane) - 1u))] = v;
+      const uint32_t bit = 1u << (v & 31);
+      const int wd = (v >> 5) & 3;
+      w0 |= wd == 0 ? bit : 0u; w1 |= wd == 1 ? bit : 0u; w2 |= wd == 2 ? bit : 0u; w3 |= wd == 3 ? bit : 0u;
+    }
+    n += __popc(bal);
+  }
+  for (int j = n + lane; j < stride; j += 32) o[j] = INT_MAX;
+  w0 = __reduce_or_sync(0xffffffffu, w0); w1 = __reduce_or_sync(0xffffffffu, w1);
+  w2 = __reduce_or_sync(0xffffffffu, w2); w3 = __reduce_or_sync(0xffffffffu, w3);
+  if (lane == 0) reinterpret_cast<uint4*>(bloom)[b] = make_uint4(w0, w1, w2, w3);
+}
+
+}  // namespace wide
 
 // ============================================================================================
 // tcgen05 path: decomposition + tensor maps + launch
@@ -485,12 +757,14 @@ EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// [rows][64] bf16 row-major, box = 64 x box_rows, 128-byte swizzle, OOB rows read as zero.
-int make_tmap_bf16_k64(CUtensorMap* out, const void* ptr, unsigned long long rows, unsigned box_rows) {
+// [rows][64] bf16 row-major, box = 64 x box_rows, 128-byte swizzle, OOB rows read as zero.  row_bytes > 128: a
+// strided view (every (row_bytes / 128)-th row of the table, the lattice sample of the wide top-K).
+int make_tmap_bf16_k64(CUtensorMap* out, const void* ptr, unsigned long long rows, unsigned box_rows,
+                       unsigned long long row_bytes = 128ull) {
   EncodeTiledFn fn = get_encode_fn();
   if (!fn) return set_error(LRB_ERR_DRIVER, "cuTensorMapEncodeTiled entry point not available");
   cuuint64_t dims[2] = {64ull, rows};
-  cuuint64_t strides[1] = {128ull};
+  cuuint64_t strides[1] = {row_bytes};
   cuuint32_t box[2] = {64u, box_rows};
   cuuint32_t estr[2] = {1u, 1u};
   CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides,
@@ -501,12 +775,14 @@ int make_tmap_bf16_k64(CUtensorMap* out, const void* ptr, unsigned long long row
 }
 
 // folded-bias block: row-major [n_tiles * 256][16] bf16 (32 B per item), box = 16 x box_rows (the whole tile, or a CTA
-// pair's 128-row half), 32-byte swizzle
-int make_tmap_bias_blocks(CUtensorMap* out, const void* ptr, unsigned long long n_tiles, unsigned box_rows) {
+// pair's 128-row half), 32-byte swizzle.  row_bytes > 32: the strided view over `view_rows` items that goes with a
+// strided table view (rows past view_rows read as zero; the kernels mask those columns by their index).
+int make_tmap_bias_blocks(CUtensorMap* out, const void* ptr, unsigned long long n_tiles, unsigned box_rows,
+                          unsigned long long row_bytes = 32ull, unsigned long long view_rows = 0ull) {
   EncodeTiledFn fn = get_encode_fn();
   if (!fn) return set_error(LRB_ERR_DRIVER, "cuTensorMapEncodeTiled entry point not available");
-  cuuint64_t dims[2] = {16ull, n_tiles * tc::BN};
-  cuuint64_t strides[1] = {32ull};
+  cuuint64_t dims[2] = {16ull, row_bytes == 32ull ? n_tiles * tc::BN : view_rows};
+  cuuint64_t strides[1] = {row_bytes};
   cuuint32_t box[2] = {16u, box_rows};
   cuuint32_t estr[2] = {1u, 1u};
   CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
@@ -517,11 +793,12 @@ int make_tmap_bias_blocks(CUtensorMap* out, const void* ptr, unsigned long long 
 }
 
 // `grid` counts MMA engines: CTAs for CG == 1, CTA pairs (clusters of 2) for CG == 2.
-template <int KMAX, int NS, bool kDense, int CG, int CMAX = tc::MAX_C_SHARE_SMALL, bool kCollect = false>
+template <int KMAX, int NS, bool kDense, int CG, int CMAX = tc::MAX_C_SHARE_SMALL, bool kCollect = false,
+          bool kCollectScores = false>
 int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tbias, const tc::ScoreParams& p,
               int grid, cudaStream_t st, bool overlap_prev = false) {
   using L = tc::SmemLayout<KMAX, NS, CG>;
-  auto kern = tc::score_topk_tc_kernel<KMAX, NS, kDense, CG, CMAX, kCollect>;
+  auto kern = tc::score_topk_tc_kernel<KMAX, NS, kDense, CG, CMAX, kCollect, kCollectScores>;
   LRB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kAlloc));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid * CG));
@@ -558,6 +835,10 @@ static size_t ring_bytes();
 // users per block of the exact-fp32 "dense + select" path (0 = the catalogue is too large for it): what fits in
 // the candidate-ring part of the scratch buffer, which lrb_score_scratch_bytes() reserves for every B
 static long long f32_select_users(long long rows) { return lrb::f32::select_block_users(rows, 2 * ring_bytes()); }
+// the largest shard the dense + select path takes (one 128-user block of score rows in the scratch)
+static long long f32_select_rows_max() {
+  return static_cast<long long>(2 * ring_bytes() / (lrb::f32::ROWS * sizeof(float))) / 4 * 4;
+}
 
 int lrb_score_topk_slots(int B, int64_t rows, int precision, int* slots) {
   LRB_REQUIRE(B > 0 && rows > 0 && slots != nullptr, "lrb_score_topk_slots: bad arguments");
@@ -614,77 +895,26 @@ size_t lrb_score_scratch_bytes(int B) {
   return n_chunks * gslots_chunk_bytes(cap) + 2 * ring_bytes();
 }
 
-int lrb_score_topk(const void* u, const void* table, const float* bias_pad, const void* bias_blk,
-                   int B, int64_t rows,
-                   int64_t row_offset, const int32_t* excl_sorted, const uint32_t* excl_bloom,
-                   int excl_stride, int K, int precision, float* part_scores, int32_t* part_ids,
-                   int32_t* part_cnt, int slots, void* scratch, void* stream) {
+// The bf16 streaming top-K of lrb_score_topk over `rows` item rows; r > 1: over the strided view of every r-th row of
+// table / bias_blk (local row i = table row r * i), the lattice sample of lrb_wide_sample_threshold.
+static int topk_bf16(const void* u, const void* table, const void* bias_blk, int B, int64_t rows, int64_t row_offset,
+                     const int32_t* excl_sorted, const uint32_t* excl_bloom, int excl_stride, int K,
+                     float* part_scores, int32_t* part_ids, int32_t* part_cnt, int slots, void* scratch,
+                     cudaStream_t st, int sms, int r) {
   using namespace lrb;
-  int rc = check_arch();
-  if (rc != LRB_OK) return rc;
-  LRB_REQUIRE(u && table && part_scores && part_ids && part_cnt, "lrb_score_topk: null pointer");
-  LRB_REQUIRE(precision != 1 || bias_pad != nullptr, "lrb_score_topk: the fp32 path needs bias_pad");
-  LRB_REQUIRE(B > 0 && rows > 0 && rows + row_offset < INT_MAX, "lrb_score_topk: bad B/rows");
-  LRB_REQUIRE(K >= 1 && K <= LRB_MAX_K, "lrb_score_topk: K must be in [1, %d]", LRB_MAX_K);
-  LRB_REQUIRE((excl_sorted == nullptr) == (excl_bloom == nullptr), "lrb_score_topk: exclusion list and bloom filter must come together");
-  cudaStream_t st = as_stream(stream);
-  int sms = device_sm_count();
-  if (precision == 1 && f32_select_users(rows) > 0) {
-    LRB_REQUIRE(slots == 1, "lrb_score_topk: slots=%d but lrb_score_topk_slots says 1", slots);
-    LRB_REQUIRE(scratch != nullptr, "lrb_score_topk: scratch is required");
-    const long long blk = f32_select_users(rows);
-    const long long ld = (rows + 3) / 4 * 4;
-    float* dense = static_cast<float*>(scratch);
-    for (long long b0 = 0; b0 < B; b0 += blk) {
-      const int nb = static_cast<int>(B - b0 < blk ? B - b0 : blk);
-      rc = f32::launch_dense(static_cast<const float*>(u) + b0 * f32::D, static_cast<const float*>(table), bias_pad,
-                             nb, static_cast<int>(rows), dense, ld, sms, st);
-      if (rc != LRB_OK) return rc;
-      f32::SelParams sp;
-      sp.dense = dense; sp.ld = ld; sp.nb = nb; sp.b0 = static_cast<int>(b0);
-      sp.rows = static_cast<int>(rows); sp.row_offset = static_cast<int>(row_offset); sp.K = K;
-      sp.excl_sorted = excl_sorted; sp.excl_stride = excl_stride;
-      sp.part_scores = part_scores; sp.part_ids = part_ids; sp.part_cnt = part_cnt;
-      f32::select_topk_kernel<<<(nb + f32::SEL_WARPS - 1) / f32::SEL_WARPS, f32::SEL_WARPS * 32, 0, st>>>(sp);
-      LRB_CUDA_TRY(cudaGetLastError());
-    }
-    return LRB_OK;
-  }
-  if (precision == 1) {
-    const int splits = f32::splits_for(B, rows, sms);
-    LRB_REQUIRE(slots == splits, "lrb_score_topk: slots=%d but lrb_score_topk_slots says %d", slots, splits);
-    f32::Params p;
-    p.u = static_cast<const float*>(u);
-    p.table = static_cast<const float*>(table);
-    p.bias_pad = bias_pad;
-    p.B = B; p.rows = static_cast<int>(rows); p.row_offset = static_cast<int>(row_offset); p.K = K;
-    p.excl_sorted = excl_sorted; p.excl_bloom = excl_bloom; p.excl_stride = excl_stride;
-    p.part_scores = part_scores; p.part_ids = part_ids; p.part_cnt = part_cnt; p.slots = slots;
-    p.dense_out = nullptr; p.dense_ld = 0;
-    const size_t smem = (f32::IT * f32::D + f32::IT) * 4 + static_cast<size_t>(K) * f32::ROWS * 8;
-    auto kern = f32::score_f32_kernel<false>;
-    LRB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    dim3 grid((B + f32::ROWS - 1) / f32::ROWS, splits);
-    kern<<<grid, f32::ROWS, smem, st>>>(p);
-    LRB_CUDA_TRY(cudaGetLastError());
-    return LRB_OK;
-  }
-  LRB_REQUIRE(precision == 0, "precision must be 0 (bf16) or 1 (fp32)");
-  LRB_REQUIRE(scratch != nullptr, "lrb_score_topk: scratch is required for the bf16 path");
-  const int want_slots = chunked_slots(B, rows, sms);
-  LRB_REQUIRE(slots == want_slots, "lrb_score_topk: slots=%d but lrb_score_topk_slots says %d", slots, want_slots);
   CUtensorMap tb1, tb2, tbias, tbias1;
-  rc = make_tmap_bf16_k64(&tb1, table, static_cast<unsigned long long>(rows), tc::BN);
+  const unsigned long long tstride = 128ull * r, bstride = 32ull * r;
+  int rc = make_tmap_bf16_k64(&tb1, table, static_cast<unsigned long long>(rows), tc::BN, tstride);
   if (rc != LRB_OK) return rc;
-  rc = make_tmap_bf16_k64(&tb2, table, static_cast<unsigned long long>(rows), tc::BN / 2);
+  rc = make_tmap_bf16_k64(&tb2, table, static_cast<unsigned long long>(rows), tc::BN / 2, tstride);
   if (rc != LRB_OK) return rc;
   tbias = tb1;   // placeholders when there is no bias block (never dereferenced)
   tbias1 = tb1;
   if (bias_blk != nullptr) {
     const unsigned long long nt = static_cast<unsigned long long>((rows + tc::BN - 1) / tc::BN);
-    rc = make_tmap_bias_blocks(&tbias, bias_blk, nt, tc::BN / 2);     // a CTA pair's halves
+    rc = make_tmap_bias_blocks(&tbias, bias_blk, nt, tc::BN / 2, bstride, rows);     // a CTA pair's halves
     if (rc != LRB_OK) return rc;
-    rc = make_tmap_bias_blocks(&tbias1, bias_blk, nt, tc::BN);        // single CTAs: the whole tile
+    rc = make_tmap_bias_blocks(&tbias1, bias_blk, nt, tc::BN, bstride, rows);        // single CTAs: the whole tile
     if (rc != LRB_OK) return rc;
   }
   LRB_CUDA_TRY(cudaMemsetAsync(part_cnt, 0, static_cast<size_t>(B) * slots * sizeof(int), st));
@@ -753,6 +983,81 @@ int lrb_score_topk(const void* u, const void* table, const float* bias_pad, cons
   return LRB_OK;
 }
 
+int lrb_score_topk(const void* u, const void* table, const float* bias_pad, const void* bias_blk,
+                   int B, int64_t rows,
+                   int64_t row_offset, const int32_t* excl_sorted, const uint32_t* excl_bloom,
+                   int excl_stride, int K, int precision, float* part_scores, int32_t* part_ids,
+                   int32_t* part_cnt, int slots, void* scratch, void* stream) {
+  using namespace lrb;
+  int rc = check_arch();
+  if (rc != LRB_OK) return rc;
+  LRB_REQUIRE(u && table && part_scores && part_ids && part_cnt, "lrb_score_topk: null pointer");
+  LRB_REQUIRE(precision != 1 || bias_pad != nullptr, "lrb_score_topk: the fp32 path needs bias_pad");
+  LRB_REQUIRE(B > 0 && rows > 0 && rows + row_offset < INT_MAX, "lrb_score_topk: bad B/rows");
+  LRB_REQUIRE(K >= 1 && K <= LRB_MAX_K_WIDE, "lrb_score_topk: K must be in [1, %d]", LRB_MAX_K_WIDE);
+  LRB_REQUIRE(K <= LRB_MAX_K || K <= rows, "lrb_score_topk: K=%d > %d needs K <= rows (%lld)", K, LRB_MAX_K,
+              static_cast<long long>(rows));
+  LRB_REQUIRE((excl_sorted == nullptr) == (excl_bloom == nullptr), "lrb_score_topk: exclusion list and bloom filter must come together");
+  if (K > LRB_MAX_K && !(precision == 1 && f32_select_users(rows) > 0))
+    return set_error(LRB_ERR_UNSUPPORTED, "lrb_score_topk: K=%d > %d only on the fp32 dense + select path "
+                     "(rows <= %lld); use lrb_wide_* for bf16", K, LRB_MAX_K, f32_select_rows_max());
+  cudaStream_t st = as_stream(stream);
+  int sms = device_sm_count();
+  if (precision == 1 && f32_select_users(rows) > 0) {
+    LRB_REQUIRE(slots == 1, "lrb_score_topk: slots=%d but lrb_score_topk_slots says 1", slots);
+    LRB_REQUIRE(scratch != nullptr, "lrb_score_topk: scratch is required");
+    const long long blk = f32_select_users(rows);
+    const long long ld = (rows + 3) / 4 * 4;
+    float* dense = static_cast<float*>(scratch);
+    for (long long b0 = 0; b0 < B; b0 += blk) {
+      const int nb = static_cast<int>(B - b0 < blk ? B - b0 : blk);
+      rc = f32::launch_dense(static_cast<const float*>(u) + b0 * f32::D, static_cast<const float*>(table), bias_pad,
+                             nb, static_cast<int>(rows), dense, ld, sms, st);
+      if (rc != LRB_OK) return rc;
+      f32::SelParams sp;
+      sp.dense = dense; sp.ld = ld; sp.nb = nb; sp.b0 = static_cast<int>(b0);
+      sp.rows = static_cast<int>(rows); sp.row_offset = static_cast<int>(row_offset); sp.K = K;
+      sp.excl_sorted = excl_sorted; sp.excl_stride = excl_stride;
+      sp.part_scores = part_scores; sp.part_ids = part_ids; sp.part_cnt = part_cnt;
+      if (K <= LRB_MAX_K) {
+        f32::select_topk_kernel<64, false, f32::SelParams><<<(nb + f32::SEL_WARPS - 1) / f32::SEL_WARPS, f32::SEL_WARPS * 32, 0, st>>>(sp);
+      } else {
+        f32::SelParamsWide wp = {};
+        static_cast<f32::SelParams&>(wp) = sp;
+        f32::select_topk_kernel<f32::SEL_CAP_WIDE, false>
+            <<<(nb + f32::SEL_WARPS_WIDE - 1) / f32::SEL_WARPS_WIDE, f32::SEL_WARPS_WIDE * 32, 0, st>>>(wp);
+      }
+      LRB_CUDA_TRY(cudaGetLastError());
+    }
+    return LRB_OK;
+  }
+  if (precision == 1) {
+    const int splits = f32::splits_for(B, rows, sms);
+    LRB_REQUIRE(slots == splits, "lrb_score_topk: slots=%d but lrb_score_topk_slots says %d", slots, splits);
+    f32::Params p;
+    p.u = static_cast<const float*>(u);
+    p.table = static_cast<const float*>(table);
+    p.bias_pad = bias_pad;
+    p.B = B; p.rows = static_cast<int>(rows); p.row_offset = static_cast<int>(row_offset); p.K = K;
+    p.excl_sorted = excl_sorted; p.excl_bloom = excl_bloom; p.excl_stride = excl_stride;
+    p.part_scores = part_scores; p.part_ids = part_ids; p.part_cnt = part_cnt; p.slots = slots;
+    p.dense_out = nullptr; p.dense_ld = 0;
+    const size_t smem = (f32::IT * f32::D + f32::IT) * 4 + static_cast<size_t>(K) * f32::ROWS * 8;
+    auto kern = f32::score_f32_kernel<false>;
+    LRB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    dim3 grid((B + f32::ROWS - 1) / f32::ROWS, splits);
+    kern<<<grid, f32::ROWS, smem, st>>>(p);
+    LRB_CUDA_TRY(cudaGetLastError());
+    return LRB_OK;
+  }
+  LRB_REQUIRE(precision == 0, "precision must be 0 (bf16) or 1 (fp32)");
+  LRB_REQUIRE(scratch != nullptr, "lrb_score_topk: scratch is required for the bf16 path");
+  const int want_slots = chunked_slots(B, rows, sms);
+  LRB_REQUIRE(slots == want_slots, "lrb_score_topk: slots=%d but lrb_score_topk_slots says %d", slots, want_slots);
+  return topk_bf16(u, table, bias_blk, B, rows, row_offset, excl_sorted, excl_bloom, excl_stride, K, part_scores,
+                   part_ids, part_cnt, slots, scratch, st, sms, 1);
+}
+
 int lrb_score_dense(const void* x, const void* table, const float* bias_pad, const void* bias_blk,
                     int64_t M, int64_t rows, int precision, float* out, int64_t ld_out, void* stream) {
   using namespace lrb;
@@ -788,9 +1093,9 @@ int lrb_score_dense(const void* x, const void* table, const float* bias_pad, con
   return launch_tc<20, 3, true, 1>(ta, tb, tbias, p, d.grid, st);
 }
 
-int lrb_score_collect(const void* u_bf16, const void* table_bf16, const void* bias_blk, int M, int64_t rows,
-                      int64_t row_offset, const float* tau, int cap, int32_t* cand_ids, int32_t* cand_cnt,
-                      void* stream) {
+static int collect_impl(const void* u_bf16, const void* table_bf16, const void* bias_blk, int M, int64_t rows,
+                        int64_t row_offset, const float* tau, int cap, int32_t* cand_ids, float* cand_scores,
+                        int32_t* cand_cnt, void* stream) {
   using namespace lrb;
   int rc = check_arch();
   if (rc != LRB_OK) return rc;
@@ -817,8 +1122,174 @@ int lrb_score_collect(const void* u_bf16, const void* table_bf16, const void* bi
   p.row_offset = static_cast<int>(row_offset); p.K = 1; p.bias_blk = static_cast<const uint8_t*>(bias_blk);
   p.s_full = d.s_full; p.rem = d.rem; p.full_tiles = d.full_tiles; p.y_tiles = d.y_tiles;
   p.collect_tau = tau; p.collect_ids = cand_ids; p.collect_cnt = cand_cnt; p.collect_cap = cap;
+  p.collect_scores = cand_scores;
   LRB_CUDA_TRY(cudaMemsetAsync(cand_cnt, 0, static_cast<size_t>(M) * sizeof(int32_t), st));
+  if (cand_scores != nullptr)
+    return launch_tc<20, 3, true, 1, tc::MAX_C_SHARE_SMALL, true, true>(ta, tb, tbias, p, d.grid, st);
   return launch_tc<20, 3, true, 1, tc::MAX_C_SHARE_SMALL, true>(ta, tb, tbias, p, d.grid, st);
+}
+
+int lrb_score_collect(const void* u_bf16, const void* table_bf16, const void* bias_blk, int M, int64_t rows,
+                      int64_t row_offset, const float* tau, int cap, int32_t* cand_ids, int32_t* cand_cnt,
+                      void* stream) {
+  return collect_impl(u_bf16, table_bf16, bias_blk, M, rows, row_offset, tau, cap, cand_ids, nullptr, cand_cnt,
+                      stream);
+}
+
+int lrb_score_collect_scores(const void* u_bf16, const void* table_bf16, const void* bias_blk, int M, int64_t rows,
+                             int64_t row_offset, const float* tau, int cap, int32_t* cand_ids, float* cand_scores,
+                             int32_t* cand_cnt, void* stream) {
+  LRB_REQUIRE(cap == 0 || cand_scores != nullptr, "lrb_score_collect_scores: null cand_scores");
+  return collect_impl(u_bf16, table_bf16, bias_blk, M, rows, row_offset, tau, cap, cand_ids, cand_scores, cand_cnt,
+                      stream);
+}
+
+// ---- wide top-K (K in [51, LRB_MAX_K_WIDE]) on the bf16 path ----------------------------------------------------
+
+static size_t align256(size_t x) { return (x + 255) & ~static_cast<size_t>(255); }
+
+struct SampleLayout {
+  long long n_lat;
+  int slots;
+  size_t excl, bloom, part_s, part_i, part_c, top_s, top_i, scratch, total;
+};
+
+static SampleLayout sample_layout(int B, int64_t rows, int excl_stride, int r, int m) {
+  SampleLayout L = {};
+  int sms = lrb::device_sm_count();
+  if (sms <= 0) sms = 148;
+  L.n_lat = (rows + r - 1) / r;
+  L.slots = lrb::chunked_slots(B, L.n_lat, sms);
+  const size_t Bs = static_cast<size_t>(B);
+  size_t o = 0;
+  L.excl = o;    o += align256(Bs * (excl_stride > 0 ? excl_stride : 0) * 4);
+  L.bloom = o;   o += align256(Bs * 16);
+  L.part_s = o;  o += align256(Bs * L.slots * m * 4);
+  L.part_i = o;  o += align256(Bs * L.slots * m * 4);
+  L.part_c = o;  o += align256(Bs * L.slots * 4);
+  L.top_s = o;   o += align256(Bs * m * 4);
+  L.top_i = o;   o += align256(Bs * m * 4);
+  L.scratch = o; o += align256(lrb_score_scratch_bytes(B));
+  L.total = o;
+  return L;
+}
+
+size_t lrb_wide_sample_workspace_bytes(int B, int64_t rows, int excl_stride, int r, int m) {
+  if (B < 1 || rows < 1 || r < 1 || m < 1 || m > LRB_MAX_K) return 256;
+  return sample_layout(B, rows, excl_stride, r, m).total;
+}
+
+int lrb_wide_sample_threshold(const void* u_bf16, const void* table_bf16, const void* bias_blk, int B, int64_t rows,
+                              int64_t row_offset, const int32_t* excl_sorted, int excl_stride, int r, int m,
+                              float* tau, void* workspace, size_t workspace_bytes, void* stream) {
+  using namespace lrb;
+  int rc = check_arch();
+  if (rc != LRB_OK) return rc;
+  LRB_REQUIRE(u_bf16 && table_bf16 && tau && workspace, "lrb_wide_sample_threshold: null pointer");
+  LRB_REQUIRE(B > 0 && rows > 0 && row_offset >= 0 && rows + row_offset < INT_MAX,
+              "lrb_wide_sample_threshold: bad shape");
+  LRB_REQUIRE(r >= 1 && r <= (1 << 20) && m >= 1 && m <= LRB_MAX_K,
+              "lrb_wide_sample_threshold: need r in [1, 2^20] and m in [1, %d]", LRB_MAX_K);
+  LRB_REQUIRE(excl_sorted == nullptr || excl_stride > 0, "lrb_wide_sample_threshold: bad excl_stride");
+  const SampleLayout L = sample_layout(B, rows, excl_sorted ? excl_stride : 0, r, m);
+  if (workspace_bytes < L.total)
+    return set_error(LRB_ERR_WORKSPACE, "lrb_wide_sample_threshold: workspace %zu < %zu bytes", workspace_bytes,
+                     L.total);
+  cudaStream_t st = as_stream(stream);
+  if (L.n_lat < m) {                            // fewer than m lattice rows: no threshold
+    wide::fill_kernel<<<(B + 255) / 256, 256, 0, st>>>(tau, B, -INFINITY);
+    LRB_CUDA_TRY(cudaGetLastError());
+    return LRB_OK;
+  }
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  int32_t* excl = nullptr;
+  uint32_t* bloom = nullptr;
+  if (excl_sorted != nullptr) {
+    excl = reinterpret_cast<int32_t*>(ws + L.excl);
+    bloom = reinterpret_cast<uint32_t*>(ws + L.bloom);
+    wide::lattice_excl_kernel<<<(B + 7) / 8, 256, 0, st>>>(excl_sorted, excl_stride, B, static_cast<int>(row_offset),
+                                                           static_cast<int>(rows), r, excl, bloom);
+    LRB_CUDA_TRY(cudaGetLastError());
+  }
+  float* part_s = reinterpret_cast<float*>(ws + L.part_s);
+  int32_t* part_i = reinterpret_cast<int32_t*>(ws + L.part_i);
+  int32_t* part_c = reinterpret_cast<int32_t*>(ws + L.part_c);
+  rc = topk_bf16(u_bf16, table_bf16, bias_blk, B, L.n_lat, 0, excl, bloom, excl_stride, m, part_s, part_i, part_c,
+                 L.slots, ws + L.scratch, st, device_sm_count(), r);
+  if (rc != LRB_OK) return rc;
+  float* top_s = reinterpret_cast<float*>(ws + L.top_s);
+  rc = lrb_merge_metrics(part_s, part_i, part_c, L.slots, m, static_cast<int64_t>(L.slots) * m, 1, L.slots, m, B, m,
+                         nullptr, nullptr, 0, top_s, reinterpret_cast<int32_t*>(ws + L.top_i), 0, nullptr, nullptr,
+                         stream);
+  if (rc != LRB_OK) return rc;
+  // tau = the m-th entry of the merged lattice list (-inf when the lattice holds fewer than m admissible rows)
+  LRB_CUDA_TRY(cudaMemcpy2DAsync(tau, sizeof(float), top_s + (m - 1), static_cast<size_t>(m) * sizeof(float),
+                                 sizeof(float), static_cast<size_t>(B), cudaMemcpyDeviceToDevice, st));
+  return LRB_OK;
+}
+
+// dense bf16 rows of the wide select's fallback: users per block so that a block of rows stays near 1 GiB
+static long long wide_dense_block(int64_t rows) {
+  const long long ld = (rows + 3) / 4 * 4;
+  const long long blk = (1ll << 30) / (ld * 4);
+  return blk < 1 ? 1 : blk;
+}
+
+size_t lrb_wide_select_workspace_bytes(int n, int64_t rows) {
+  if (n < 1 || rows < 1) return 256;
+  const long long ld = (rows + 3) / 4 * 4;
+  const long long blk = wide_dense_block(rows);
+  return align256(static_cast<size_t>(n < blk ? n : blk) * ld * sizeof(float));
+}
+
+int lrb_wide_select(const int32_t* users, int n, const void* u_bf16, const void* table_bf16, const void* bias_blk,
+                    int64_t rows, int64_t row_offset, const int32_t* excl_sorted, int excl_stride, float* cand_scores,
+                    int32_t* cand_ids, const int32_t* cand_cnt, int cap, int K, int ok_path, float* out_scores,
+                    int32_t* out_ids, int32_t* out_cnt, int8_t* path, float* tau_out, void* workspace,
+                    size_t workspace_bytes, void* stream) {
+  using namespace lrb;
+  int rc = check_arch();
+  if (rc != LRB_OK) return rc;
+  LRB_REQUIRE(users && out_scores && out_ids && out_cnt && path, "lrb_wide_select: null pointer");
+  LRB_REQUIRE(n > 0 && rows > 0 && row_offset >= 0 && rows + row_offset < INT_MAX, "lrb_wide_select: bad shape");
+  LRB_REQUIRE(K >= 1 && K <= LRB_MAX_K_WIDE, "lrb_wide_select: K must be in [1, %d]", LRB_MAX_K_WIDE);
+  LRB_REQUIRE(K <= rows, "lrb_wide_select: K=%d > rows (%lld)", K, static_cast<long long>(rows));
+  LRB_REQUIRE(ok_path >= 0 && ok_path <= 127, "lrb_wide_select: ok_path must be in [0, 127]");
+  LRB_REQUIRE(excl_sorted == nullptr || excl_stride > 0, "lrb_wide_select: bad excl_stride");
+  cudaStream_t st = as_stream(stream);
+  f32::SelParamsWide sp = {};
+  sp.rows = static_cast<int>(rows); sp.row_offset = static_cast<int>(row_offset); sp.K = K;
+  sp.excl_sorted = excl_sorted; sp.excl_stride = excl_stride;
+  sp.part_scores = out_scores; sp.part_ids = out_ids; sp.part_cnt = out_cnt;
+  sp.path = path; sp.ok_path = ok_path; sp.tau_out = tau_out;
+  constexpr int W = f32::SEL_WARPS_WIDE;
+  if (cand_scores != nullptr) {                 // explicit candidate lists
+    LRB_REQUIRE(cand_ids && cand_cnt && tau_out && cap >= 1, "lrb_wide_select: candidate lists need ids, counts, "
+                "tau_out and cap >= 1");
+    sp.nb = n; sp.users = users;
+    sp.cand_scores = cand_scores; sp.cand_ids = cand_ids; sp.cand_cnt = cand_cnt; sp.cap = cap;
+    f32::select_topk_kernel<f32::SEL_CAP_WIDE, true><<<(n + W - 1) / W, W * 32, 0, st>>>(sp);
+    LRB_CUDA_TRY(cudaGetLastError());
+    return LRB_OK;
+  }
+  // dense bf16 rows (lrb_score_dense precision 0) of u_bf16 row i = user users[i], in blocks of the workspace
+  LRB_REQUIRE(u_bf16 && table_bf16 && workspace, "lrb_wide_select: the dense loader needs u_bf16, table and workspace");
+  const size_t need = lrb_wide_select_workspace_bytes(n, rows);
+  if (workspace_bytes < need)
+    return set_error(LRB_ERR_WORKSPACE, "lrb_wide_select: workspace %zu < %zu bytes", workspace_bytes, need);
+  const long long ld = (rows + 3) / 4 * 4;
+  const long long blk = wide_dense_block(rows);
+  float* dense = static_cast<float*>(workspace);
+  for (long long i0 = 0; i0 < n; i0 += blk) {
+    const int nb = static_cast<int>(n - i0 < blk ? n - i0 : blk);
+    rc = lrb_score_dense(static_cast<const uint8_t*>(u_bf16) + i0 * 128, table_bf16, nullptr, bias_blk, nb, rows, 0,
+                         dense, ld, stream);
+    if (rc != LRB_OK) return rc;
+    sp.dense = dense; sp.ld = ld; sp.nb = nb; sp.users = users + i0;
+    f32::select_topk_kernel<f32::SEL_CAP_WIDE, false><<<(nb + W - 1) / W, W * 32, 0, st>>>(sp);
+    LRB_CUDA_TRY(cudaGetLastError());
+  }
+  return LRB_OK;
 }
 
 }  // extern "C"

@@ -101,6 +101,8 @@ struct ScoreParams {
   int* collect_ids;
   int* collect_cnt;
   int collect_cap;
+  // collect mode with scores only (kCollectScores): the collected item's score goes to collect_scores[b][slot]
+  float* collect_scores;
 };
 
 struct Segment {
@@ -444,8 +446,10 @@ LRB_DEVINL uint64_t umma_desc_k16_sw32(uint32_t smem_addr) {
 // ~1500 cycles of hand-offs (remote mbarrier arrivals of the pair's other CTA, the MMA warp's wake-up and issue, the
 // commit's arrival) on top of the MMA itself; throughput = TMEM columns in flight / that cycle, hence four small
 // stages instead of two large ones, and every hand-off kept as short as it goes.
-// kCollect (with kDense): threshold collect instead of the dense write-out (lrb_score_collect).
-template <int KMAX, int NS, bool kDense, int CG, int CMAX = MAX_C_SHARE_SMALL, bool kCollect = false>
+// kCollect (with kDense): threshold collect instead of the dense write-out (lrb_score_collect); kCollectScores
+// (with kCollect) also stores every collected item's score (lrb_score_collect_scores).
+template <int KMAX, int NS, bool kDense, int CG, int CMAX = MAX_C_SHARE_SMALL, bool kCollect = false,
+          bool kCollectScores = false>
 __global__ void __launch_bounds__(128 + EPI_WARPS * 32, 1)
 score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
                      const __grid_constant__ CUtensorMap tmap_b,
@@ -903,8 +907,10 @@ score_topk_tc_kernel(const __grid_constant__ CUtensorMap tmap_a,
                       const int c = col0 + g * 16 + j;
                       if (c < p.rows && q[j] >= tau) {
                         const int slot = atomicAdd(p.collect_cnt + row, 1);
-                        if (slot < p.collect_cap)
+                        if (slot < p.collect_cap) {
                           p.collect_ids[static_cast<size_t>(row) * p.collect_cap + slot] = p.row_offset + c;
+                          if (kCollectScores) p.collect_scores[static_cast<size_t>(row) * p.collect_cap + slot] = q[j];
+                        }
                       }
                     }
                   }

@@ -26,6 +26,26 @@ from .packing import pack_encoder_weights, unpack_encoder_grads
 
 SMALL_CATALOGUE_ROWS = 1 << 17   # up to here 'auto' precision scores in exact fp32
 EXACT_CAP = 4096                 # precision="exact": collected ids per user before it goes to the fp32 path
+MAX_K = 50                       # longest list of the streaming top-K kernels (LRB_MAX_K)
+MAX_K_WIDE = 1024                # longest list of the wide path and of the fp32 dense + select path (LRB_MAX_K_WIDE)
+WIDE_SAMPLE_M = 20               # k > 50 on bf16: the threshold is the m-th best score of a lattice sample
+
+
+class UnsupportedK(_lib.LrbError, ValueError):
+    """k > 50 with precision="exact" on a shard of more than 131 072 rows: a ValueError, and an LrbError as this
+    refusal has always been."""
+
+
+def wide_policy(k: int, excl_stride: int, topk_cap: Optional[int] = None):
+    """(m, r, cap) of the wide bf16 top-K (DESIGN section 2.2): the threshold is the m-th best score over the rows
+    j = 0 (mod r), so that about m * r = 4k items are expected to reach it; `cap` collected items per user (history
+    items included) before a user overflows."""
+    m = WIDE_SAMPLE_M
+    r = max(1, -(-4 * k // m))
+    cap = int(topk_cap) if topk_cap is not None else 8 * k + excl_stride
+    if cap < 1:
+        raise ValueError(f"topk_cap must be >= 1, got {topk_cap}")
+    return m, r, cap
 
 
 def _on_model_device(fn):
@@ -137,6 +157,8 @@ class LRURec(nn.Module):
         self._ws: Dict[tuple, torch.Tensor] = {}
         # optional list; when set, retrieve() appends (start, end) CUDA events around the scoring launch
         self.profile_events = None
+        # optional list; when set, a k > 50 bf16 retrieve() appends (phase, start, end) CUDA events per phase
+        self.wide_profile_events = None
         # row shard of the item table owned by this instance: [row_begin, row_end)
         self.row_begin, self.row_end = 0, vocab
 
@@ -187,7 +209,7 @@ class LRURec(nn.Module):
                  u_bf16: Optional[torch.Tensor] = None, merge: bool = True,
                  packed_out: Optional[torch.Tensor] = None, seq: Optional[dict] = None,
                  scatter: Optional[dict] = None, packed_layout: str = "planes",
-                 exact_cap: int = EXACT_CAP) -> Dict[str, torch.Tensor]:
+                 exact_cap: int = EXACT_CAP, topk_cap: Optional[int] = None) -> Dict[str, torch.Tensor]:
         """encode -> catalogue score -> (history mask) -> top-k -> (metrics), all on device.  Eval semantics in either
         mode: no dropout.
 
@@ -213,12 +235,38 @@ class LRURec(nn.Module):
         of ids collected for each user (also past `exact_cap`; 0 where nothing was collected).  An exact call
         synchronises with the host at most twice, to size the collected and the fp32 sub-batches.  It needs the
         fp32 states (`u`, or `x`).
+
+        k up to 50 runs the streaming top-K kernels.  k in [51, 1024] (DESIGN section 2.2) needs k <= the shard's
+        rows.  With a bf16 precision it runs the wide path: a threshold from a lattice sample of the catalogue, every
+        item whose bf16 score reaches it collected (at most `topk_cap` per user, default 8k + the history width),
+        then a per-user select; users that overflow the cap are collected again at a higher threshold, and users
+        still without an exact list get dense bf16 rows.  The lists equal those of the single-CTA tensor-core scores
+        fully sorted.  `topk_path` [B] int8 says which pass produced each list (0 = first collect, 1 = second
+        collect, 2 = dense rows) and `topk_collected` [B] int32 the items the last collect found (also past the cap).
+        Such a call synchronises with the host at most twice.  "fp32" takes k > 50 where the fp32 dense + select
+        path runs (shards of up to ~568 k rows on 148 SMs), "exact" on shards of up to 131 072 rows (where it is that
+        path); beyond those sizes they raise ValueError before any work (for "exact" an `UnsupportedK`, which is
+        also an LrbError).
         """
         lib = _lib.load()
         c = self._prepare()
         dev = c["table_f32"].device
         rows = self.row_end - self.row_begin
         prec = self._precision(precision, rows)
+        k = int(k)
+        if k > MAX_K and prec != 0:
+            # fp32 / exact: only the fp32 dense + select path takes lists longer than the streaming kernels'
+            slots = _lib.c_int(0)
+            _lib.check(lib.lrb_score_topk_slots(1, rows, 1, _lib.ctypes.byref(slots)))
+            if slots.value != 1:
+                raise ValueError(f'precision={precision!r} with k={k} > {MAX_K} needs the fp32 dense + select path, '
+                                 f'which takes shards of up to ~568 k rows (this shard has {rows}); use '
+                                 f'precision="bf16" for longer lists on large catalogues')
+            if prec == 2:
+                # above 131 072 rows "exact" is the bf16-candidate path, whose lists stop at 50
+                raise UnsupportedK(-1, f'precision="exact" with k={k} > {MAX_K} runs only on shards of up to '
+                                       f'{SMALL_CATALOGUE_ROWS} rows (this shard has {rows}); use precision="fp32" '
+                                       f'(up to ~568 k rows) or "bf16"')
         if x is None:
             if seq is None or (u is None and u_bf16 is None):
                 raise ValueError("retrieve(x=None) needs the user states (u / u_bf16) and a prepared `seq`")
@@ -236,6 +284,9 @@ class LRURec(nn.Module):
             u, u_bf16, _ = self._encode(x, all_positions=False, want_bf16=(prec == 0), seq=seq)
         elif prec == 0 and u_bf16 is None:
             u_bf16 = u.to(torch.bfloat16).contiguous()
+        if prec == 0 and k > MAX_K:
+            return self._retrieve_wide(u_bf16, seq if exclude_history else None, k, labels, ks, merge, packed_out,
+                                       scatter, packed_layout, topk_cap, u)
         if prec == 2:
             return self._retrieve_exact(u, seq if exclude_history else None, k, labels, ks, merge, packed_out,
                                         scatter, packed_layout, exact_cap)
@@ -360,6 +411,100 @@ class LRURec(nn.Module):
         out["u"] = u
         out["exact_path"] = path
         out["exact_collected"] = collected
+        return out
+
+    def _retrieve_wide(self, u_bf16, seq, k, labels, ks, merge, packed_out, scatter, packed_layout, topk_cap, u):
+        """k in [51, 1024] on the bf16 path (see retrieve; DESIGN section 2.2)."""
+        lib = _lib.load()
+        c = self._prepare()
+        dev = u_bf16.device
+        rows = self.row_end - self.row_begin
+        B = u_bf16.shape[0]
+        u_bf16 = u_bf16.contiguous()
+        if k > MAX_K_WIDE or k > rows:
+            raise _lib.LrbError(-1, f"k={k} must be <= {MAX_K_WIDE} and <= the shard's rows ({rows})")
+        excl = seq["excl_sorted"] if seq is not None else None
+        stride = seq["excl_stride"] if seq is not None else 0
+        m, r, cap = wide_policy(k, stride, topk_cap)
+        st = _lib.stream_handle()
+        tbl, bias = _lib.ptr(c["table_bf16"]), _lib.ptr(c["bias_blk"])
+        prof = self.wide_profile_events
+
+        def mark(name):
+            if prof is not None:
+                ev = torch.cuda.Event(enable_timing=True)
+                ev.record()
+                if prof and prof[-1][2] is None:
+                    prof[-1] = (prof[-1][0], prof[-1][1], ev)
+                prof.append((name, ev, None))
+
+        mark("sample")
+        # 1. threshold from the lattice sample
+        tau = torch.empty(B, dtype=torch.float32, device=dev)
+        ws_bytes = lib.lrb_wide_sample_workspace_bytes(B, rows, stride, r, m)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        _lib.check(lib.lrb_wide_sample_threshold(_lib.ptr(u_bf16), tbl, bias, B, rows, self.row_begin, _lib.ptr(excl),
+                                                 stride, r, m, _lib.ptr(tau), _lib.ptr(ws), ws_bytes, st))
+        del ws
+        out_s = torch.empty(B, 1, k, dtype=torch.float32, device=dev)
+        out_i = torch.empty(B, 1, k, dtype=torch.int32, device=dev)
+        out_c = torch.zeros(B, 1, dtype=torch.int32, device=dev)
+        path = torch.empty(B, dtype=torch.int8, device=dev)
+        tau2 = torch.empty(B, dtype=torch.float32, device=dev)
+        collected = torch.zeros(B, dtype=torch.int32, device=dev)
+
+        def collect_select(users, ub, tb, ok_path):
+            n = ub.shape[0]
+            ids = torch.empty(n, cap, dtype=torch.int32, device=dev)
+            scs = torch.empty(n, cap, dtype=torch.float32, device=dev)
+            cnt = torch.empty(n, dtype=torch.int32, device=dev)
+            _lib.check(lib.lrb_score_collect_scores(_lib.ptr(ub), tbl, bias, n, rows, self.row_begin, _lib.ptr(tb),
+                                                    cap, _lib.ptr(ids), _lib.ptr(scs), _lib.ptr(cnt), st))
+            _lib.check(lib.lrb_wide_select(_lib.ptr(users), n, None, None, None, rows, self.row_begin, _lib.ptr(excl),
+                                           stride, _lib.ptr(scs), _lib.ptr(ids), _lib.ptr(cnt), cap, k, ok_path,
+                                           _lib.ptr(out_s), _lib.ptr(out_i), _lib.ptr(out_c), _lib.ptr(path),
+                                           _lib.ptr(tau2), None, 0, st))
+            return cnt
+
+        # 2. + 3. collect at tau with scores, select
+        mark("collect+select")
+        all_users = torch.arange(B, dtype=torch.int32, device=dev)
+        collected.copy_(collect_select(all_users, u_bf16, tau, 0))
+        # path -2 (short), -1 (overflow, tau2 set), 0 (done): one host synchronisation sizes the retry
+        order = torch.argsort(path, stable=True).to(torch.int32)
+        n_short, n_over = torch.bincount((path.to(torch.int64) + 2).clamp(0, 2), minlength=3).tolist()[:2]
+        mark("retry")
+        if n_over > 0:
+            # overflow: collect again at the K-th best stored score
+            users = order[n_short:n_short + n_over].contiguous()
+            u64 = users.to(torch.int64)
+            collected[u64] = collect_select(users, u_bf16.index_select(0, u64).contiguous(),
+                                            tau2.index_select(0, u64).contiguous(), 1)
+            fb = torch.nonzero(path < 0).flatten().to(torch.int32)                        # host sync 2
+        else:
+            fb = order[:n_short]
+        # 4. users still short or overflowing: dense bf16 rows, always exact
+        mark("fallback")
+        if fb.numel() > 0:
+            fb = fb.contiguous()
+            n_fb = fb.numel()
+            ws_bytes = lib.lrb_wide_select_workspace_bytes(n_fb, rows)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            ub = u_bf16.index_select(0, fb.to(torch.int64)).contiguous()
+            _lib.check(lib.lrb_wide_select(_lib.ptr(fb), n_fb, _lib.ptr(ub), tbl, bias, rows, self.row_begin,
+                                           _lib.ptr(excl), stride, None, None, None, 0, k, 2, _lib.ptr(out_s),
+                                           _lib.ptr(out_i), _lib.ptr(out_c), _lib.ptr(path), None, _lib.ptr(ws),
+                                           ws_bytes, st))
+        mark("merge")
+        if not merge:
+            return {"part_scores": out_s, "part_ids": out_i, "part_cnt": out_c, "u": u, "topk_path": path,
+                    "topk_collected": collected}
+        out = merge_lists(out_s, out_i, out_c, k_out=k, labels=labels, ks=ks, packed_out=packed_out, scatter=scatter,
+                          packed_layout=packed_layout)
+        out["u"] = u
+        out["topk_path"] = path
+        out["topk_collected"] = collected
+        mark("end")
         return out
 
     def ce_loss(self, x: torch.Tensor, labels: torch.Tensor, ignore_index: int = 0,

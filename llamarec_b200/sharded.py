@@ -39,6 +39,12 @@ import torch
 import torch.distributed as dist
 
 
+def _check_k(k: int) -> None:
+    # the exchange buffers and the scatter merge are built for the streaming kernels' lists
+    if int(k) > 50:
+        raise ValueError(f"row-sharded retrieval takes k <= 50, got k={k} (LRURec.retrieve takes up to 1024)")
+
+
 def shard_range(n: int, rank: int, world: int) -> Tuple[int, int]:
     """Contiguous split of range(n) into `world` pieces of ceil(n/world) (the last may be short/empty)."""
     per = (n + world - 1) // world
@@ -69,6 +75,7 @@ class CudaBackend:
 
     def local_topk_packed(self, x: torch.Tensor, u: torch.Tensor, k: int, exclude_history: bool) -> torch.Tensor:
         """Local top-k as ONE gather payload: int32 [2, B, k] = scores (bit pattern), ids."""
+        _check_k(k)
         B = x.shape[0]
         key = (B, k, str(u.device))
         buf = self._packed.get(key)
@@ -102,6 +109,7 @@ class CudaBackend:
                         scatter: Optional[dict] = None) -> Optional[torch.Tensor]:
         """All R*b users against this rank's rows -> int32 [R*b, 2, k]: per user scores (bit pattern), ids.
         With `scatter` the rows are written into the owners' recv buffers instead (nothing is returned)."""
+        _check_k(k)
         B = state.shape[0]
         if scatter is not None and self.rows[1] > self.rows[0]:
             seq = {"excl_sorted": excl, "excl_bloom": bloom, "excl_stride": excl_stride}
@@ -310,6 +318,7 @@ class ShardedRetriever:
                     labels: Optional[torch.Tensor] = None, ks: Optional[Sequence[int]] = None) -> Dict[str, torch.Tensor]:
         """x: THIS rank's users [b, L] (every rank passes the same b; labels likewise [b]).  Returns the final
         top-k of the local users against the WHOLE catalogue (+ metric sums over the local users)."""
+        _check_k(k)
         b = x.shape[0]
         mark = self._mark
         mark("begin")
@@ -341,6 +350,7 @@ class ShardedRetriever:
     def retrieve(self, x: torch.Tensor, k: int = 20, exclude_history: bool = True,
                  labels: Optional[torch.Tensor] = None, ks: Optional[Sequence[int]] = None) -> Dict[str, torch.Tensor]:
         """x: the FULL batch of id sequences [B, L], identical on every rank."""
+        _check_k(k)
         B = x.shape[0]
         per = (B + self.world - 1) // self.world
         lo, hi = shard_range(B, self.rank, self.world)
